@@ -1,13 +1,16 @@
 #!/usr/bin/env python
 """Benchmark of the stage03 env step: env-steps/s on N B200s, next to the CPU oracle.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs E_per_gpu] [--preset exp02_vFinal]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs E_per_gpu] [--preset exp02_vFinal] [--dump-outputs DIR]
     python bench.py --impl reference ...      # the CPU arm on the box's host cores
 
 One "step" = one pass of the hot path (Env.step of the reference, 16 physics substeps + logic +
 observation) over every env of the shard.  N > 1 is launched by torchrun (one rank per GPU): envs are
 sharded by index range with no collective on the step path; the only collective is one NCCL
 all-reduce of the episode statistics after the timed region.  Rank 0 prints ONE JSON line.
+
+--dump-outputs DIR writes what the last timed step returned (rank 0's shard) as DIR/<name>.npy, so that two builds can
+be compared output for output: the same arguments give the same seeded actions, hence the same inputs, on every run.
 """
 from __future__ import annotations
 
@@ -83,6 +86,28 @@ class ClockSampler:
         reasons = sorted({n for r in self.rows if len(r) >= 8 for n, v in zip(names, r[4:8]) if v.lower().startswith("active")})
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "samples": len(sm), "reasons": reasons}
+
+
+DUMP_BUDGET_BYTES = 48 << 20          # what --dump-outputs writes in all stays under 64 MB
+
+
+def dump_outputs(folder, arrays, seed=0):
+    """Write ``arrays`` (name -> device tensor whose first axis is the env) as ``folder/<name>.npy``: float32 tensors as
+    float32, every other dtype as float64 (exact for the bool / uint8 / int32 outputs).  When all envs would exceed
+    DUMP_BUDGET_BYTES, the same fixed, seeded sample of env rows is taken from every array; ``env_index.npy`` lists the
+    rows written."""
+    import numpy as np
+    import torch
+    E = next(iter(arrays.values())).shape[0]
+    per_env = sum((4 if t.dtype == torch.float32 else 8) * (t.numel() // E) for t in arrays.values()) + 8
+    n = min(E, max(1, DUMP_BUDGET_BYTES // per_env))
+    rows = np.arange(E) if n == E else np.sort(np.random.RandomState(seed).choice(E, n, replace=False))
+    os.makedirs(folder, exist_ok=True)
+    idx = torch.from_numpy(rows).to(next(iter(arrays.values())).device)
+    for name, t in arrays.items():
+        a = t.index_select(0, idx).cpu().numpy()
+        np.save(os.path.join(folder, name + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
+    np.save(os.path.join(folder, "env_index.npy"), rows.astype(np.float64))
 
 
 # --------------------------------------------------------------------------------------------- CPU arm
@@ -265,6 +290,10 @@ def run_gpu_arm(a):
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     clocks = sampler.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:
+        # step and step_graph return these buffers of the env: they hold the last timed step's outputs until the next step
+        dump_outputs(a.dump_outputs, {**{"obs_" + k: v for k, v in env.obs.items()}, "reward": env.reward, "done": env.done,
+                                      "info": env.info}, seed=a.seed)
     ms = float(ms.item())
     armed = float((env.get_state()["armed"]).mean()) if rank == 0 else 0.0
     # the one collective of the path: episode statistics at rollout end
@@ -463,6 +492,8 @@ def run_lidar_bench(a):
     ms = ev0.elapsed_time(ev1) / a.steps
     launches = _lib.lib().dc_launch_count() - l0
     clocks = sampler.stop()
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"spheres": out}, seed=a.seed)
     spheres = E * O
     # end to end: host positions/quaternions in (pinned), spheres out (pinned)
     h_pos, h_quat = pos.cpu().pin_memory(), quat.cpu().pin_memory()
@@ -528,7 +559,14 @@ def main():
     p.add_argument("--e2e-steps", type=int, default=30)
     p.add_argument("--no-e2e", action="store_true")
     p.add_argument("--no-cpu", action="store_true")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write the outputs of the last timed step as DIR/<name>.npy (float32 / float64; a fixed, seeded "
+                        "sample of envs when all of them would pass 48 MB)")
     a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        p.error("--dump-outputs records the GPU path; the reference arm has no outputs to write")
     if a.impl == "reference":
         return run_reference_arm(a)
     if a.workload == "lidar":
