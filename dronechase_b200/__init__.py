@@ -8,15 +8,15 @@ def __getattr__(name):
     if name in ("BatchedThreatEngageEnv", "lidar_project", "lidar_raycast", "INFO_KEYS"):
         from . import sim
         return getattr(sim, name)
-    if name == "DeviceRollout":
-        from .rollout import DeviceRollout
-        return DeviceRollout
+    if name in ("DeviceRollout", "PPORollout"):
+        from . import rollout
+        return getattr(rollout, name)
     if name in ("DatasetWriter", "MultiFileDataset", "IOData", "collect_data", "collect_data_multiobs"):
         from . import io_data
         return getattr(io_data, name)
-    if name == "LidarInertialActionPolicy":
-        from .policy import LidarInertialActionPolicy
-        return LidarInertialActionPolicy
+    if name in ("LidarInertialActionPolicy", "LidarInertialActorCritic"):
+        from . import policy
+        return getattr(policy, name)
     if name == "VecMonitor":
         from .vec_monitor import VecMonitor
         return VecMonitor

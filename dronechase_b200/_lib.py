@@ -11,7 +11,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "csrc", "libdronechase_b200.so")
 
-DC_ABI_VERSION = 8
+DC_ABI_VERSION = 9
 DC_QUAD_PARAM_WORDS = 88
 DC_INFO_WORDS = 8
 DC_STATE_QUADS = 13
@@ -49,6 +49,12 @@ class dc_policy_weights(C.Structure):
                 ("inertial_w", _F * 3), ("inertial_b", _F * 3), ("action_w", _F * 3), ("action_b", _F * 3),
                 ("final_w", _F), ("final_b", _F), ("pi_w", _F * 8), ("pi_b", _F * 8), ("head_w", _F), ("head_b", _F),
                 ("low", C.c_float * 4), ("high", C.c_float * 4)]
+
+
+class dc_value_weights(C.Structure):
+    _F = C.POINTER(C.c_float)
+    _fields_ = [("n_vf", C.c_int32), ("vf", C.c_int32 * 8), ("vf_w", _F * 8), ("vf_b", _F * 8), ("value_w", _F), ("value_b", _F),
+                ("log_std", _F)]
 
 
 class DroneChaseError(RuntimeError):
@@ -116,6 +122,13 @@ def lib():
     L.dc_policy_create.restype = C.c_int
     L.dc_policy_forward.argtypes = [C.c_void_p] * 4 + [C.c_int64, C.c_void_p, C.c_int32, C.c_void_p]
     L.dc_policy_forward.restype = C.c_int
+    L.dc_policy_create_ac.argtypes = [C.POINTER(dc_policy_weights), C.POINTER(dc_value_weights), C.c_int, C.POINTER(C.c_void_p)]
+    L.dc_policy_create_ac.restype = C.c_int
+    L.dc_policy_act.argtypes = ([C.c_void_p] * 4 + [C.c_int64, C.c_uint64, C.c_int64, C.c_uint32, C.c_int32] + [C.c_void_p] * 4
+                                + [C.c_int32, C.c_void_p])
+    L.dc_policy_act.restype = C.c_int
+    L.dc_gae.argtypes = [C.c_void_p] * 4 + [C.c_int64, C.c_int64, C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.dc_gae.restype = C.c_int
     L.dc_policy_destroy.argtypes = [C.c_void_p]
     L.dc_policy_destroy.restype = None
     L.dc_quad_is_builtin.argtypes = [C.c_void_p]
@@ -129,7 +142,7 @@ def lib():
 EXPORTS = ("dc_create", "dc_bind", "dc_reset", "dc_step", "dc_set_actions", "dc_note_graph_replay", "dc_destroy", "dc_last_error", "dc_copy_state",
            "dc_state_bytes", "dc_lidar_project", "dc_lidar_raycast", "dc_launch_count", "dc_host_scatter_sphere", "dc_host_scatter_stack", "dc_scatter_hits",
            "dc_scatter_stack", "dc_abi_info", "dc_host_register", "dc_host_unregister", "dc_mirror_hits", "dc_lw_observe", "dc_quad_is_builtin", "dc_diff_hits", "dc_host_apply_pairs",
-           "dc_policy_create", "dc_policy_forward", "dc_policy_destroy")
+           "dc_policy_create", "dc_policy_forward", "dc_policy_destroy", "dc_policy_create_ac", "dc_policy_act", "dc_gae")
 
 
 def check(code: int, what: str):

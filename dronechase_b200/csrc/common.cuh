@@ -65,7 +65,8 @@ __device__ __forceinline__ double fast_rcp(double x) { return 1.0 / x; }
 template <typename R> __device__ __forceinline__ R clamp_(R v, R lo, R hi) { return min_(max_(v, lo), hi); }
 
 // ---- Philox4x32-10, same stream layout as oracle/philox.py ------------------------------------
-enum { STREAM_HIT = 1, STREAM_SPAWN = 2, STREAM_MOTOR = 3, STREAM_FUSE = 4 };
+// STREAM_POLICY: the Gaussian noise of the sampled actions (policy_kernel.cu, dc_policy_act; index = the caller's running counter)
+enum { STREAM_HIT = 1, STREAM_SPAWN = 2, STREAM_MOTOR = 3, STREAM_FUSE = 4, STREAM_POLICY = 5 };
 
 __device__ __forceinline__ uint4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
                                                uint32_t k0, uint32_t k1) {

@@ -86,6 +86,9 @@ class LidarInertialActionPolicy(nn.Module):
                 "deterministic mean action")
 
     # ------------------------------------------------------------------ weights of a reference-trained SB3 model
+    # (SB3 key prefix, own prefix) of everything but the features extractor
+    _SB3_KEYS = (("mlp_extractor.policy_net.", "policy_net."), ("action_net.", "action_net."))
+
     def load_sb3_state_dict(self, sd: Dict[str, torch.Tensor]) -> "LidarInertialActionPolicy":
         """``sd`` = ``model.policy.state_dict()`` of an SB3 PPO (keys ``features_extractor.*`` or ``pi_features_extractor.*``,
         ``mlp_extractor.policy_net.*``, ``action_net.*``); value-function and log_std entries are ignored."""
@@ -94,10 +97,9 @@ class LidarInertialActionPolicy(nn.Module):
         for k, v in sd.items():
             if k.startswith(fx):
                 mine[k[len(fx):]] = v
-            elif k.startswith("mlp_extractor.policy_net."):
-                mine["policy_net." + k[len("mlp_extractor.policy_net."):]] = v
-            elif k.startswith("action_net."):
-                mine[k] = v
+            for theirs, ours in self._SB3_KEYS:
+                if k.startswith(theirs):
+                    mine[ours + k[len(theirs):]] = v
         want = {k for k in self.state_dict() if k not in ("low", "high")}
         missing = want - set(mine)
         if missing:
@@ -105,19 +107,95 @@ class LidarInertialActionPolicy(nn.Module):
         self.load_state_dict({**{k: mine[k] for k in want}, "low": self.low, "high": self.high})
         return self
 
+    @staticmethod
+    def _sb3_widths(sd: Dict[str, torch.Tensor], net: str):
+        out, i = [], 0
+        while f"mlp_extractor.{net}.{i}.weight" in sd:
+            out.append(sd[f"mlp_extractor.{net}.{i}.weight"].shape[0])
+            i += 2
+        return out
+
+    @classmethod
+    def _sb3_sizes(cls, sd: Dict[str, torch.Tensor]) -> Dict[str, object]:
+        return {"pi": cls._sb3_widths(sd, "policy_net")}
+
     @classmethod
     def from_sb3_zip(cls, path: str, env=None, **kw) -> "LidarInertialActionPolicy":
         """Build from an SB3 ``model.save`` archive: reads ``policy.pth``, infers pi sizes and features_dim from the shapes."""
         with zipfile.ZipFile(path) as z:
             sd = torch.load(io.BytesIO(z.read("policy.pth")), map_location="cpu", weights_only=True)
-        pi, i = [], 0
-        while f"mlp_extractor.policy_net.{i}.weight" in sd:
-            pi.append(sd[f"mlp_extractor.policy_net.{i}.weight"].shape[0])
-            i += 2
         fx = "pi_features_extractor." if any(k.startswith("pi_features_extractor.") for k in sd) else "features_extractor."
         kw.setdefault("features_dim", sd[fx + "final_layer.0.weight"].shape[0])
         kw.setdefault("lidar_channels", sd[fx + "lidar_feature_extractor.0.weight"].shape[1])
-        return cls(env=env, pi=pi, seed=None, **kw).load_sb3_state_dict(sd)
+        return cls(env=env, seed=None, **cls._sb3_sizes(sd), **kw).load_sb3_state_dict(sd)
+
+
+class LidarInertialActorCritic(LidarInertialActionPolicy):
+    """The whole SB3 ``ActorCriticPolicy`` of the reference's PPO (shared features extractor, ``net_arch = dict(pi=h, vf=h)``,
+    ``DiagGaussianDistribution`` with ``log_std_init = 0``): the actor of ``LidarInertialActionPolicy`` plus ``vf_net``
+    (= ``mlp_extractor.value_net``: hidden layers over the features, the activation of pi), ``value_net`` and ``log_std``.
+    The value-branch parameters are created after the actor's, so a seeded actor is initialised as in the parent class.
+    ``forward`` stays the clipped mean action; ``forward_train``, ``evaluate_actions`` and ``predict_values`` are
+    differentiable, for the PPO update.  ``fused()`` gives the one-kernel rollout policy (``FusedPolicy.act`` / ``values``)."""
+
+    _SB3_KEYS = LidarInertialActionPolicy._SB3_KEYS + (("mlp_extractor.value_net.", "vf_net."), ("value_net.", "value_net."),
+                                                       ("log_std", "log_std"))
+
+    def __init__(self, env=None, lidar_channels: int = 3, features_dim: int = 256, pi: Sequence[int] = (128, 256, 512),
+                 vf: Optional[Sequence[int]] = None, activation: str = "tanh", seed: Optional[int] = 0, device=None):
+        super().__init__(env, lidar_channels, features_dim, pi, activation, seed, device)
+        device = env.device if env is not None else device
+        act = {"tanh": nn.Tanh, "relu": nn.ReLU}[activation]
+        vf = tuple(int(h) for h in (pi if vf is None else vf))
+        layers, n = [], int(features_dim)
+        for h in vf:
+            layers += [nn.Linear(n, h), act()]
+            n = h
+        self.vf_net = nn.Sequential(*layers)
+        self.value_net = nn.Linear(n, 1)
+        self.log_std = nn.Parameter(torch.zeros(4))
+        self.vf = vf
+        if device is not None:
+            self.to(device)
+        self.eval()
+
+    def forward_train(self, obs: Dict[str, torch.Tensor]):
+        """(mean action, unclipped [N, 4]; value [N, 1]) from one evaluation of the features."""
+        f = self.features(obs)
+        return self.action_net(self.policy_net(f)), self.value_net(self.vf_net(f))
+
+    def predict_values(self, obs: Dict[str, torch.Tensor]) -> torch.Tensor:
+        """SB3 ``predict_values``: [N, 1]."""
+        return self.value_net(self.vf_net(self.features(obs)))
+
+    def evaluate_actions(self, obs: Dict[str, torch.Tensor], actions: torch.Tensor):
+        """SB3 ``evaluate_actions``: (value [N, 1], log_prob [N], entropy [N]) of the UNCLIPPED ``actions`` under the diagonal
+        Gaussian N(mean, exp(log_std)^2)."""
+        mean, value = self.forward_train(obs)
+        dist = torch.distributions.Normal(mean, torch.ones_like(mean) * self.log_std.exp())
+        return value, dist.log_prob(actions).sum(dim=-1), dist.entropy().sum(dim=-1)
+
+    def describe(self) -> str:
+        n = sum(p.numel() for p in self.parameters())
+        return (f"LidarInertialActionExtractor (ppo_policies.py:234-342) + pi {list(self.pi)} + action_net, vf {list(self.vf)} + "
+                f"value_net, log_std; {n} parameters, float32, diagonal Gaussian actor-critic")
+
+    def load_sb3_state_dict(self, sd: Dict[str, torch.Tensor]) -> "LidarInertialActorCritic":
+        """As the parent's, and ``mlp_extractor.value_net.*``, ``value_net.*`` and ``log_std`` too.  The value branch must read the
+        actor's features: an archive trained with ``share_features_extractor=False`` (its ``vf_features_extractor.*`` differ from
+        the actor's extractor) raises ``ValueError``."""
+        fx = "pi_features_extractor." if any(k.startswith("pi_features_extractor.") for k in sd) else "features_extractor."
+        for k, v in sd.items():
+            if k.startswith("vf_features_extractor."):
+                mine = sd.get(fx + k[len("vf_features_extractor."):])
+                if mine is None or mine.shape != v.shape or not torch.equal(mine, v):
+                    raise ValueError("this SB3 policy has a separate vf_features_extractor (share_features_extractor=False): "
+                                     "LidarInertialActorCritic evaluates the value branch on the actor's features")
+        return super().load_sb3_state_dict(sd)
+
+    @classmethod
+    def _sb3_sizes(cls, sd: Dict[str, torch.Tensor]) -> Dict[str, object]:
+        return {"pi": cls._sb3_widths(sd, "policy_net"), "vf": cls._sb3_widths(sd, "value_net")}
 
 
 class FusedPolicy:
@@ -128,7 +206,13 @@ class FusedPolicy:
     The weights are re-laid out once, here; call ``refresh()`` after the module's parameters changed (PPO update).
     Shapes the kernel holds: features_dim and the hidden widths of ``pi`` multiples of 64 up to 256, the last one up to 1024
     (the defaults and ``net_arch`` of the reference's apps); anything else raises, use the module itself.  There is no
-    fallback: without the CUDA library or a device this class raises."""
+    fallback: without the CUDA library or a device this class raises.
+
+    Built from a ``LidarInertialActorCritic`` (``dc_policy_create_ac``), it also runs the actor-critic kernel
+    (``dc_policy_act``): ``act`` samples actions for PPO rollout collection, ``values`` gives V(s).  Precision matters more
+    there: the log-probability error is about ``|eps| * (mean error) / sigma``.  With ``"tf32"`` (5e-3 on the mean) that is
+    about 1e-2 in log-probability, a 1 % bias in PPO's first-epoch probability ratio; the default ``"3xtf32"`` keeps it near
+    1e-4."""
 
     PRECISIONS = {"3xtf32": 0, "tf32": 1}
 
@@ -171,15 +255,26 @@ class FusedPolicy:
         w.head_w, w.head_b = ptr(wa["head_w"]), ptr(wa["head_b"])
         for k in range(4):
             w.low[k], w.high[k] = float(m.low[k]), float(m.high[k])
-        torch.cuda.synchronize(dev)
         h = C.c_void_p()
-        _lib.check(_lib.lib().dc_policy_create(C.byref(w), dev.index or 0, C.byref(h)), "dc_policy_create")
+        if isinstance(m, LidarInertialActorCritic):
+            if len(m.vf) > 8:
+                raise ValueError("FusedPolicy: at most 8 hidden layers in vf")
+            v = _lib.dc_value_weights()
+            v.n_vf = len(m.vf)
+            vl = [x for x in m.vf_net if isinstance(x, nn.Linear)]
+            for i, h_ in enumerate(m.vf):
+                v.vf[i], v.vf_w[i], v.vf_b[i] = h_, ptr(vl[i].weight), ptr(vl[i].bias)
+            v.value_w, v.value_b, v.log_std = ptr(m.value_net.weight), ptr(m.value_net.bias), ptr(m.log_std)
+            torch.cuda.synchronize(dev)
+            _lib.check(_lib.lib().dc_policy_create_ac(C.byref(w), C.byref(v), dev.index or 0, C.byref(h)), "dc_policy_create_ac")
+        else:
+            torch.cuda.synchronize(dev)
+            _lib.check(_lib.lib().dc_policy_create(C.byref(w), dev.index or 0, C.byref(h)), "dc_policy_create")
         self.close()
         self._handle, self.device = h, dev
         return self
 
-    def __call__(self, obs: Dict[str, torch.Tensor], out: Optional[torch.Tensor] = None) -> torch.Tensor:
-        C = self._C
+    def _check_obs(self, obs: Dict[str, torch.Tensor]):
         lidar, inertial, last = obs["lidar"], obs["inertial_data"], obs["last_action"]
         E = lidar.shape[0]
         for t in (lidar, inertial, last):
@@ -188,6 +283,11 @@ class FusedPolicy:
         if tuple(lidar.shape[1:]) != (self.module.lidar_feature_extractor[0].in_channels, 13, 26) or inertial.numel() != E * 15 \
                 or last.numel() != E * 4:
             raise ValueError("FusedPolicy: observation shapes must be lidar [E,C,13,26], inertial_data [E,15], last_action [E,4]")
+        return lidar, inertial, last, E
+
+    def __call__(self, obs: Dict[str, torch.Tensor], out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        C = self._C
+        lidar, inertial, last, E = self._check_obs(obs)
         if out is None:
             out = torch.empty(E, 4, dtype=torch.float32, device=self.device)
         with torch.cuda.device(self.device):
@@ -195,6 +295,44 @@ class FusedPolicy:
                 self._handle, C.c_void_p(lidar.data_ptr()), C.c_void_p(inertial.data_ptr()), C.c_void_p(last.data_ptr()), E,
                 C.c_void_p(out.data_ptr()), self._prec, C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)), "dc_policy_forward")
         return out
+
+    def _run_act(self, obs, counter: int, seed: int, env_offset: int, sample: int, env_actions, raw_actions, log_prob, value):
+        if not isinstance(self.module, LidarInertialActorCritic):
+            raise self._lib.DroneChaseError("FusedPolicy.act / values need a LidarInertialActorCritic module (value branch, log_std)")
+        C = self._C
+        lidar, inertial, last, E = self._check_obs(obs)
+
+        def buf(t, shape):
+            if t is None:
+                return torch.empty(shape, dtype=torch.float32, device=self.device)
+            if t.dtype != torch.float32 or not t.is_contiguous() or t.device != self.device or tuple(t.shape) != shape:
+                raise ValueError(f"FusedPolicy: outputs must be contiguous float32 tensors of shape {shape} on the policy's device")
+            return t
+        env_actions, value = buf(env_actions, (E, 4)), buf(value, (E,))
+        if sample:
+            raw_actions, log_prob = buf(raw_actions, (E, 4)), buf(log_prob, (E,))
+        p = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None      # noqa: E731
+        with torch.cuda.device(self.device):
+            self._lib.check(self._lib.lib().dc_policy_act(
+                self._handle, p(lidar), p(inertial), p(last), E, int(seed) & 0xFFFFFFFFFFFFFFFF, int(env_offset),
+                int(counter) & 0xFFFFFFFF, sample, p(env_actions), p(raw_actions) if sample else None,
+                p(log_prob) if sample else None, p(value), self._prec,
+                C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)), "dc_policy_act")
+        return env_actions, raw_actions, log_prob, value
+
+    def act(self, obs: Dict[str, torch.Tensor], counter: int, *, seed: int = 0, env_offset: int = 0,
+            env_actions: Optional[torch.Tensor] = None, raw_actions: Optional[torch.Tensor] = None,
+            log_prob: Optional[torch.Tensor] = None, value: Optional[torch.Tensor] = None, sample: bool = True):
+        """One PPO collection step in one launch: (env_actions [E,4] clipped to the action box, raw_actions [E,4] the unclipped
+        Gaussian sample that goes into the rollout buffer, log_prob [E], value [E]).  The noise of row e is a pure function of
+        (seed, counter, env_offset + e): Philox4x32-10 stream 5 of the simulator's counter-based generator.  Outputs given as
+        arguments are written in place.  ``sample=False``: env_actions = the clipped mean action, bit for bit what ``__call__``
+        returns, and raw_actions / log_prob are None."""
+        return self._run_act(obs, counter, seed, env_offset, int(bool(sample)), env_actions, raw_actions, log_prob, value)
+
+    def values(self, obs: Dict[str, torch.Tensor], out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """V(s) [E] (the actor-critic kernel without sampling: ``predict_values`` for the bootstrap of the last step)."""
+        return self._run_act(obs, 0, 0, 0, 0, None, None, None, out)[3]
 
     def describe(self) -> str:
         return self.module.describe().replace("float32", "one fused kernel, " + ("3 x TF32 (float32-grade)" if self._prec == 0 else "TF32"))

@@ -51,20 +51,28 @@ class DeviceRollout:
         return sum(t.numel() * t.element_size() for t in (self.hits, self.inertial, self.last_action, self.actions,
                                                           self.rewards, self.dones, self.mask) if t is not None)
 
-    def add(self, actions: torch.Tensor):
-        """Store the env's CURRENT observation with `actions`, step the env, store reward and done (SB3 order)."""
-        e, t = self.env, self.pos
+    def _store_obs(self, t: int):
+        e = self.env
         self.hits[t].copy_(e.lidar_hits, non_blocking=True)
         if self.level5:
             self.mask[t].copy_(e.obs["validity_mask"], non_blocking=True)
         self.inertial[t].copy_(e.obs["inertial_data"], non_blocking=True)
         self.last_action[t].copy_(e.obs["last_action"], non_blocking=True)
-        if actions.data_ptr() != self.actions[t].data_ptr():      # a policy may have written the slab itself (FusedPolicy, out=)
-            self.actions[t].copy_(actions, non_blocking=True)
-        e.step(self.actions[t])                                   # zero copy: the kernel reads the stored slab
+
+    def _step(self, t: int, env_actions: torch.Tensor):
+        e = self.env
+        e.step(env_actions)                                       # zero copy: the kernel reads the slab
         self.rewards[t].copy_(e.reward, non_blocking=True)
         self.dones[t].copy_(e.done, non_blocking=True)
         self.pos += 1
+
+    def add(self, actions: torch.Tensor):
+        """Store the env's CURRENT observation with `actions`, step the env, store reward and done (SB3 order)."""
+        t = self.pos
+        self._store_obs(t)
+        if actions.data_ptr() != self.actions[t].data_ptr():      # a policy may have written the slab itself (FusedPolicy, out=)
+            self.actions[t].copy_(actions, non_blocking=True)
+        self._step(t, self.actions[t])
 
     def collect(self, policy: Callable[[Dict[str, torch.Tensor]], torch.Tensor], n_steps: Optional[int] = None):
         """Fill the buffer from position 0: actions = policy(env.obs) on the device, nothing touches the host."""
@@ -104,3 +112,76 @@ class DeviceRollout:
                 "inertial_data": self.inertial.view(T * E, 15)[idx], "last_action": self.last_action.view(T * E, 4)[idx],
                 "actions": self.actions.view(T * E, 4)[idx], "rewards": self.rewards.view(T * E)[idx],
                 "dones": self.dones.view(T * E)[idx]}
+
+
+class PPORollout(DeviceRollout):
+    """The device rollout of SB3's ``collect_rollouts`` for PPO: per step ONE actor-critic kernel launch
+    (``FusedPolicy.act`` of a ``LidarInertialActorCritic``) samples the action, its log-probability and V(s); ``actions``
+    keeps the unclipped sample, as SB3's buffer does, and the env steps on the clipped copy.  After the loop V(s_T) goes to
+    ``last_values`` and ``compute_returns_and_advantage`` runs GAE in one kernel (``dc_gae``).
+
+        env = BatchedThreatEngageEnv("exp02_v2_full", n_envs=65536, with_hits=True)
+        ro = PPORollout(env, n_steps=128, seed=1)
+        fused = LidarInertialActorCritic(env=env).fused()
+        ro.collect(fused).compute_returns_and_advantage(gamma=0.99, gae_lambda=0.95)
+        batch = ro.minibatch(torch.randperm(ro.n_steps * env.n_envs, device="cuda")[:4096])
+
+    The noise of env e at a step is a pure function of (seed, counter, env.env_offset + e); the counter counts the steps
+    this rollout has collected, across ``collect`` calls.  level5 is not supported: its stacked observation is not what
+    the fused kernel reads."""
+
+    def __init__(self, env: BatchedThreatEngageEnv, n_steps: int, seed: int = 0):
+        if env.cfg.family == "level5":
+            raise _lib.DroneChaseError("PPORollout: level5's stacked observation is not what the fused policy kernel reads")
+        super().__init__(env, n_steps)
+        T, E = self.n_steps, env.n_envs
+        f32 = dict(dtype=torch.float32, device=env.device)
+        self.values = torch.empty(T, E, **f32)
+        self.log_probs = torch.empty(T, E, **f32)
+        self.advantages = torch.zeros(T, E, **f32)
+        self.returns = torch.zeros(T, E, **f32)
+        self.last_values = torch.zeros(E, **f32)
+        self.env_actions = torch.empty(E, 4, **f32)              # the clipped actions env.step reads in place
+        assert self.env_actions.data_ptr() % 16 == 0
+        self.seed, self.counter = int(seed), 0
+
+    @property
+    def bytes(self) -> int:
+        return super().bytes + sum(t.numel() * t.element_size() for t in (self.values, self.log_probs, self.advantages,
+                                                                          self.returns, self.last_values, self.env_actions))
+
+    def collect(self, fused, n_steps: Optional[int] = None):
+        """Fill the buffer from position 0 with ``fused`` (a FusedPolicy of a LidarInertialActorCritic); nothing touches the
+        host.  Then last_values = V(observation after the last step)."""
+        if not hasattr(fused, "act"):
+            raise TypeError("PPORollout.collect needs a FusedPolicy of a LidarInertialActorCritic")
+        e = self.env
+        self.pos = 0
+        for _ in range(n_steps or self.n_steps):
+            t = self.pos
+            self._store_obs(t)
+            fused.act(e.obs, self.counter, seed=self.seed, env_offset=e.env_offset, env_actions=self.env_actions,
+                      raw_actions=self.actions[t], log_prob=self.log_probs[t], value=self.values[t])
+            self.counter += 1
+            self._step(t, self.env_actions)
+        fused.values(e.obs, out=self.last_values)
+        return self
+
+    def compute_returns_and_advantage(self, gamma: float = 0.99, gae_lambda: float = 0.95):
+        """SB3's RolloutBuffer.compute_returns_and_advantage over the collected steps, in one kernel (dc_gae)."""
+        e, T = self.env, self.pos
+        p = lambda t: C.c_void_p(t.data_ptr())      # noqa: E731
+        with torch.cuda.device(e.device):
+            _lib.check(_lib.lib().dc_gae(p(self.rewards), p(self.dones), p(self.values), p(self.last_values), T, e.n_envs,
+                                         float(gamma), float(gae_lambda), p(self.advantages), p(self.returns),
+                                         C.c_void_p(torch.cuda.current_stream(e.device).cuda_stream)), "dc_gae")
+        return self
+
+    def minibatch(self, flat_index: torch.Tensor) -> Dict[str, torch.Tensor]:
+        """The parent's batch (``actions`` = the unclipped samples) + ``old_values``, ``old_log_prob``, ``advantages``,
+        ``returns``."""
+        b = super().minibatch(flat_index)
+        idx = flat_index.to(device=self.env.device, dtype=torch.int64)
+        n = self.n_steps * self.env.n_envs
+        return {**b, "old_values": self.values.view(n)[idx], "old_log_prob": self.log_probs.view(n)[idx],
+                "advantages": self.advantages.view(n)[idx], "returns": self.returns.view(n)[idx]}

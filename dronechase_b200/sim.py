@@ -186,6 +186,11 @@ class BatchedThreatEngageEnv:
         _lib.check(self._L.dc_bind(self._sim, C.byref(b)), "dc_bind")
         self.steps_done = 0
 
+    @property
+    def env_offset(self) -> int:
+        """Global index of this env batch's first env (dc_config.env_offset): the env coordinate of its random streams."""
+        return int(self._c.env_offset)
+
     # ------------------------------------------------------------------ gym-like API
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)

@@ -39,7 +39,7 @@
 extern "C" {
 #endif
 
-#define DC_ABI_VERSION 8   /* v8: dc_policy_* (the agent's network as one kernel; dc_config / dc_buffers unchanged); v7: dc_host_register / dc_host_unregister / dc_mirror_hits */
+#define DC_ABI_VERSION 9   /* v9: dc_policy_create_ac / dc_policy_act / dc_gae (PPO rollout collection on the device); v8: dc_policy_* (the agent's network as one kernel; dc_config / dc_buffers unchanged); v7: dc_host_register / dc_host_unregister / dc_mirror_hits */
 
 enum dc_status {
     DC_OK = 0,
@@ -352,6 +352,34 @@ int dc_policy_create(const dc_policy_weights* weights, int device, dc_policy** o
 int dc_policy_forward(dc_policy* policy, const float* lidar, const float* inertial, const float* last_action, int64_t n_envs,
                       float* actions, int32_t precision, void* stream);
 void dc_policy_destroy(dc_policy* policy);
+
+/* ---- PPO rollout collection on the device: what SB3's OnPolicyAlgorithm.collect_rollouts asks of the policy each step (a sampled
+ * action, its log-probability, V(s)) and, after the last step, RolloutBuffer.compute_returns_and_advantage.
+ * dc_value_weights: the rest of SB3's ActorCriticPolicy with a shared features extractor and net_arch = dict(pi=..., vf=...):
+ * mlp_extractor.value_net (hidden layers over the features, the activation of pi), value_net, and the DiagGaussian's log_std.
+ * Device pointers in torch layout, read once by dc_policy_create_ac. */
+typedef struct dc_value_weights {
+    int32_t n_vf; int32_t vf[8];                 /* hidden widths of mlp_extractor.value_net: 0..8 layers, the rules of pi */
+    const float* vf_w[8]; const float* vf_b[8];
+    const float* value_w; const float* value_b;  /* value_net: [1][last width], [1] */
+    const float* log_std;                        /* [4], read once, like the weights */
+} dc_value_weights;
+/* A policy that dc_policy_act can run as well as dc_policy_forward (which runs the plain kernel on it, unchanged). */
+int dc_policy_create_ac(const dc_policy_weights* weights, const dc_value_weights* value, int device, dc_policy** out);
+/* One launch for n_envs rows.  mean = action_net(...) (unclipped), value[e] = V(s).  sample = 1: eps = four standard normals
+ * (Box-Muller on the Philox4x32-10 block of key seed, counter (counter, 5, env_offset + e, 0)), raw_actions[e] = mean +
+ * exp(log_std) * eps, env_actions[e] = clip(raw) to the action box, log_prob[e] = sum_k(-eps_k^2 / 2 - log_std_k) - 2 log(2 pi).
+ * sample = 0: env_actions = clip(mean), bit for bit what dc_policy_forward writes; raw_actions and log_prob are not written and
+ * may be NULL.  The same bits on every run and for any split of the rows (pass the split's env_offset). */
+int dc_policy_act(dc_policy* policy, const float* lidar, const float* inertial, const float* last_action, int64_t n_envs,
+                  uint64_t seed, int64_t env_offset, uint32_t counter, int32_t sample,
+                  float* env_actions /*[n][4] clipped*/, float* raw_actions /*[n][4], NULL if !sample*/,
+                  float* log_prob /*[n], NULL if !sample*/, float* value /*[n]*/, int32_t precision, void* stream);
+/* Generalized advantage estimation over a [T][E] rollout, float32 device arrays (dones uint8: 1 = the episode ended AFTER step
+ * t): delta_t = r_t + gamma V_{t+1} (1 - d_t) - V_t with V_T = last_values [E]; A_t = delta_t + gamma lambda (1 - d_t) A_{t+1};
+ * returns = A + V.  SB3's compute_returns_and_advantage with episode_starts[t + 1] = dones[t]. */
+int dc_gae(const float* rewards, const uint8_t* dones, const float* values, const float* last_values, int64_t T, int64_t E,
+           float gamma, float gae_lambda, float* advantages, float* returns, void* stream);
 
 #ifdef __cplusplus
 }
