@@ -15,8 +15,16 @@ from tests.test_gpu_policy import _obs
 pytestmark = pytest.mark.gpu
 
 TOL = {"3xtf32": 2e-5, "tf32": 5e-3}
-NETS = [(3, 256, (128, 256, 512), "tanh"), (2, 128, (64,), "tanh"), (3, 192, (), "tanh"), (3, 256, (256, 256, 256), "relu"),
-        (1, 64, (256, 1024), "tanh")]
+# (C, features_dim, pi, vf, activation); vf = None: the module copies pi.  Together they reach every path of value_branch and
+# every width class widths_ok accepts: pi = () with a vf (final_layer evaluated a second time into the stash), vf = () after
+# a pi layer narrower than the features (value_net on the stash), an intermediate layer of 192 columns (idle column warps), a
+# last layer of 320 / 960 columns (the last head_layer pass partly filled), and 8 pi + 8 vf layers (15 of MAX_LAYERS = 16).
+NETS = [(3, 256, (128, 256, 512), None, "tanh"), (2, 128, (64,), None, "tanh"), (3, 192, (), None, "tanh"),
+        (3, 256, (256, 256, 256), None, "relu"), (1, 64, (256, 1024), None, "tanh"),
+        (3, 256, (192, 320), (64, 1024), "tanh"), (2, 64, (), (256, 128), "relu"), (1, 128, (64,), (), "tanh"),
+        (3, 192, (256, 64), (192,), "tanh"), (3, 256, (64,) * 7 + (960,), (256,) * 7 + (448,), "tanh")]
+NET_IDS = [f"{C}-{F}-pi{i}-{a}" if vf is None else f"{C}-{F}-pi{i}-vf{i}-{a}" for i, (C, F, pi, vf, a) in enumerate(NETS)]
+BATCHES = (1, 63, 64, 65, 127, 128, 1000, 4133)            # one env, ragged last blocks, whole blocks, several blocks
 LOW, HIGH = torch.tensor([-1.0, -1, -1, 0]), torch.tensor([1.0, 1, 1, 1])
 
 
@@ -32,51 +40,67 @@ def _ac(C, features_dim, pi, activation, log_std, scale=1.6, vf=None):
     return ac
 
 
-@pytest.mark.parametrize("log_std", [0.0, -1.0])
-@pytest.mark.parametrize("precision", ["3xtf32", "tf32"])
-@pytest.mark.parametrize("C,features_dim,pi,activation", NETS)
-def test_act_against_the_plain_kernel_the_module_and_the_oracle(precision, C, features_dim, pi, activation, log_std):
+def _check_act(ac, fused, precision, log_std, E, C):
+    """One batch of E envs through act: sample = 0 is the plain kernel bit for bit and V(s) is the float32 module's; sample = 1
+    gives the same V(s), env_action = clip(raw), the oracle's normals and the float64 log-probability."""
     from oracle.policy_ac_fragment_model import policy_normals
-    ac = _ac(C, features_dim, pi, activation, log_std)
-    fused = ac.fused(precision)
     seed, counter, off = 0x1234_5678_9ABC, 3, 100
     sigma = math.exp(log_std)
     low, high = LOW.cuda(), HIGH.cuda()
-    for E in (1, 63, 64, 65, 1000, 4133):
-        obs = _obs(E, C, seed=E)
-        mean_a, raw0, lp0, v0 = fused.act(obs, counter, sample=False)
-        assert raw0 is None and lp0 is None
-        assert torch.equal(mean_a, fused(obs)), "sample = 0: not the plain kernel's action bit for bit"
+    obs = _obs(E, C, seed=E)
+    mean_a, raw0, lp0, v0 = fused.act(obs, counter, sample=False)
+    assert raw0 is None and lp0 is None
+    assert torch.equal(mean_a, fused(obs)), "sample = 0: not the plain kernel's action bit for bit"
+    with torch.no_grad():
+        _, want_v = ac.forward_train(obs)
+    err_v = float((v0 - want_v[:, 0]).abs().max())
+    assert err_v < TOL[precision], f"E={E}: |value - float32 module| = {err_v}"
+    env_a, raw, lp, v = fused.act(obs, counter, seed=seed, env_offset=off)
+    torch.cuda.synchronize()
+    assert torch.equal(v, v0)
+    assert torch.equal(env_a, torch.minimum(torch.maximum(raw, low), high)), "env_action is not clip(raw)"
+    eps64 = policy_normals(seed, counter, off + np.arange(E))
+    # where the mean is inside the box the sample = 0 action IS the kernel's mean: recover the kernel's eps there
+    m = mean_a.double().cpu().numpy()
+    inside = (m > LOW.numpy()) & (m < HIGH.numpy())
+    r = raw.double().cpu().numpy()
+    eps = (r - m) / np.float32(sigma)
+    assert inside.sum() > 0.2 * inside.size
+    assert np.abs(eps - eps64)[inside].max() < 1e-5 + 1e-6 * np.abs(r[inside]).max() / sigma, "eps differs from the oracle"
+    assert np.abs(r - (m + np.float32(sigma) * eps64))[inside].max() < 2e-6 * (1 + np.abs(r).max())
+    lp64 = (-0.5 * eps64 ** 2 - log_std).sum(1) - 2 * math.log(2 * math.pi)
+    assert np.abs(lp.double().cpu().numpy() - lp64).max() < 1e-4
+    if precision == "3xtf32" and log_std == 0.0:
         with torch.no_grad():
-            _, want_v = ac.forward_train(obs)
-        err_v = float((v0 - want_v[:, 0]).abs().max())
-        assert err_v < TOL[precision], f"E={E}: |value - float32 module| = {err_v}"
-        env_a, raw, lp, v = fused.act(obs, counter, seed=seed, env_offset=off)
-        torch.cuda.synchronize()
-        assert torch.equal(v, v0)
-        assert torch.equal(env_a, torch.minimum(torch.maximum(raw, low), high)), "env_action is not clip(raw)"
-        eps64 = policy_normals(seed, counter, off + np.arange(E))
-        # where the mean is inside the box the sample = 0 action IS the kernel's mean: recover the kernel's eps there
-        m = mean_a.double().cpu().numpy()
-        inside = (m > LOW.numpy()) & (m < HIGH.numpy())
-        r = raw.double().cpu().numpy()
-        eps = (r - m) / np.float32(sigma)
-        assert inside.sum() > 0.2 * inside.size
-        assert np.abs(eps - eps64)[inside].max() < 1e-5 + 1e-6 * np.abs(r[inside]).max() / sigma, "eps differs from the oracle"
-        assert np.abs(r - (m + np.float32(sigma) * eps64))[inside].max() < 2e-6 * (1 + np.abs(r).max())
-        lp64 = (-0.5 * eps64 ** 2 - log_std).sum(1) - 2 * math.log(2 * math.pi)
-        assert np.abs(lp.double().cpu().numpy() - lp64).max() < 1e-4
-        if precision == "3xtf32" and log_std == 0.0:
-            with torch.no_grad():
-                _, want_lp, _ = ac.evaluate_actions(obs, raw)
-            assert float((lp - want_lp).abs().max()) < 5e-4
+            _, want_lp, _ = ac.evaluate_actions(obs, raw)
+        assert float((lp - want_lp).abs().max()) < 5e-4
+
+
+@pytest.mark.parametrize("log_std", [0.0, -1.0])
+@pytest.mark.parametrize("precision", ["3xtf32", "tf32"])
+@pytest.mark.parametrize("C,features_dim,pi,vf,activation", NETS, ids=NET_IDS)
+def test_act_against_the_plain_kernel_the_module_and_the_oracle(precision, C, features_dim, pi, vf, activation, log_std):
+    ac = _ac(C, features_dim, pi, activation, log_std, vf=vf)
+    fused = ac.fused(precision)
+    for E in BATCHES:
+        _check_act(ac, fused, precision, log_std, E, C)
     # the same bits on every run, and for any batch a row travels in (with the batch's env_offset)
+    seed, off = 0x1234_5678_9ABC, 100
     obs = _obs(1000, C, seed=1)
     a = fused.act(obs, 7, seed=seed, env_offset=off)
     b = fused.act(obs, 7, seed=seed, env_offset=off)
     part = fused.act({k: x[640:].contiguous() for k, x in obs.items()}, 7, seed=seed, env_offset=off + 640)
     for x, y, z in zip(a, b, part):
         assert torch.equal(x, y) and torch.equal(x[640:], z)
+    fused.close()
+
+
+def test_act_on_a_ragged_batch_of_65537():
+    """1,025 blocks, the last with one env: grid-sized row and env indices."""
+    C, features_dim, pi, vf, activation = NETS[0]
+    ac = _ac(C, features_dim, pi, activation, 0.0, vf=vf)
+    fused = ac.fused("3xtf32")
+    _check_act(ac, fused, "3xtf32", 0.0, 65537, C)
     fused.close()
 
 

@@ -31,27 +31,44 @@ def _module(C, features_dim, pi, activation="tanh", scale=1.6):
     return pol
 
 
+def _check_against_the_module(pol, fused, precision, E, C):
+    obs = _obs(E, C, seed=E)
+    want = pol(obs)
+    got = fused(obs)
+    torch.cuda.synchronize()
+    err = float((got - want).abs().max())
+    assert got.shape == (E, 4) and err < TOL[precision], f"E={E}: |fused - float32 module| = {err}"
+    assert float(got[:, 3].min()) >= 0 and float(got.abs().max()) <= 1
+    assert float(want.std()) > 0.05 and bool((want.abs() < 1).any()), "vacuous comparison: every action clipped"
+
+
+# the last five: an intermediate layer of 192 columns (idle column warps of the 32 x 32 tiles), last layers of 320 and 960
+# columns (the last 256-column pass of head_layer partly filled), pi = () on 64 features, one layer narrower than the
+# features, and the deepest net the kernel holds (8 pi layers: 15 of its 16 layers)
 @pytest.mark.parametrize("precision", ["3xtf32", "tf32"])
 @pytest.mark.parametrize("C,features_dim,pi,activation", [(3, 256, (128, 256, 512), "tanh"), (2, 128, (64,), "tanh"),
                                                           (3, 192, (), "tanh"), (3, 256, (256, 256, 256), "relu"),
-                                                          (1, 64, (256, 1024), "tanh")])
+                                                          (1, 64, (256, 1024), "tanh"), (3, 256, (192, 320), "tanh"),
+                                                          (2, 64, (), "relu"), (1, 128, (64,), "tanh"),
+                                                          (3, 192, (256, 64), "tanh"), (3, 256, (64,) * 7 + (960,), "tanh")])
 def test_fused_policy_matches_the_float32_module(precision, C, features_dim, pi, activation):
     pol = _module(C, features_dim, pi, activation)
     fused = pol.fused(precision)
-    for E in (1, 63, 64, 65, 1000, 4133):                 # ragged last block, single env, several blocks
-        obs = _obs(E, C, seed=E)
-        want = pol(obs)
-        got = fused(obs)
-        torch.cuda.synchronize()
-        err = float((got - want).abs().max())
-        assert got.shape == (E, 4) and err < TOL[precision], f"E={E}: |fused - float32 module| = {err}"
-        assert float(got[:, 3].min()) >= 0 and float(got.abs().max()) <= 1
-        assert float(want.std()) > 0.05 and bool((want.abs() < 1).any()), "vacuous comparison: every action clipped"
+    for E in (1, 63, 64, 65, 127, 128, 1000, 4133):       # ragged last block, single env, whole blocks, several blocks
+        _check_against_the_module(pol, fused, precision, E, C)
     # the same bits on every run, and for any batch a row travels in
     obs = _obs(1000, C, seed=1)
     a, b = fused(obs), fused(obs)
     part = fused({k: v[640:].contiguous() for k, v in obs.items()})
     assert torch.equal(a, b) and torch.equal(a[640:], part)
+    fused.close()
+
+
+def test_fused_policy_on_a_ragged_batch_of_65537():
+    """1,025 blocks, the last with one env: grid-sized row indices."""
+    pol = _module(3, 256, (128, 256, 512))
+    fused = pol.fused("3xtf32")
+    _check_against_the_module(pol, fused, "3xtf32", 65537, 3)
     fused.close()
 
 
