@@ -11,7 +11,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "csrc", "libdronechase_b200.so")
 
-DC_ABI_VERSION = 9
+DC_ABI_VERSION = 10
 DC_QUAD_PARAM_WORDS = 88
 DC_INFO_WORDS = 8
 DC_STATE_QUADS = 13
@@ -129,6 +129,8 @@ def lib():
     L.dc_policy_act.restype = C.c_int
     L.dc_gae.argtypes = [C.c_void_p] * 4 + [C.c_int64, C.c_int64, C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p]
     L.dc_gae.restype = C.c_int
+    L.dc_policy_serve.argtypes = [C.c_void_p] * 4 + [C.c_int32, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]
+    L.dc_policy_serve.restype = C.c_int
     L.dc_policy_destroy.argtypes = [C.c_void_p]
     L.dc_policy_destroy.restype = None
     L.dc_quad_is_builtin.argtypes = [C.c_void_p]
@@ -142,7 +144,7 @@ def lib():
 EXPORTS = ("dc_create", "dc_bind", "dc_reset", "dc_step", "dc_set_actions", "dc_note_graph_replay", "dc_destroy", "dc_last_error", "dc_copy_state",
            "dc_state_bytes", "dc_lidar_project", "dc_lidar_raycast", "dc_launch_count", "dc_host_scatter_sphere", "dc_host_scatter_stack", "dc_scatter_hits",
            "dc_scatter_stack", "dc_abi_info", "dc_host_register", "dc_host_unregister", "dc_mirror_hits", "dc_lw_observe", "dc_quad_is_builtin", "dc_diff_hits", "dc_host_apply_pairs",
-           "dc_policy_create", "dc_policy_forward", "dc_policy_destroy", "dc_policy_create_ac", "dc_policy_act", "dc_gae")
+           "dc_policy_create", "dc_policy_forward", "dc_policy_destroy", "dc_policy_create_ac", "dc_policy_act", "dc_gae", "dc_policy_serve")
 
 
 def check(code: int, what: str):

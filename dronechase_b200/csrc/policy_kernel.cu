@@ -28,6 +28,13 @@
 // in the plain kernel, and evaluated a second time into the stash.  The epilogue draws eps ~ N(0, I) (Box-Muller on one Philox
 // block per env: STREAM_POLICY), raw = mean + exp(log_std) * eps, env_action = clip(raw), log_prob of raw under the diagonal
 // Gaussian; with sample = 0 the action is the plain kernel's clipped mean, bit for bit.
+//
+// Serve mode (policy_serve_kernel, dc_policy_serve): the plain kernel for ONE policy-driven wingman slot of a level4 task
+// (drivers.TaskDrivers).  Row e reads its sphere and inertial vector in place from the [E][n_lw] slabs dc_lw_observe wrote
+// (row strides n_lw * 3 * 338 and n_lw * 15 floats) and its last action from the task's shared [E][4] last_action; the
+// epilogue writes the clipped mean action to lw_actions[e][slot] and, where lw_present[e][slot], to last_action[e] too.
+// Only the addressing and the epilogue differ from the plain kernel: the same bits as dc_policy_forward on contiguous
+// copies of the slot.
 #include "../../include/dronechase_b200.h"
 #include "common.cuh"
 
@@ -95,6 +102,15 @@ struct ACParams {
     float* value;                    // [n]
     uint32_t k0, k1, env_offset, counter;
     int sample;
+};
+
+// The serve kernel's parameters: the plain kernel's with p.lidar / p.inertial / p.actions at slot `slot` of the wingman slabs
+// (row e = p.lidar + e * n_lw * 3 * 338, p.inertial + e * n_lw * 15, p.actions + e * n_lw * 4) and p.last_action = last_action.
+struct ServeParams {
+    Params p;
+    const uint8_t* present;          // lw_present + slot, row stride n_lw
+    float* last_action;              // == p.last_action: advanced in place where present
+    int n_lw;
 };
 
 __device__ __forceinline__ uint32_t tf32_rna(float x) {
@@ -197,9 +213,11 @@ __device__ __forceinline__ void mma_block(float (&acc)[MT][NT][4], ALoad&& aload
 
 // One dense layer over the block's 64 rows: a warp owns 16*MT rows x NT*8 columns, chosen per width so that the 16 warps all
 // have a tile.  Outputs are written after a barrier, so in_off / out_off may overlap.  The input rows are `in` (row stride LDI),
-// the outputs `out` (row stride LDO): act for the plain kernel, the stash for the value branch.
-template <int MT, int NT, bool X3, int LDI = S, int LDO = S>
-__device__ __forceinline__ void dense_layer(const float* in, float* out, const Layer& L, const Params& P, long long env0, int warp, int lane) {
+// the outputs `out` (row stride LDO): act for the plain kernel, the stash for the value branch.  SERVE: the inertial vector
+// of row e is at P.inertial + e * inertial_ld (a wingman slab) instead of e * 15.
+template <int MT, int NT, bool X3, int LDI = S, int LDO = S, bool SERVE = false>
+__device__ __forceinline__ void dense_layer(const float* in, float* out, const Layer& L, const Params& P, long long env0, int warp, int lane,
+                                            long long inertial_ld = 0) {
     constexpr int RG = BM / (16 * MT);
     const int g = lane >> 2, t = lane & 3;
     const int rg = warp % RG, cc = warp / RG;
@@ -224,13 +242,15 @@ __device__ __forceinline__ void dense_layer(const float* in, float* out, const L
         } else {
             const float* src = L.src == SRC_INERTIAL ? P.inertial : P.last_action;
             const int ld = L.K;
+            long long rs = ld;                                  // row stride of the source
+            if constexpr (SERVE) if (L.src == SRC_INERTIAL) rs = inertial_ld;
             mma_block<MT, NT, 8, X3>(acc, [&](int mt, int ks, float (&a)[4]) {
                 const long long ea = env0 + row0 + mt * 16 + g, eb = ea + 8;
                 const int k0 = ks * 8 + t, k1 = k0 + 4;
-                a[0] = (ea < P.n_envs && k0 < ld) ? __ldg(src + ea * ld + k0) : 0.f;
-                a[1] = (eb < P.n_envs && k0 < ld) ? __ldg(src + eb * ld + k0) : 0.f;
-                a[2] = (ea < P.n_envs && k1 < ld) ? __ldg(src + ea * ld + k1) : 0.f;
-                a[3] = (eb < P.n_envs && k1 < ld) ? __ldg(src + eb * ld + k1) : 0.f;
+                a[0] = (ea < P.n_envs && k0 < ld) ? __ldg(src + ea * rs + k0) : 0.f;
+                a[1] = (eb < P.n_envs && k0 < ld) ? __ldg(src + eb * rs + k0) : 0.f;
+                a[2] = (ea < P.n_envs && k1 < ld) ? __ldg(src + ea * rs + k1) : 0.f;
+                a[3] = (eb < P.n_envs && k1 < ld) ? __ldg(src + eb * rs + k1) : 0.f;
             }, L.KS, wh, wl, nt0, lane);
         }
     }
@@ -359,9 +379,9 @@ __device__ __forceinline__ float value_branch(const float* act, float* stash, fl
 }
 
 // tid = threadIdx.x, read by the kernel itself: there it carries the range of __launch_bounds__ (the code of policy_kernel is
-// what it was before the actor-critic mode, instruction for instruction)
-template <bool X3, bool AC>
-__device__ __forceinline__ void policy_body(const Params& P, const ACParams* A, const int tid) {
+// what it was before the actor-critic mode, instruction for instruction).  V: the serve kernel's parameters (SERVE only).
+template <bool X3, bool AC, bool SERVE = false>
+__device__ __forceinline__ void policy_body(const Params& P, const ACParams* A, const int tid, const ServeParams* V = nullptr) {
     extern __shared__ __align__(16) float smem[];
     float* act = smem;
     float* red = smem + BM * S;
@@ -372,7 +392,8 @@ __device__ __forceinline__ void policy_body(const Params& P, const ACParams* A, 
     // ---- conv1: rows (patch, env), 12 patches (2 x 6) of C x 4 x 4, K = 16 C, N = 32; h1 -> act[env][patch*32 + channel]
     {
         const int KS = 2 * P.C;                          // <= 6
-        const size_t env_stride = (size_t)P.C * 338;
+        size_t env_stride = (size_t)P.C * 338;
+        if constexpr (SERVE) env_stride = (size_t)V->n_lw * 3 * 338;     // P.C == 3 (dc_policy_serve)
         const float2* wh = P.w_hi + P.conv1_w;
         const float2* wl = P.w_lo + P.conv1_w;
         for (int pass = 0; pass < 3; ++pass) {
@@ -466,11 +487,13 @@ __device__ __forceinline__ void policy_body(const Params& P, const ACParams* A, 
     }
 
     // ---- the two input MLPs, final_layer, the hidden layers of pi but the last
+    long long inertial_ld = 0;
+    if constexpr (SERVE) inertial_ld = (long long)V->n_lw * 15;
     for (int li = 0; li + 1 < P.n_layers; ++li) {
         const Layer& L = P.layers[li];
-        if (L.N == 128 || L.N == 64) dense_layer<1, 4, X3>(act, act, L, P, env0, warp, lane);
-        else if (DCP_WIDE) dense_layer<2, 4, X3>(act, act, L, P, env0, warp, lane);
-        else dense_layer<1, 8, X3>(act, act, L, P, env0, warp, lane);
+        if (L.N == 128 || L.N == 64) dense_layer<1, 4, X3, S, S, SERVE>(act, act, L, P, env0, warp, lane, inertial_ld);
+        else if (DCP_WIDE) dense_layer<2, 4, X3, S, S, SERVE>(act, act, L, P, env0, warp, lane, inertial_ld);
+        else dense_layer<1, 8, X3, S, S, SERVE>(act, act, L, P, env0, warp, lane, inertial_ld);
         if constexpr (AC) {
             // keep the features for the value branch: the next layer overwrites act only after its first barrier
             if (li == FINAL_LAYER) {
@@ -496,7 +519,17 @@ __device__ __forceinline__ void policy_body(const Params& P, const ACParams* A, 
                 float v = __ldg(P.fp + P.head_b + k);
                 const int n_units = L.N / UNIT;
                 for (int c = 0; c < n_units; ++c) v += red[(c * BM + row) * 4 + k];      // fixed order: the same bits every run
-                P.actions[env * 4 + k] = fminf(fmaxf(v, P.low[k]), P.high[k]);
+                const float a = fminf(fmaxf(v, P.low[k]), P.high[k]);
+                if constexpr (SERVE) {
+                    // last_action is read (P.last_action, first action-MLP layer) and written (here) in the same launch.
+                    // Safe in place: row e reads only last_action[e], and only in that layer; the barriers of every later
+                    // layer separate that read from this write, and the rows of different blocks are disjoint.  So no
+                    // thread reads a word that this launch has already written.
+                    P.actions[env * (4LL * V->n_lw) + k] = a;
+                    if (__ldg(V->present + env * V->n_lw)) V->last_action[env * 4 + k] = a;
+                } else {
+                    P.actions[env * 4 + k] = a;
+                }
             }
         } else {
             float mean = 0.f;                             // the Gaussian's mean: action_net's output, unclipped
@@ -545,6 +578,11 @@ __global__ void __launch_bounds__(THREADS, 1) policy_kernel(const __grid_constan
 template <bool X3>
 __global__ void __launch_bounds__(THREADS, 1) policy_ac_kernel(const __grid_constant__ ACParams A) {
     policy_body<X3, true>(A.p, &A, threadIdx.x);
+}
+
+template <bool X3>
+__global__ void __launch_bounds__(THREADS, 1) policy_serve_kernel(const __grid_constant__ ServeParams V) {
+    policy_body<X3, false, true>(V.p, nullptr, threadIdx.x, &V);
 }
 
 // Weights [N][K] (torch layout) -> B fragments in consumption order, split into a TF32 head and tail.
@@ -718,6 +756,8 @@ int create(const dc_policy_weights* w, const dc_value_weights* v, int device, dc
     P->a.p = p;
     if ((e = cudaFuncSetAttribute(policy_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES)) != cudaSuccess ||
         (e = cudaFuncSetAttribute(policy_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES)) != cudaSuccess ||
+        (e = cudaFuncSetAttribute(policy_serve_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES)) != cudaSuccess ||
+        (e = cudaFuncSetAttribute(policy_serve_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES)) != cudaSuccess ||
         (v && (e = cudaFuncSetAttribute(policy_ac_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_AC_BYTES)) != cudaSuccess) ||
         (v && (e = cudaFuncSetAttribute(policy_ac_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_AC_BYTES)) != cudaSuccess)) {
         cleanup();
@@ -778,6 +818,42 @@ int dc_policy_act(dc_policy* P, const float* lidar, const float* inertial, const
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (precision == 0) policy_ac_kernel<true><<<(unsigned)blocks, THREADS, SMEM_AC_BYTES, st>>>(a);
     else policy_ac_kernel<false><<<(unsigned)blocks, THREADS, SMEM_AC_BYTES, st>>>(a);
+    dc_internal_count_launches(1);
+    DCP_CUDA(cudaGetLastError());
+    return DC_OK;
+}
+
+int dc_policy_serve(dc_policy* P, const float* lw_lidar, const float* lw_inertial, const uint8_t* lw_present, int32_t n_lw,
+                    int32_t slot, int64_t n_envs, float* last_action, float* lw_actions, int32_t precision, void* stream) {
+    using namespace dcp;
+    if (n_lw < 1 || slot < 0 || slot >= n_lw) return pfail(DC_ERR_ARG, "dc_policy_serve: slot must lie in [0, n_lw), n_lw >= 1");
+    if (!lw_lidar || !lw_inertial || !lw_present || !last_action || !lw_actions || n_envs < 0)
+        return pfail(DC_ERR_ARG, "dc_policy_serve: bad argument (null pointer or n_envs < 0)");
+    if (precision != 0 && precision != 1) return pfail(DC_ERR_ARG, "dc_policy_serve: precision must be 0 (3 x TF32, float32-grade) or 1 (TF32)");
+    // every float the kernel touches is a 4-byte access (conv1 too: its A fragments are single words)
+    if ((reinterpret_cast<uintptr_t>(lw_lidar) | reinterpret_cast<uintptr_t>(lw_inertial) | reinterpret_cast<uintptr_t>(last_action) |
+         reinterpret_cast<uintptr_t>(lw_actions)) & 3)
+        return pfail(DC_ERR_ARG, "dc_policy_serve: lw_lidar, lw_inertial, last_action and lw_actions must be 4-byte aligned");
+    if (!P) return pfail(DC_ERR_ARG, "dc_policy_serve: null policy");
+    if (P->p.C != 3)
+        return pfail(DC_ERR_ARG, "dc_policy_serve: the policy reads " + std::to_string(P->p.C) +
+                                 " lidar channels; the wingman sphere lw_lidar has 3 (lidar_channels must be 3)");
+    if (n_envs == 0) return DC_OK;
+    const long long blocks = (n_envs + BM - 1) / BM;
+    if (blocks > 0x7fffffffLL) return pfail(DC_ERR_ARG, "dc_policy_serve: too many envs for one launch");
+    ServeParams v{};
+    v.p = P->p;
+    v.p.lidar = lw_lidar + (size_t)slot * 3 * 338;
+    v.p.inertial = lw_inertial + (size_t)slot * 15;
+    v.p.last_action = last_action;
+    v.p.actions = lw_actions + (size_t)slot * 4;
+    v.p.n_envs = n_envs;
+    v.present = lw_present + slot;
+    v.last_action = last_action;
+    v.n_lw = n_lw;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (precision == 0) policy_serve_kernel<true><<<(unsigned)blocks, THREADS, SMEM_BYTES, st>>>(v);
+    else policy_serve_kernel<false><<<(unsigned)blocks, THREADS, SMEM_BYTES, st>>>(v);
     dc_internal_count_launches(1);
     DCP_CUDA(cudaGetLastError());
     return DC_OK;

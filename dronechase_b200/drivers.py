@@ -7,7 +7,9 @@ The reference serves the armed wingmen one after the other: ``observation = comp
 ``last_action`` is ONE variable of the task, so a wingman sees the action of whichever wingman was served before it (in
 this step, or in the previous one), and ``init_globals`` zeroes it at a reset (:141).  ``TaskDrivers`` does that loop for the
 whole batch on the device: per policy slot one batched policy call over all envs, the shared ``last_action`` advanced only in
-the envs where that wingman was served.
+the envs where that wingman was served.  A slot whose policy is a ``policy.FusedPolicy`` is served by ``FusedPolicy.serve``: one
+kernel launch that reads the slot's rows of the wingman slabs in place, writes ``env.lw_actions[:, slot]`` and advances
+``last_action`` in the same launch, with the same bits as the generic path.
 """
 from __future__ import annotations
 
@@ -36,7 +38,8 @@ class TaskDrivers:
         missing = [j for j in env.cfg.policy_slots if j not in self.policies]
         if missing:
             raise ValueError(f"no policy for the policy-driven wingman slots {missing}")
-        self.last_action = torch.zeros(env.n_envs, 4, dtype=torch.float32, device=env.device)      # the task's shared variable
+        # the task's shared variable: ONE tensor, only ever updated in place (FusedPolicy.serve writes it from its kernel)
+        self.last_action = torch.zeros(env.n_envs, 4, dtype=torch.float32, device=env.device)
 
     def reset(self, mask: Optional[torch.Tensor] = None):
         """Task.init_globals at Env.reset: last_action = zeros."""
@@ -50,11 +53,15 @@ class TaskDrivers:
         env = self.env
         lw = env.lw_observe()
         for j in env.cfg.policy_slots:                    # pursuers are served in slot order
+            policy = self.policies[j]
+            if hasattr(policy, "precision") and hasattr(policy, "refresh"):       # policy.FusedPolicy: one launch, in place
+                policy.serve(lw, j, self.last_action, env.lw_actions)
+                continue
             present = lw["present"][:, j]
             obs = {"lidar": lw["lidar"][:, j], "inertial_data": lw["inertial_data"][:, j], "last_action": self.last_action}
-            a = self.policies[j](obs).to(torch.float32)
+            a = policy(obs).to(torch.float32)
             env.lw_actions[:, j] = a
-            self.last_action = torch.where(present[:, None], a, self.last_action)
+            self.last_action.copy_(torch.where(present[:, None], a, self.last_action))
         return env.lw_actions
 
     def step(self, actions: Optional[torch.Tensor] = None):
@@ -63,5 +70,5 @@ class TaskDrivers:
         self.serve()
         out = self.env.step(actions)
         if self.env._c.auto_reset:
-            self.last_action = torch.where(self.env.done.bool()[:, None], torch.zeros_like(self.last_action), self.last_action)
+            self.last_action.masked_fill_(self.env.done.bool()[:, None], 0.0)
         return out

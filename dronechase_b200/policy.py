@@ -212,7 +212,10 @@ class FusedPolicy:
     (``dc_policy_act``): ``act`` samples actions for PPO rollout collection, ``values`` gives V(s).  Precision matters more
     there: the log-probability error is about ``|eps| * (mean error) / sigma``.  With ``"tf32"`` (5e-3 on the mean) that is
     about 1e-2 in log-probability, a 1 % bias in PPO's first-epoch probability ratio; the default ``"3xtf32"`` keeps it near
-    1e-4."""
+    1e-4.
+
+    ``serve`` runs the same network for one policy-driven wingman slot of a level4 task (``drivers.TaskDrivers``): it reads
+    the wingman slabs of ``env.lw_observe()`` in place and advances the task's shared ``last_action`` in the same launch."""
 
     PRECISIONS = {"3xtf32": 0, "tf32": 1}
 
@@ -295,6 +298,33 @@ class FusedPolicy:
                 self._handle, C.c_void_p(lidar.data_ptr()), C.c_void_p(inertial.data_ptr()), C.c_void_p(last.data_ptr()), E,
                 C.c_void_p(out.data_ptr()), self._prec, C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)), "dc_policy_forward")
         return out
+
+    def serve(self, lw: Dict[str, torch.Tensor], slot: int, last_action: torch.Tensor, lw_actions: torch.Tensor) -> torch.Tensor:
+        """Serve policy-driven wingman ``slot`` of a level4 task in one launch (``dc_policy_serve``).  ``lw`` is the dict
+        ``env.lw_observe()`` returns (``lidar`` [E,n_lw,3,13,26], ``inertial_data`` [E,n_lw,15], ``present`` [E,n_lw]); the
+        kernel reads the slot's rows in place.  ``lw_actions[:, slot]`` ([E,n_lw,4]) receives the clipped mean action of every
+        env, and ``last_action`` ([E,4], the task's shared chain, which is also the policy's input) is overwritten with it
+        where ``present[:, slot]``.  Bit for bit ``self`` on contiguous copies of the slot followed by ``torch.where``.
+        Needs a 3-channel policy.  Returns ``lw_actions``."""
+        C = self._C
+        lidar, inertial, present = lw["lidar"], lw["inertial_data"], lw["present"]
+        for t in (lidar, inertial, last_action, lw_actions):
+            if t.dtype != torch.float32 or not t.is_contiguous() or t.device != self.device:
+                raise ValueError("FusedPolicy.serve: the wingman slabs, last_action and lw_actions must be contiguous float32 "
+                                 "tensors on the policy's device")
+        if present.dtype not in (torch.bool, torch.uint8) or not present.is_contiguous() or present.device != self.device:
+            raise ValueError("FusedPolicy.serve: present must be a contiguous bool or uint8 tensor on the policy's device")
+        E, n_lw = lidar.shape[:2] if lidar.dim() == 5 else (-1, -1)
+        if (tuple(lidar.shape) != (E, n_lw, 3, 13, 26) or tuple(inertial.shape) != (E, n_lw, 15) or tuple(present.shape) != (E, n_lw)
+                or tuple(last_action.shape) != (E, 4) or tuple(lw_actions.shape) != (E, n_lw, 4)):
+            raise ValueError("FusedPolicy.serve: shapes must be lidar [E,n_lw,3,13,26], inertial_data [E,n_lw,15], present [E,n_lw], "
+                             "last_action [E,4], lw_actions [E,n_lw,4]")
+        p = lambda t: C.c_void_p(t.data_ptr())      # noqa: E731
+        with torch.cuda.device(self.device):
+            self._lib.check(self._lib.lib().dc_policy_serve(
+                self._handle, p(lidar), p(inertial), p(present), n_lw, int(slot), E, p(last_action), p(lw_actions), self._prec,
+                C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)), "dc_policy_serve")
+        return lw_actions
 
     def _run_act(self, obs, counter: int, seed: int, env_offset: int, sample: int, env_actions, raw_actions, log_prob, value):
         if not isinstance(self.module, LidarInertialActorCritic):

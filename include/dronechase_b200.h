@@ -39,7 +39,7 @@
 extern "C" {
 #endif
 
-#define DC_ABI_VERSION 9   /* v9: dc_policy_create_ac / dc_policy_act / dc_gae (PPO rollout collection on the device); v8: dc_policy_* (the agent's network as one kernel; dc_config / dc_buffers unchanged); v7: dc_host_register / dc_host_unregister / dc_mirror_hits */
+#define DC_ABI_VERSION 10  /* v10: dc_policy_serve (policy-driven wingmen served by the fused kernel in place); v9: dc_policy_create_ac / dc_policy_act / dc_gae (PPO rollout collection on the device); v8: dc_policy_* (the agent's network as one kernel; dc_config / dc_buffers unchanged); v7: dc_host_register / dc_host_unregister / dc_mirror_hits */
 
 enum dc_status {
     DC_OK = 0,
@@ -351,6 +351,17 @@ int dc_policy_create(const dc_policy_weights* weights, int device, dc_policy** o
  * accumulate (within 5e-3).  Stream-ordered on `stream`; the same bits on every run. */
 int dc_policy_forward(dc_policy* policy, const float* lidar, const float* inertial, const float* last_action, int64_t n_envs,
                       float* actions, int32_t precision, void* stream);
+/* One policy-driven wingman slot of a level4 task (dronechase_b200.drivers.TaskDrivers) in one launch of the same network: row e
+ * reads its sphere at lw_lidar[e][slot] ([E][n_lw][3][13][26]), its inertial vector at lw_inertial[e][slot] ([E][n_lw][15]) --
+ * the slabs dc_lw_observe writes, read in place -- and its last action from the task's shared last_action[e] ([E][4]).  The
+ * clipped mean action goes to lw_actions[e][slot] ([E][n_lw][4]) for every row and, where lw_present[e][slot] ([E][n_lw], 0/1)
+ * is set, to last_action[e] as well (in place: each row reads its own last_action before it is written).  Bit for bit what
+ * dc_policy_forward gives on contiguous copies of the slot.  Works on a policy of dc_policy_create or dc_policy_create_ac with
+ * lidar_channels = 3.  Refuses slot outside [0, n_lw), null pointers, float pointers that are not 4-byte aligned.
+ * Stream-ordered on `stream`; never synchronises. */
+int dc_policy_serve(dc_policy* policy, const float* lw_lidar, const float* lw_inertial, const uint8_t* lw_present,
+                    int32_t n_lw, int32_t slot, int64_t n_envs, float* last_action, float* lw_actions,
+                    int32_t precision, void* stream);
 void dc_policy_destroy(dc_policy* policy);
 
 /* ---- PPO rollout collection on the device: what SB3's OnPolicyAlgorithm.collect_rollouts asks of the policy each step (a sampled
