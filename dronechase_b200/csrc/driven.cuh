@@ -1,4 +1,4 @@
-// dronechase_b200 -- observations of the wingmen that are flown by policies INSIDE the task (stage03 "driven" family, FAM 5).
+// dronechase_b200 -- observations of the wingmen that are flown by policies INSIDE the task (stage03 family FAM_DRIVEN).
 //
 //   Evaluation_Task.compute_lw_observation   evaluation_task.py:283-312   (drive_lw :257-277, drivers of type "nn")
 //   Exp05_vFinal_Task.compute_lw_observation exp05_vFinal_task.py:265-296 (drive_lw_rl_agent :252-260)

@@ -98,6 +98,7 @@ struct dc_sim {
     int D = 0, epb = 0, env_blocks = 0, env_threads = 0, dyn_blocks = 0, parity = 0;
     uint32_t div_m = 0;
     int epw = 32;
+    int fam = dc::FAM_STAGE03;       // the step kernels' family instantiation (stage03.cuh FAM_*), see kernel_family
     bool quad_builtin = false;       // dc_config.quad is the built-in cf2x model (dyn_kernel<..., BUILTIN>)
     int gs = 1;                      // lanes per env in env_kernel's game-logic pass (stage03.cuh EnvCtx GS)
     long long n_slots = 0;
@@ -221,21 +222,31 @@ template <typename A> cudaError_t launch_step(void (*kern)(const A), int grid, i
     return cudaLaunchKernelEx(&cfg, kern, a);
 }
 
+// The dyn_kernel instantiation: motor noise on or off, and (float32 only) the built-in cf2x model folded into the code
+template <typename R, int FAM> auto dyn_kernel_for(bool noise, bool builtin) -> void (*)(const dc::StepArgs<R>) {
+    if constexpr (sizeof(R) == 4 && FAM != dc::FAM_STAGE01) {
+        if (builtin) return noise ? dc::dyn_kernel<R, true, FAM, true> : dc::dyn_kernel<R, false, FAM, true>;
+    }
+    return noise ? dc::dyn_kernel<R, true, FAM> : dc::dyn_kernel<R, false, FAM>;
+}
+
+// The env_kernel instantiation: gs = 8 lanes per env (swarm envs, stage03 only, see create_sim) or one
+template <typename R, int MODE, int FAM> auto env_kernel_for(int gs) -> void (*)(const dc::StepArgs<R>) {
+    if constexpr (FAM == dc::FAM_STAGE03) {
+        if (gs == 8) return dc::env_kernel<R, MODE, FAM, 8>;
+    }
+    return dc::env_kernel<R, MODE, FAM>;
+}
+
 template <typename R, int FAM> int launch_family(dc_sim* s, int mode, const uint8_t* mask, cudaStream_t st) {
     dc::StepArgs<R> a = make_args<R>(s, mask);
-    const bool noise = s->cfg.quad[8] != 0.0;
     if (mode == dc::MODE_RESET) {
         // env_kernel<RESET> rebuilds the whole work list the next dyn_kernel reads
         DC_CUDA(cudaMemsetAsync(s->count + s->parity, 0, sizeof(int32_t), st));
-        if constexpr (FAM == DC_FAMILY_STAGE03) {
-            if (s->gs == 8) dc::env_kernel<R, dc::MODE_RESET, FAM, 8><<<s->env_blocks, s->env_threads, s->smem, st>>>(a);
-            else dc::env_kernel<R, dc::MODE_RESET, FAM><<<s->env_blocks, s->env_threads, s->smem, st>>>(a);
-        } else
-        dc::env_kernel<R, dc::MODE_RESET, FAM><<<s->env_blocks, s->env_threads, s->smem, st>>>(a);
+        DC_CUDA(launch_step(env_kernel_for<R, dc::MODE_RESET, FAM>(s->gs), s->env_blocks, s->env_threads, s->smem, st, false, a));
         g_launches.fetch_add(1, std::memory_order_relaxed);
-        if (s->cfg.family == DC_FAMILY_LEVEL5) launch_stacks<R>(s, a, st);
+        if constexpr (dc::fam_l5(FAM)) launch_stacks<R>(s, a, st);
     } else {
-        const int grid = s->dyn_blocks;
 #ifdef DC_PROFILE_PHASES
         a.tl_slot = g_tl_seq.fetch_add(2) & 255;      // dyn_kernel stamps row tl_slot, env_kernel row tl_slot + 1
         g_tl_sim[a.tl_slot] = g_tl_sim[a.tl_slot + 1] = (int)(((uintptr_t)s >> 4) & 0xffff);
@@ -250,45 +261,42 @@ template <typename R, int FAM> int launch_family(dc_sim* s, int mode, const uint
 #else
         constexpr int pdl = 2;                 // 1: env_kernel only, 2: both step kernels
 #endif
-        if (skip != 1) {
-            bool folded = false;
-            if constexpr (sizeof(R) == 4 && FAM != DC_FAMILY_STAGE01) {
-                if (s->quad_builtin) {                 // the built-in cf2x model: constants folded into the code
-                    folded = true;
-                    if (noise) DC_CUDA(launch_step(dc::dyn_kernel<R, true, FAM, true>, grid, dc::DYN_THREADS, 0, st, pdl >= 2, a));
-                    else DC_CUDA(launch_step(dc::dyn_kernel<R, false, FAM, true>, grid, dc::DYN_THREADS, 0, st, pdl >= 2, a));
-                }
-            }
-            if (folded) {}
-            else if (noise) DC_CUDA(launch_step(dc::dyn_kernel<R, true, FAM>, grid, dc::DYN_THREADS, 0, st, pdl >= 2, a));
-            else DC_CUDA(launch_step(dc::dyn_kernel<R, false, FAM>, grid, dc::DYN_THREADS, 0, st, pdl >= 2, a));
-        }
+        if (skip != 1)
+            DC_CUDA(launch_step(dyn_kernel_for<R, FAM>(s->cfg.quad[8] != 0.0, s->quad_builtin), s->dyn_blocks, dc::DYN_THREADS, 0,
+                                st, pdl >= 2, a));
 #ifdef DC_PROFILE_PHASES
         a.tl_slot += 1;
 #endif
-        if constexpr (FAM == DC_FAMILY_STAGE03) {
-            if (skip == 2) {}
-            else if (s->gs == 8) DC_CUDA(launch_step(dc::env_kernel<R, dc::MODE_STEP, FAM, 8>, s->env_blocks, s->env_threads, s->smem, st, pdl >= 1, a));
-            else DC_CUDA(launch_step(dc::env_kernel<R, dc::MODE_STEP, FAM>, s->env_blocks, s->env_threads, s->smem, st, pdl >= 1, a));
-        } else
-        if (skip != 2) DC_CUDA(launch_step(dc::env_kernel<R, dc::MODE_STEP, FAM>, s->env_blocks, s->env_threads, s->smem, st, pdl >= 1, a));
+        if (skip != 2)
+            DC_CUDA(launch_step(env_kernel_for<R, dc::MODE_STEP, FAM>(s->gs), s->env_blocks, s->env_threads, s->smem, st, pdl >= 1, a));
         g_launches.fetch_add(2, std::memory_order_relaxed);
-        if (s->cfg.family == DC_FAMILY_LEVEL5 && skip == 0) launch_stacks<R>(s, a, st);
+        if constexpr (dc::fam_l5(FAM)) {
+            if (skip == 0) launch_stacks<R>(s, a, st);
+        }
         s->parity ^= 1;
     }
     DC_CUDA(cudaGetLastError());
     return DC_OK;
 }
 
+// The family instantiation of a config's step kernels: dc_config.family, except that the level5 multi-observer /
+// evaluation envs and the stage03 tasks with policy-driven wingmen have kernels of their own
+int kernel_family(const dc_config* cfg, bool driven) {
+    if (cfg->family == DC_FAMILY_LEVEL5 && cfg->level5_multi_obs) return dc::FAM_L5_MULTI;
+    if (cfg->family == DC_FAMILY_STAGE03 && driven) return dc::FAM_DRIVEN;
+    return cfg->family;
+}
+
 template <typename R> int launch(dc_sim* s, int mode, const uint8_t* mask, cudaStream_t st) {
-    switch (s->cfg.family) {
-        case DC_FAMILY_STAGE02: return launch_family<R, DC_FAMILY_STAGE02>(s, mode, mask, st);
-        case DC_FAMILY_STAGE01: return launch_family<R, DC_FAMILY_STAGE01>(s, mode, mask, st);
-        case DC_FAMILY_LEVEL5: return s->cfg.level5_multi_obs ? launch_family<R, 4>(s, mode, mask, st)      // see DC_L5 in stage03.cuh
-                                                              : launch_family<R, DC_FAMILY_LEVEL5>(s, mode, mask, st);
-        default: return s->driven ? launch_family<R, 5>(s, mode, mask, st)      // policy-driven wingmen: own instantiation (stage03.cuh FAM 5)
-                                  : launch_family<R, DC_FAMILY_STAGE03>(s, mode, mask, st);
+    switch (s->fam) {
+        case dc::FAM_STAGE03: return launch_family<R, dc::FAM_STAGE03>(s, mode, mask, st);
+        case dc::FAM_STAGE02: return launch_family<R, dc::FAM_STAGE02>(s, mode, mask, st);
+        case dc::FAM_STAGE01: return launch_family<R, dc::FAM_STAGE01>(s, mode, mask, st);
+        case dc::FAM_L5: return launch_family<R, dc::FAM_L5>(s, mode, mask, st);
+        case dc::FAM_L5_MULTI: return launch_family<R, dc::FAM_L5_MULTI>(s, mode, mask, st);
+        case dc::FAM_DRIVEN: return launch_family<R, dc::FAM_DRIVEN>(s, mode, mask, st);
     }
+    return fail(DC_ERR_ARG, "launch: unknown kernel family");
 }
 
 template <typename R> int copy_drone_state(dc_sim* s, void* host, int to_device) {
@@ -465,6 +473,7 @@ static int create_sim(const dc_config* cfg, int device, dc_sim** out, bool allow
     if (!s) return fail(DC_ERR_ARG, "dc_create: out of host memory");
     s->cfg = *cfg; s->device = device;
     s->driven = driven; s->has_nn = has_nn;
+    s->fam = kernel_family(cfg, driven);
     s->D = cfg->n_lw + cfg->n_lm;
     s->n_slots = (long long)cfg->n_envs * s->D;
     s->rsz = cfg->precision == DC_PRECISION_F64 ? 8 : 4;
@@ -491,7 +500,7 @@ static int create_sim(const dc_config* cfg, int device, dc_sim** out, bool allow
     s->env_blocks = (cfg->n_envs + epb - 1) / epb;
     s->epw = epw;
     // many drones per env (swarm): 8 lanes share an env's game logic, their O(drones) loops strided over the group
-    s->gs = (cfg->family == DC_FAMILY_STAGE03 && !driven && s->D >= 32 && epw <= 4) ? 8 : 1;
+    s->gs = (s->fam == dc::FAM_STAGE03 && s->D >= 32 && epw <= 4) ? 8 : 1;
     s->env_threads = 32 * ((epb + epw - 1) / epw);
     s->div_m = (uint32_t)((1u << 20) / (unsigned)s->D + 1u);
     for (int i = 0; i < epb * s->D; ++i)

@@ -15,11 +15,24 @@
 // every lane of every dynamics warp carries a live drone whatever the wave, and the two kernels can
 // each run at their own register budget / occupancy.
 #pragma once
+#include "../../include/dronechase_b200.h"
 #include "common.cuh"
 #include "lidar.cuh"
 #include "quad_dynamics.cuh"
 
 namespace dc {
+
+// The task families both step kernels are compiled for, their template parameter FAM: every family gets its own
+// specialisation without the other families' branches (each runtime family switch had cost ~6 % of the step).  The first
+// four are dc_config.family.  FAM_L5_MULTI (dc_config.level5_multi_obs: Level5DumbMultiObs, Level52BTEvaluationEnvironment)
+// is split from FAM_L5 so that its extra code costs the hot level5 kernels nothing (it did: + 2.8 % on level5_c1 as
+// run-time branches); FAM_DRIVEN is stage03 with wingmen flown by policies inside the task (driven.cuh).
+enum { FAM_STAGE03 = DC_FAMILY_STAGE03, FAM_STAGE02 = DC_FAMILY_STAGE02, FAM_STAGE01 = DC_FAMILY_STAGE01,
+       FAM_L5 = DC_FAMILY_LEVEL5, FAM_L5_MULTI = 4, FAM_DRIVEN = 5 };
+// the level5 (threatsense) envs: the RL agent is a random wingman, every wingman keeps an IMU record and a LiDAR ring
+__host__ __device__ constexpr bool fam_l5(int f) { return f == FAM_L5 || f == FAM_L5_MULTI; }
+// the families whose munitions come in waves, spawned by env_kernel's spawn pass
+__host__ __device__ constexpr bool fam_waves(int f) { return f == FAM_STAGE03 || f == FAM_DRIVEN || fam_l5(f); }
 
 #ifndef DC_DYN_THREADS
 #define DC_DYN_THREADS 128
@@ -72,7 +85,7 @@ struct TaskParams {
     int l5_eval;             // level5: Level52BTEvaluationEnvironment (dc_config.level5_multi_obs == 2): l5_multi's piloting
                              // and termination, plus no agent draw, no z test, no reward, no observation
     int support_munition;    // stage02: Gun() default of the support wingman
-    // stage03 "driven" instantiation (FAM 5): wingmen flown by policies INSIDE the task -- Evaluation_Task
+    // FAM_DRIVEN: wingmen flown by policies INSIDE the task -- Evaluation_Task
     // (evaluation_task.py:257-277,630-643) and Exp05_vFinal_Task (exp05_vFinal_task.py:252-260)
     int lw_driver[8];        // per wingman slot: DRV_*
     int eval_task;           // Evaluation_Task: no reward, no origin processing, no agent-dead / altitude termination,
@@ -109,7 +122,7 @@ template <typename R> struct SimPtrs {
     int2* stack_prev;        // [E][5*D+1]  hit list of the stacked observation (level5_stack.cuh), -1 terminated
     int32_t* mo_prev_n;      // marked cells of the student stack [E] / of the multi-observer stacks [E][n_lw]
                              // (the agent's own count is the env5 word W5_PREV_N: 32-byte rows)
-    // ---- FAM 5 only ----
+    // ---- FAM_DRIVEN only ----
     int2* lw_desc;           // [E][n_lw][D]  like sphere_desc, for the per-wingman spheres dc_buffers.lw_lidar
     int32_t* lw_kills;       // [E][n_lw]     Evaluation_Task.lw_kills (successful shots of the episode)
 };
@@ -128,7 +141,7 @@ template <typename R> struct StepArgs {
     float* mo_inertial;      // [E][n_lw][15]
     float* mo_last_action;   // [E][n_lw][4]  the wingman's last command = info["teacher_actions"]
     uint8_t* mo_present;     // [E][n_lw]     armed at compute_info time
-    // FAM 5 (policy-driven wingmen): what compute_lw_observation (evaluation_task.py:283-312) hands to the policies
+    // FAM_DRIVEN (policy-driven wingmen): what compute_lw_observation (evaluation_task.py:283-312) hands to the policies
     const float* lw_actions; // [E][n_lw][4]  actions of the policy-driven wingmen for THIS step
     float* lw_lidar;         // [E][n_lw][C][13][26]  sphere of every policy-driven wingman as of the NEXT on_step_start
     float* lw_inertial;      // [E][n_lw][15]
@@ -158,16 +171,9 @@ __device__ __forceinline__ double sq3(double x, double y, double z) { return x *
 // ================================================================================================
 // dyn_kernel
 // ================================================================================================
-// DC_L5: the two level5 instantiations -- 3 = the agent-centred envs (C1, base env), 4 = the multi-observer / evaluation
-// envs (dc_config.level5_multi_obs: Level5DumbMultiObs, Level52BTEvaluationEnvironment).  4 is a separate instantiation so
-// that its extra code costs the hot level5 kernels nothing (it did: + 2.8 % on level5_c1 as run-time branches).
-#define DC_L5(F) ((F) == 3 || (F) == 4)
-// FAM (the task family, TaskParams::family) is a template parameter of both kernels: every family gets its own
-// specialisation without the other families' branches (each runtime family switch had cost ~6 % of the step).
-// BUILTIN (float32 only): the drone model is the built-in cf2x, folded into the code (quad_dynamics.cuh Cf2x).
+// FAM: FAM_* above.  BUILTIN (float32 only): the drone model is the built-in cf2x, folded into the code (quad_dynamics.cuh Cf2x).
 template <typename R, bool NOISE, int FAM, bool BUILTIN = false>
 __global__ void __launch_bounds__(DYN_THREADS, (sizeof(R) == 4 ? DC_DYN_MIN_BLOCKS : 2)) dyn_kernel(const StepArgs<R> A) {
-    constexpr bool S01 = FAM == 2;
     const TaskParams& T = A.t;
     const int par = A.parity;
     // launched with programmatic stream serialisation: nothing is read or written before the previous grid (the
@@ -191,7 +197,7 @@ __global__ void __launch_bounds__(DYN_THREADS, (sizeof(R) == 4 ? DC_DYN_MIN_BLOC
         const V4<R>* pp = A.p.state + s;
 #pragma unroll
         for (int q = 0; q < 10; ++q)
-            if (!(BUILTIN && sizeof(R) == 4 && FAM != 2 && q == 7))
+            if (!(BUILTIN && sizeof(R) == 4 && FAM != FAM_STAGE01 && q == 7))
                 asm volatile("prefetch.global.L2 [%0];" :: "l"(pp + q * stride));
         asm volatile("prefetch.global.L2 [%0];" :: "l"(A.p.env + (long long)env * ENV_WORDS));
     }
@@ -203,12 +209,12 @@ __global__ void __launch_bounds__(DYN_THREADS, (sizeof(R) == 4 ? DC_DYN_MIN_BLOC
     bool driven = false;
     // level5: the RL agent is a random wingman (entities_manager.py:350-383) and guns/tasks read the step of the
     // last AGENT_STEP_BROADCAST, which the id clash with munition 0 can zero (see env_kernel)
-    const int agent_slot = DC_L5(FAM) ? A.p.env5[(long long)env * ENV5_WORDS + W5_AGENT] : 0;
+    const int agent_slot = fam_l5(FAM) ? A.p.env5[(long long)env * ENV5_WORDS + W5_AGENT] : 0;
     // behaviour tree (LoyalWingmanBehaviorTree, loyalwingman_navigator.py:79-86): gun available (or empty) -> chase, else formation
     auto bt_command = [&]() {
         const int ammo = A.p.flagw[s] >> F_AMMO_SHIFT;
-        const int cur_step = DC_L5(FAM) ? A.p.env5[(long long)env * ENV5_WORDS + W5_GUN_STEP]
-                                           : A.p.env[(long long)env * ENV_WORDS + W_STEP];
+        const int cur_step = fam_l5(FAM) ? A.p.env5[(long long)env * ENV5_WORDS + W5_GUN_STEP]
+                                         : A.p.env[(long long)env * ENV_WORDS + W_STEP];
         const bool avail = ammo <= 0 || T.cooldown <= (double)cur_step - (double)own.w;
         double tx = mx, ty = my, tz = mz;
         if (avail) {
@@ -228,8 +234,8 @@ __global__ void __launch_bounds__(DYN_THREADS, (sizeof(R) == 4 ? DC_DYN_MIN_BLOC
         cmd[3] = T.bt_speed;
     };
     bool policy32 = false;                           // the command is the float32 array of an SB3 policy (see below)
-    const int drv = (FAM == 5 && is_lw) ? T.lw_driver[d] : DRV_LEGACY;
-    if (FAM == 5 && drv != DRV_LEGACY) {
+    const int drv = (FAM == FAM_DRIVEN && is_lw) ? T.lw_driver[d] : DRV_LEGACY;
+    if (FAM == FAM_DRIVEN && drv != DRV_LEGACY) {
         if (drv == DRV_BT) { bt_command(); driven = true; }
         else if (drv == DRV_STOP) { cmd[3] = 1.0; driven = true; }
         else {
@@ -243,13 +249,13 @@ __global__ void __launch_bounds__(DYN_THREADS, (sizeof(R) == 4 ? DC_DYN_MIN_BLOC
                 cmd[0] = a.x; cmd[1] = a.y; cmd[2] = a.z; cmd[3] = a.w; driven = true; policy32 = true;
             }
         }
-    } else if (d == agent_slot && !(FAM == 4) && !(FAM == 5 && T.eval_task)) {
+    } else if (d == agent_slot && FAM != FAM_L5_MULTI && !(FAM == FAM_DRIVEN && T.eval_task)) {
         const float4 a = reinterpret_cast<const float4*>(A.actions)[env];
         cmd[0] = a.x; cmd[1] = a.y; cmd[2] = a.z; cmd[3] = a.w; driven = true;
-    } else if (S01) {
+    } else if (FAM == FAM_STAGE01) {
         // stage01: the idle wingman keeps its zero setpoint; the munition holds its spawn point in QuadX
         // mode 7 with setpoint (x, y, yaw 0, z) (level2/components/quadcopter_manager.py:166-179), see below
-    } else if (FAM == 1) {
+    } else if (FAM == FAM_STAGE02) {
         // stage02: munitions are driven with [0,0,0,0.5] (zero direction: hover) and drive_support_pursuers
         // loops over the invaders again, so the support wingman keeps its zero setpoint
         // (level3/components/quadcopter_manager.py:176-205)
@@ -300,7 +306,7 @@ __global__ void __launch_bounds__(DYN_THREADS, (sizeof(R) == 4 ? DC_DYN_MIN_BLOC
         cmd[3] = T.lm_speed; driven = true;
     } else {
         // drive_loyalwingmen: get_armed_pursuers()[1:]; level5: get_allies(armed=True) = every wingman but the agent
-        int armed_before = DC_L5(FAM) ? 1 : 0;
+        int armed_before = fam_l5(FAM) ? 1 : 0;
         for (int j = 0; j < d; ++j) armed_before += (A.p.flagw[b + j] & F_ARMED) ? 1 : 0;
         if (armed_before >= 1) {
             if (T.ally_mode == 1) { cmd[3] = T.ally_stop; }
@@ -308,11 +314,11 @@ __global__ void __launch_bounds__(DYN_THREADS, (sizeof(R) == 4 ? DC_DYN_MIN_BLOC
             driven = true;
         }
     }
-    if (FAM == 4 && is_lw && driven && A.mo_last_action)     // Quadcopter.last_action (quadcopter.py:415-419) = the teacher action
+    if (FAM == FAM_L5_MULTI && is_lw && driven && A.mo_last_action)     // Quadcopter.last_action (quadcopter.py:415-419) = the teacher action
         reinterpret_cast<float4*>(A.mo_last_action)[(long long)env * T.n_lw + d] =
             make_float4((float)cmd[0], (float)cmd[1], (float)cmd[2], (float)cmd[3]);
     R sp[4] = {0, 0, 0, 0};
-    if (FAM == 5 && policy32) {
+    if (FAM == FAM_DRIVEN && policy32) {
         // convert_command_to_setpoint on the float32 array predict() returns: numpy keeps norm, division and product in
         // float32 (quadcopter.py:391-396); the setpoint array itself is float64
         const float cx = (float)cmd[0], cy = (float)cmd[1], cz = (float)cmd[2], cm = (float)cmd[3];
@@ -328,7 +334,7 @@ __global__ void __launch_bounds__(DYN_THREADS, (sizeof(R) == 4 ? DC_DYN_MIN_BLOC
         sp[2] = 0; sp[3] = (R)(cmd[3] * (cmd[2] / dn));
     }
 
-    const bool mode7 = S01 && !is_lw;
+    const bool mode7 = FAM == FAM_STAGE01 && !is_lw;
     if (mode7) {
         const V4<R> f = ld4(A.p.state + 12 * stride + s);           // replace() stored the hold point here
         sp[0] = f.x; sp[1] = f.y; sp[2] = 0; sp[3] = f.z;
@@ -341,12 +347,12 @@ __global__ void __launch_bounds__(DYN_THREADS, (sizeof(R) == 4 ? DC_DYN_MIN_BLOC
     v = ld4(gp + 2 * stride); st.vx = v.x; st.vy = v.y; st.vz = v.z;
     v = ld4(gp + 3 * stride); st.wx = v.x; st.wy = v.y; st.wz = v.z;
     v = ld4(gp + 4 * stride); st.thr[0] = v.x; st.thr[1] = v.y; st.thr[2] = v.z; st.thr[3] = v.w;
-    constexpr int NPID = S01 ? 6 : 5;                               // quad 10 holds the mode-7 words
+    constexpr int NPID = FAM == FAM_STAGE01 ? 6 : 5;                              // quad 10 holds the mode-7 words
     // The folded cf2x model (BUILTIN) has ki = kd = 0 in the angle loop and kd = 0 in the yaw-rate loop: of the 20 mode-6
     // controller words only 11 are ever read -- ang_vel integrators 0..2 and previous errors 3, 4, lin_vel 12..15, z_vel 16, 17.
     // The others are neither loaded nor written back (they keep what the last reset left): 9 registers less across the
     // substep loop and 56 bytes less traffic per drone and direction.
-    constexpr bool PID_DIET = BUILTIN && sizeof(R) == 4 && !S01;
+    constexpr bool PID_DIET = BUILTIN && sizeof(R) == 4 && FAM != FAM_STAGE01;
     if constexpr (PID_DIET) {
 #pragma unroll
         for (int k = 0; k < 24; ++k) st.pid[k] = 0;
@@ -364,7 +370,7 @@ __global__ void __launch_bounds__(DYN_THREADS, (sizeof(R) == 4 ? DC_DYN_MIN_BLOC
     Imu<R> imu;
     const uint32_t env_id = T.env_offset + (uint32_t)env;
     const uint32_t phys0 = (uint32_t)A.p.env[(long long)env * ENV_WORDS + W_PHYS_CTR];
-    if (S01) {
+    if (FAM == FAM_STAGE01) {
         // replace_invader ends with one update_imu/update_control/update_physics outside the stepping loop:
         // PID and motors advance once more and the applied force is still pending at the next
         // stepSimulation, i.e. it adds to the first substep (quadcopter_manager.py:176-179)
@@ -394,8 +400,9 @@ __global__ void __launch_bounds__(DYN_THREADS, (sizeof(R) == 4 ? DC_DYN_MIN_BLOC
     }
     asm volatile("griddepcontrol.launch_dependents;");      // env_kernel's blocks may be placed while the state drains
     st4(A.p.imu[par ^ 1] + s, V4<R>{imu.px, imu.py, imu.pz, own.w});
-    if ((DC_L5(FAM) || FAM == 5) ? is_lw : d == 0) {
-        V4<R>* ag = reinterpret_cast<V4<R>*>(A.p.agent + ((long long)env * T.n_rec + ((DC_L5(FAM) || FAM == 5) ? d : 0)) * AG_WORDS);
+    constexpr bool REC_PER_LW = fam_l5(FAM) || FAM == FAM_DRIVEN;     // an imu record per wingman (TaskParams::n_rec)
+    if (REC_PER_LW ? is_lw : d == 0) {
+        V4<R>* ag = reinterpret_cast<V4<R>*>(A.p.agent + ((long long)env * T.n_rec + (REC_PER_LW ? d : 0)) * AG_WORDS);
         st4(ag, V4<R>{imu.ub, imu.vb, imu.wb, imu.roll});
         st4(ag + 1, V4<R>{imu.pitch, quat_yaw(imu.qx, imu.qy, imu.qz, imu.qw), imu.p, imu.q});
         st4(ag + 2, V4<R>{imu.r, imu.qx, imu.qy, imu.qz});
@@ -505,7 +512,7 @@ template <typename R, int FAM, int GS = 1> struct EnvCtx {
     // next broadcast.
     int agent = 0, gun_step = 0;
     bool registered = false;
-    int32_t* kills = nullptr;        // FAM 5: this env's row of SimPtrs::lw_kills
+    int32_t* kills = nullptr;        // FAM_DRIVEN: this env's row of SimPtrs::lw_kills
     int g = 0;                       // lane within the env's group, and the group's lane mask (GS > 1)
     unsigned gmask = 0xffffffffu;
     __device__ void gsync() const { if (GS > 1) __syncwarp(gmask); }
@@ -524,16 +531,16 @@ template <typename R, int FAM, int GS = 1> struct EnvCtx {
     }
     __device__ EnvCtx(const TaskParams& t, Smem<R>& s, int base, int local_env, uint32_t id, int32_t* words)
         : T(t), S(s), b(base), le(local_env), env_id(id), w(words) {}
-    __device__ int gstep() const { return DC_L5(FAM) ? gun_step : w[W_STEP]; }
+    __device__ int gstep() const { return fam_l5(FAM) ? gun_step : w[W_STEP]; }
     __device__ void broadcast_step() { gun_step = w[W_STEP]; registered = true; }
 
     __device__ void disarm(int d) {                       // Quadcopter.disarm quadcopter.py:461-478
         S.ev[b + d] = (S.ev[b + d] & ~(EV_LIVE | EV_SNAP)) | EV_ZEROED;
-        if (DC_L5(FAM) && d == T.n_lw && registered) { gun_step = 0; registered = false; }
+        if (fam_l5(FAM) && d == T.n_lw && registered) { gun_step = 0; registered = false; }
     }
     __device__ void arm(int d) {                          // Quadcopter.arm quadcopter.py:445-459 (gun.reset())
         S.ev[b + d] = (S.ev[b + d] & ~EV_SNAP) | EV_LIVE | EV_REARMED;
-        S.ammo[b + d] = d >= T.n_lw ? 10 : (FAM == 1 && d > 0) ? T.support_munition : T.munition;
+        S.ammo[b + d] = d >= T.n_lw ? 10 : (FAM == FAM_STAGE02 && d > 0) ? T.support_munition : T.munition;
         S.last[b + d] = (R)(-T.cooldown);
     }
     __device__ void replace(int d, double x, double y, double z) {   // quadcopter.py:433-439
@@ -690,7 +697,7 @@ template <typename R, int FAM, int GS = 1> struct EnvCtx {
     }
     // Env.reset -> Task.on_reset  exp02_vFinal_environment.py:133-151, task :254-273
     __device__ void reset_env(double* lw_init) {
-        if (FAM == 5 && kills) for (int j = 0; j < T.n_lw; ++j) kills[j] = 0;      // on_episode_start evaluation_task.py:360-364
+        if (FAM == FAM_DRIVEN && kills) for (int j = 0; j < T.n_lw; ++j) kills[j] = 0;      // on_episode_start evaluation_task.py:360-364
         w[W_STEP] = 0; w[W_MAX_STEP] = T.max_step;
         w[W_AGENT_KILLS] = w[W_ALLIES_KILLS] = w[W_DEADS] = 0; w[W_BUILDING] = 1;
         set_last_closest(T.dome);
@@ -743,7 +750,7 @@ template <typename R, int FAM, int GS = 1> struct EnvCtx {
             replace(j, p[0], p[1], p[2]);
         }
         w[W_SPAWN_CTR] += 2 * T.n_lw;
-        if (FAM == 4 && T.l5_eval) agent = 0;                            // Teacher_Student=False: no agent is chosen, no draw
+        if (FAM == FAM_L5_MULTI && T.l5_eval) agent = 0;                            // Teacher_Student=False: no agent is chosen, no draw
         else {
             agent = (int)(spawn_u((uint32_t)w[W_SPAWN_CTR]) * T.n_lw);     // entities_manager.py:350-383, randomness as data
             w[W_SPAWN_CTR] += 1;
@@ -841,7 +848,7 @@ __device__ long long g_phase_clk[8192 * 8];
 
 template <typename R, int MODE, int FAM, int GS = 1>
 __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOCKS : 1)) env_kernel(const StepArgs<R> A) {
-    static_assert(GS == 1 || FAM == 0, "lane groups are built for the stage03 family only");
+    static_assert(GS == 1 || FAM == FAM_STAGE03, "lane groups are built for the stage03 family only");
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const TaskParams& T = A.t;
     // Warp-autonomous: warp wi of the block owns the EPW envs [EPW wi, EPW wi + EPW) of the block and their slots
@@ -855,7 +862,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
     const int nenv = min(EPB, T.n_envs - env0);
     const int LE_LO = min((tid >> 5) * A.epw, nenv), LE_HI = min(LE_LO + A.epw, nenv);
     const int S_LO = LE_LO * D, S_HI = LE_HI * D;
-    Smem<R> S = carve_smem<R>(smem_raw, EPB * D, EPB, DC_L5(FAM));
+    Smem<R> S = carve_smem<R>(smem_raw, EPB * D, EPB, fam_l5(FAM));
     const long long slot0 = (long long)env0 * D;
     const long long stride = (long long)T.n_envs * D;
     // MODE_STEP: dyn_kernel wrote this step's imu into imu[parity^1]; MODE_RESET edits the snapshot
@@ -876,7 +883,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
     }
     DC_STAMP(0);
     if (MODE == MODE_STEP) DC_TL_BEGIN(A.tl_slot);
-    constexpr bool STASH_DESC = MODE == MODE_STEP && !DC_L5(FAM);
+    constexpr bool STASH_DESC = MODE == MODE_STEP && !fam_l5(FAM);
     auto env_of = [&](int s) { return (int)(((uint32_t)s * A.div_m) >> 20); };
     {
         constexpr int U = 4;
@@ -890,7 +897,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
                 // Evaluation_Task: the episode goes on after wingman 0 died and the env keeps observing it
                 // (EvaluationEnvironment.compute_observation: get_all_pursuers()[0]): its last imu position / last_fired
                 // live on in the snapshot buffer of the previous step (P5 carries them forward)
-                const bool KEEP0 = FAM == 5 && MODE == MODE_STEP && T.eval_task && ok && !(fwv[u] & F_ARMED) && s - env_of(s) * D == 0;
+                const bool KEEP0 = FAM == FAM_DRIVEN && MODE == MODE_STEP && T.eval_task && ok && !(fwv[u] & F_ARMED) && s - env_of(s) * D == 0;
                 qv[u] = ok ? ld4((KEEP0 ? A.p.imu[A.parity] : imu_g) + slot0 + s) : V4<R>{0, 0, 0, 0};
                 if (STASH_DESC) dv[u] = ok ? *reinterpret_cast<const long long*>(A.p.sphere_desc + slot0 + s) : -1LL;
             }
@@ -902,7 +909,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
                 const bool armed = fw & F_ARMED;
                 S.ammo[s] = fw >> F_AMMO_SHIFT;
                 V4<R> q = qv[u];
-                const bool keep0 = FAM == 5 && MODE == MODE_STEP && T.eval_task && s - env_of(s) * D == 0;
+                const bool keep0 = FAM == FAM_DRIVEN && MODE == MODE_STEP && T.eval_task && s - env_of(s) * D == 0;
                 if (!(armed || keep0 || (MODE == MODE_RESET && (fw & F_OFF)))) q = V4<R>{0, 0, 0, (R)(-T.cooldown)};
                 S.imu[3 * s] = q.x; S.imu[3 * s + 1] = q.y; S.imu[3 * s + 2] = q.z; S.last[s] = q.w;
                 S.ev[s] = MODE == MODE_STEP ? (armed ? (EV_LIVE | EV_OFF | EV_WAS_ARMED | EV_SNAP) : 0)     // on_middle_step: snapshot := armed set
@@ -928,10 +935,10 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
         }
         EnvCtx<R, FAM, GS> C(T, S, b, le, T.env_offset + (uint32_t)env, w);
         if (GS > 1) { C.g = gl; C.gmask = ((1u << GS) - 1u) << (lane & ~(GS - 1)); }
-        if (FAM == 5) C.kills = A.p.lw_kills + (long long)env * T.n_lw;
+        if (FAM == FAM_DRIVEN) C.kills = A.p.lw_kills + (long long)env * T.n_lw;
         double* lw_init = A.p.lw_init + (long long)env * T.n_lw * 3;
-        int32_t* w5 = DC_L5(FAM) ? A.p.env5 + (long long)env * ENV5_WORDS : nullptr;
-        if (DC_L5(FAM)) { C.agent = w5[W5_AGENT]; C.gun_step = w5[W5_GUN_STEP]; C.registered = w5[W5_REGISTERED] != 0; }
+        int32_t* w5 = fam_l5(FAM) ? A.p.env5 + (long long)env * ENV5_WORDS : nullptr;
+        if (fam_l5(FAM)) { C.agent = w5[W5_AGENT]; C.gun_step = w5[W5_GUN_STEP]; C.registered = w5[W5_REGISTERED] != 0; }
         float inertial[15];
         float act[4] = {0.f, 0.f, 0.f, 0.f};
         auto gun_state_of = [&](int as, float* g) {       // Gun.get_state gun.py:101-113
@@ -969,7 +976,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
 #pragma unroll
                 for (int k = 0; k < 4; ++k) { V4<R> t = ld4(agp + k); ag[4 * k] = t.x; ag[4 * k + 1] = t.y; ag[4 * k + 2] = t.z; ag[4 * k + 3] = t.w; }
             }
-            if (!(FAM == 5 && T.eval_task)) {              // EvaluationEnvironment.last_action is never set: zeros
+            if (!(FAM == FAM_DRIVEN && T.eval_task)) {              // EvaluationEnvironment.last_action is never set: zeros
                 const float4 a4 = reinterpret_cast<const float4*>(A.actions)[env];
                 act[0] = a4.x; act[1] = a4.y; act[2] = a4.z; act[3] = a4.w;
             }
@@ -981,7 +988,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
             const double apx = C.pos(C.agent, 0), apy = C.pos(C.agent, 1), apz = C.pos(C.agent, 2);
             double* last_dist = A.p.last_dist + (long long)env * T.n_lm;
             bool caught = false;
-            if (FAM == 2) {
+            if (FAM == FAM_STAGE01) {
                 // ================= stage01: compute_reward / compute_termination (level2 modified_v2 :157-191) =================
                 const int lm = T.n_lw;
                 const double dcur = sqrt(C.dist2(lm, 0));
@@ -996,7 +1003,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
                 done |= norm3(C.pos(lm, 0), C.pos(lm, 1), C.pos(lm, 2)) > T.dome;
                 gun_state(g);
                 C.set_last_closest(dcur);
-            } else if (FAM == 1) {
+            } else if (FAM == FAM_STAGE02) {
                 // ================= stage02: L3Stage1.on_step_middle (level3/components/stages.py:144-179) =================
                 int shots = 0, exploded = 0;
                 C.nearest_all();
@@ -1047,7 +1054,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
                 done |= lw_out > 0;
                 done |= C.count_outside_dome(T.n_lw, D) > 0;
                 done |= n_armed_lw < T.n_lw;
-            } else if (DC_L5(FAM)) {
+            } else if (fam_l5(FAM)) {
                 // ================= level5: Level5C1FusionTask.on_step_middle (level5_c1_fusion_task.py:298-336) =================
                 const int as = C.agent;
                 int agent_shots = 0, ally_shots = 0;
@@ -1075,7 +1082,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
                 w[W_AGENT_KILLS] += agent_shots; w[W_ALLIES_KILLS] += ally_shots; w[W_DEADS] += exploded;
                 for (int i = T.n_lw; i < D; ++i)               // process_invaders_in_origin
                     if (C.off(i) && sq3(C.pos(i, 0), C.pos(i, 1), C.pos(i, 2)) < 0.2 * 0.2) C.disarm(i);
-                if (FAM == 4 && T.l5_eval) reward = 0.0;                   // "EVALUATION TASK DO NOT USES REWARD" (level5_2bt_evaluation_task.py:418-427)
+                if (FAM == FAM_L5_MULTI && T.l5_eval) reward = 0.0;                   // "EVALUATION TASK DO NOT USES REWARD" (level5_2bt_evaluation_task.py:418-427)
                 else if (T.reward == 2) {
                     // Level5FusionTask.compute_reward (level5_fusion_task.py:448-555; allies_dead is never passed)
                     double score, bonus = 0, penalty = 0;
@@ -1143,8 +1150,8 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
                 done |= lw_out > 0;
                 done |= C.count_outside_dome(T.n_lw, D) > 0;
                 done |= !lw_alive;
-                if (FAM != 4) done |= !C.live(as);
-                if (!(FAM == 4 && T.l5_eval)) done |= apz < -5.99;
+                if (FAM != FAM_L5_MULTI) done |= !C.live(as);
+                if (!(FAM == FAM_L5_MULTI && T.l5_eval)) done |= apz < -5.99;
                 gun_state(g);
             } else {
             if (T.reward == 1) {                           // update_building_life (exp02_v2_full_task.py)
@@ -1167,7 +1174,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
                 w[W_HIT_CTR] += 1;
                 if (u < T.fire_p) {
                     C.disarm(tgt); if (j == 0) ++agent_shots; else ++ally_shots;
-                    if (FAM == 5) A.p.lw_kills[(long long)env * T.n_lw + j] += 1;       // Evaluation_Task.lw_kills :491-494
+                    if (FAM == FAM_DRIVEN) A.p.lw_kills[(long long)env * T.n_lw + j] += 1;       // Evaluation_Task.lw_kills :491-494
                 }
             }
             // process_explosion_range_invaders :358-389 (same, now stale, distance matrix)
@@ -1182,7 +1189,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
                 else if (S.ammo[b + j] == 0) ++ally_suicide;
                 else ++exploded;
             }
-            const bool EVAL = FAM == 5 && T.eval_task;     // Evaluation_Task.on_step_middle evaluation_task.py:383-407
+            const bool EVAL = FAM == FAM_DRIVEN && T.eval_task;     // Evaluation_Task.on_step_middle evaluation_task.py:383-407
             if (!EVAL) {
             w[W_AGENT_KILLS] += agent_shots; w[W_ALLIES_KILLS] += ally_shots; w[W_DEADS] += exploded;
             C.gsync();
@@ -1261,7 +1268,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
                 done |= !C.live(0);
                 done |= apz < (T.reward == 1 ? 0.01 : -5.99);
             }
-            if (FAM == 5 && A.lw_info) {                   // compute_info (evaluation_task.py:554-574), between middle and end
+            if (FAM == FAM_DRIVEN && A.lw_info) {                   // compute_info (evaluation_task.py:554-574), between middle and end
                 for (int j = 0; j < T.n_lw; ++j)
                     reinterpret_cast<int4*>(A.lw_info)[(long long)env * T.n_lw + j] =
                         make_int4(A.p.lw_kills[(long long)env * T.n_lw + j], C.live(j) ? 1 : 0, S.ammo[b + j], 0);
@@ -1286,7 +1293,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
             inertial[9] = nrm(ag[AG_P], i_2pi); inertial[10] = nrm(ag[AG_Q], i_2pi); inertial[11] = nrm(ag[AG_R], i_2pi);
             inertial[12] = g[0]; inertial[13] = g[1]; inertial[14] = g[2];
             write_obs = true;
-            if (FAM == 4 && !T.l5_eval) {
+            if (FAM == FAM_L5_MULTI && !T.l5_eval) {
                 // Level5DumbMultiObs.compute_info (level5_dumb_multiobs.py:112-150): inertial + gun vector of every ARMED
                 // wingman, at the point between on_step_middle and on_step_end
                 for (int P = 0; P < T.n_lw; ++P) {
@@ -1311,7 +1318,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
             C.gsync();
             if (C.live(C.agent)) S.envflag[le] |= EF_LIDAR;
 
-            if (FAM == 2) {
+            if (FAM == FAM_STAGE01) {
                 // replace_invader_if_close + update_last_distance (:148-155,193-198)
                 if (caught) {
                     const int lm = T.n_lw;
@@ -1322,7 +1329,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
                     C.set_last_closest(norm3((double)S.newpos[3 * (b + lm)] - apx, (double)S.newpos[3 * (b + lm) + 1] - apy,
                                              (double)S.newpos[3 * (b + lm) + 2] - apz));
                 }
-            } else if (FAM == 1) {
+            } else if (FAM == FAM_STAGE02) {
                 // disarmed munitions reappear at once (stages.py:170-174,370-376); on_step_end: last offsets := current
                 int n_dead = 0;
                 for (int i = T.n_lw; i < D; ++i) n_dead += C.live(i) ? 0 : 1;
@@ -1342,7 +1349,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
                 const double qnan = __longlong_as_double(0x7ff8000000000000LL);
                 for (int i = T.n_lw; i < D; ++i)
                     last_dist[i - T.n_lw] = (C.off(i) && j0 >= 0) ? sqrt(C.dist2(j0, i)) : qnan;
-            } else if (DC_L5(FAM)) {
+            } else if (fam_l5(FAM)) {
                 // Task.on_step_end :338-350 + advance_round :139-152 (setup_round disarms every munition first: the id
                 // clash zeroes the guns' step until the next broadcast)
                 if (!all_over && !lm_alive && lw_alive) {
@@ -1362,7 +1369,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
                     w5[W5_STACK_MODE] = (C.live(C.agent) ? STACK_BUILD : STACK_EMPTY) | (cand << 8);
                     w5[W5_OBS_CALL] += 3;
                 } else {
-                    w5[W5_STACK_MODE] = (FAM == 4 || C.live(C.agent)) ? STACK_BUILD : STACK_KEEP;   // a dead agent's flight state keeps its last stack
+                    w5[W5_STACK_MODE] = (FAM == FAM_L5_MULTI || C.live(C.agent)) ? STACK_BUILD : STACK_KEEP;   // a dead agent's flight state keeps its last stack
                     w5[W5_OBS_CALL] += 1;
                 }
                 S.envflag[le] |= (w[W_STEP] % RING) << 8;     // ring slot of this step for the feature pass
@@ -1384,17 +1391,17 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
                     atomicAdd(A.stats + 4, (double)w[W_ALLIES_KILLS]); atomicAdd(A.stats + 5, (double)w[W_DEADS]);
                     atomicAdd(A.stats + 6, (double)w[W_ROUND]);
                 }
-                if (DC_L5(FAM)) { C.reset_env5(); w5[W5_STACK_MODE] = STACK_EMPTY; w5[W5_OBS_CALL] += T.l5_base ? 3 : 1; S.envflag[le] &= ~EF_LIDAR; }
-                else if (FAM == 2) C.reset_env_stage01(); else if (FAM == 1) C.reset_env_stage02(last_dist); else C.reset_env(lw_init);
+                if (fam_l5(FAM)) { C.reset_env5(); w5[W5_STACK_MODE] = STACK_EMPTY; w5[W5_OBS_CALL] += T.l5_base ? 3 : 1; S.envflag[le] &= ~EF_LIDAR; }
+                else if (FAM == FAM_STAGE01) C.reset_env_stage01(); else if (FAM == FAM_STAGE02) C.reset_env_stage02(last_dist); else C.reset_env(lw_init);
                 // level5 C1 reports agent.last_action, the command the drone keeps across the reset (quadcopter.py:415-419);
                 // the base level5 env reports its own last_action, zeroed by init_globals (level5_envrionment.py:153-155)
-                if (!DC_L5(FAM) || T.l5_base) act[0] = act[1] = act[2] = act[3] = 0.f;
+                if (!fam_l5(FAM) || T.l5_base) act[0] = act[1] = act[2] = act[3] = 0.f;
                 const int ra = 3 * (b + C.agent);
                 inertial[0] = nrm(S.newpos[ra], inv_dome); inertial[1] = nrm(S.newpos[ra + 1], inv_dome);
                 inertial[2] = nrm(S.newpos[ra + 2], inv_dome);
                 for (int k = 3; k < 12; ++k) inertial[k] = 0.f;
                 gun_state(g); inertial[12] = g[0]; inertial[13] = g[1]; inertial[14] = g[2];
-                if (FAM == 4 && !T.l5_eval) write_multi_reset();
+                if (FAM == FAM_L5_MULTI && !T.l5_eval) write_multi_reset();
             }
         } else {
             // ---- MODE_RESET: Env.__init__ on first use, then Env.reset for the masked envs ----
@@ -1403,17 +1410,17 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
             double* last_dist = A.p.last_dist + (long long)env * T.n_lm;
             if (first) {
                 for (int k = 0; k < ENV_WORDS; ++k) w[k] = 0;
-                if (DC_L5(FAM)) {
+                if (fam_l5(FAM)) {
                     for (int k = 0; k < ENV5_WORDS; ++k) w5[k] = 0;
                     w5[W5_LAST_DIST_LO] = 0; w5[W5_LAST_DIST_HI] = 0x7ff80000;     // NaN: last_distance not set yet
                     C.env_init5();
-                } else if (FAM == 2) C.env_init_stage01(); else if (FAM == 1) C.env_init_stage02(last_dist); else C.env_init(lw_init);
+                } else if (FAM == FAM_STAGE01) C.env_init_stage01(); else if (FAM == FAM_STAGE02) C.env_init_stage02(last_dist); else C.env_init(lw_init);
                 S.envflag[le] |= EF_FIRST;                  // first use: start from an empty sphere
             }
-            if (DC_L5(FAM)) w5[W5_STACK_MODE] = STACK_KEEP;
+            if (fam_l5(FAM)) w5[W5_STACK_MODE] = STACK_KEEP;
             if (masked || first) {
-                if (DC_L5(FAM)) { C.reset_env5(); w5[W5_STACK_MODE] = STACK_EMPTY; w5[W5_OBS_CALL] += T.l5_base ? 3 : 1; }
-                else if (FAM == 2) C.reset_env_stage01(); else if (FAM == 1) C.reset_env_stage02(last_dist); else C.reset_env(lw_init);
+                if (fam_l5(FAM)) { C.reset_env5(); w5[W5_STACK_MODE] = STACK_EMPTY; w5[W5_OBS_CALL] += T.l5_base ? 3 : 1; }
+                else if (FAM == FAM_STAGE01) C.reset_env_stage01(); else if (FAM == FAM_STAGE02) C.reset_env_stage02(last_dist); else C.reset_env(lw_init);
                 float g[3]; gun_state(g);
                 const int ra = 3 * (b + C.agent);
                 inertial[0] = nrm(S.newpos[ra], inv_dome); inertial[1] = nrm(S.newpos[ra + 1], inv_dome);
@@ -1421,16 +1428,16 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
                 for (int k = 3; k < 12; ++k) inertial[k] = 0.f;
                 inertial[12] = g[0]; inertial[13] = g[1]; inertial[14] = g[2];
                 write_obs = true;
-                if (FAM == 4 && !T.l5_eval) write_multi_reset();
+                if (FAM == FAM_L5_MULTI && !T.l5_eval) write_multi_reset();
             }
         }
         if (write_obs && lead) {
             float* oi = A.obs_inertial + (long long)env * 15;
             for (int k = 0; k < 15; ++k) oi[k] = inertial[k];
-            if (!(MODE == MODE_RESET && DC_L5(FAM) && !T.l5_base && !(S.envflag[le] & EF_FIRST)))      // level5 C1 reset keeps agent.last_action
+            if (!(MODE == MODE_RESET && fam_l5(FAM) && !T.l5_base && !(S.envflag[le] & EF_FIRST)))      // level5 C1 reset keeps agent.last_action
                 reinterpret_cast<float4*>(A.obs_last_action)[env] = make_float4(act[0], act[1], act[2], act[3]);
         }
-        if (DC_L5(FAM)) { w5[W5_AGENT] = C.agent; w5[W5_GUN_STEP] = C.gun_step; w5[W5_REGISTERED] = C.registered ? 1 : 0; }
+        if (fam_l5(FAM)) { w5[W5_AGENT] = C.agent; w5[W5_GUN_STEP] = C.gun_step; w5[W5_REGISTERED] = C.registered ? 1 : 0; }
         int4* wp = reinterpret_cast<int4*>(A.p.env + (long long)env * ENV_WORDS);
 #pragma unroll
         for (int k = 0; k < 4; ++k) if (lead) wp[k] = make_int4(w[4 * k], w[4 * k + 1], w[4 * k + 2], w[4 * k + 3]);
@@ -1450,7 +1457,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
         if (s < S_HI) {
             const int ev = S.ev[s];
             live = ev & EV_LIVE;
-            if ((FAM == 0 || FAM == 5 || DC_L5(FAM)) && (ev & EV_SPAWNJOB)) {
+            if (fam_waves(FAM) && (ev & EV_SPAWNJOB)) {
                 const int* jp = reinterpret_cast<const int*>(S.newpos + 3 * s);
                 const uint32_t base = (uint32_t)jp[0];
                 const int n = jp[1], i = jp[2];
@@ -1492,7 +1499,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
             A.p.flagw[slot0 + s] = nf;
             if (S.envflag[le] & EF_NAV_RESET) A.p.nav[slot0 + s] = NAV_WAIT;
             // imu position | last_fired of every drone that is in the snapshot or alive
-            if ((ev & (EV_WAS_ARMED | EV_REARMED | EV_OFF)) || live || (FAM == 5 && T.eval_task && s - le * D == 0))
+            if ((ev & (EV_WAS_ARMED | EV_REARMED | EV_OFF)) || live || (FAM == FAM_DRIVEN && T.eval_task && s - le * D == 0))
                 st4(imu_g + slot0 + s, V4<R>{ix, iy, iz, S.last[s]});
         }
     }
@@ -1504,10 +1511,10 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
     if (MODE == MODE_STEP) asm volatile("griddepcontrol.launch_dependents;");     // the next step's dyn_kernel waits for the whole grid
     // ---- P4: projection LiDAR of the agent (slot 0) over the entities alive after engagement --------
     const int ch = T.lidar == 0 ? 3 : 2;
-    const int per_env = (DC_L5(FAM) ? N_STACK * 3 : ch) * N_CELLS;
+    const int per_env = (fam_l5(FAM) ? N_STACK * 3 : ch) * N_CELLS;
     double* s_rn = S.rn;
     int* s_cell = S.cell;
-    if (MODE == MODE_STEP && DC_L5(FAM)) {
+    if (MODE == MODE_STEP && fam_l5(FAM)) {
         // level5: every armed wingman P runs FusedLIDAR.update_data (level5_c1_fusion_environment.py:25-26); what the
         // agent's ring keeps of it -- P's float32 pose and the kept features (r_n, theta, phi float64, type, id) -- goes
         // to ring slot step % 10.  stack_kernel assembles the observation from the ring afterwards.
@@ -1563,10 +1570,10 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
         // 1.0, then the new hits are written -- bit-identical to rebuilding LIDARSpec.empty_sphere() + add_features,
         // at a few dozen bytes per env instead of 4 KB.  When the agent is no longer a publisher nothing is
         // touched: the reference keeps the previous sphere (fused_lidar.py:160-166).
-        // FAM 5, wingman 0 flown by a policy: its FusedLIDAR keeps ONE sphere that the step-start update (lw_obs_kernel,
+        // FAM_DRIVEN, wingman 0 flown by a policy: its FusedLIDAR keeps ONE sphere that the step-start update (lw_obs_kernel,
         // dc_buffers.lw_lidar[:,0], SimPtrs::lw_desc) and this end-of-step update both overwrite.  When this update is
         // skipped (wingman 0 is no publisher any more) the observation shows that object as the step-start update left it.
-        const bool SYNC0 = FAM == 5 && A.lw_lidar && (T.lw_driver[0] == DRV_NN || T.lw_driver[0] == DRV_NN_ALLY);
+        const bool SYNC0 = FAM == FAM_DRIVEN && A.lw_lidar && (T.lw_driver[0] == DRV_NN || T.lw_driver[0] == DRV_NN_ALLY);
         if (!SYNC0) {
             // One pass over the warp's slots: a slot whose entity held a cell of the previous sphere gives it back (cell and
             // remembered-hit record), and the entities that can mark a cell now -- alive after the engagement, not the
@@ -1672,7 +1679,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
             for (int i = lane; i < n_proj; i += 32) {
                 const int s = s_list[i];
                 const int le = env_of(s), b = le * D;
-                const R* ag = A.p.agent + (long long)(env0 + le) * T.n_rec * AG_WORDS;      // record of wingman 0 (n_rec = n_lw in FAM 5)
+                const R* ag = A.p.agent + (long long)(env0 + le) * T.n_rec * AG_WORDS;      // record of wingman 0 (n_rec = n_lw in FAM_DRIVEN)
                 if (T.lidar == 0) {    // float32 snapshot (perception_snapshot.py:91-110)
                     int c; double rn;
                     lidar_cell_fused(2 * T.dome, (double)(float)S.imu[3 * b], (double)(float)S.imu[3 * b + 1],
