@@ -43,6 +43,7 @@
 #include <cstdio>
 #include <new>
 #include <string>
+#include <utility>
 #include <vector>
 
 extern "C" void dc_internal_set_error(const char* msg);
@@ -51,16 +52,7 @@ extern "C" void dc_internal_count_launches(int n);
 namespace dcp {
 
 constexpr int BM = 64, WARPS = 16, THREADS = 32 * WARPS, S = 452, MAX_LAYERS = 16, MAX_CHUNKS = 16;
-#ifndef DCP_WIDE
-#define DCP_WIDE 1                 // 32-row x 32-column warp tiles for the wide layers (a B fragment serves two m-tiles: 20 % fewer
-                                   // operand bytes through L1 per MMA than 16 x 64; 0 = 16 x 64 tiles.  profiles/r2av_variants.txt)
-#endif
-#ifndef DCP_PF_TF32
-#define DCP_PF_TF32 2              // k-steps of B fragments in flight per warp, TF32 mode (3 and 4 measured the same: r2av)
-#endif
-#ifndef DCP_PF_X3
-#define DCP_PF_X3 1                // the same, 3xTF32 mode (head + tail fragments)
-#endif
+constexpr int UNIT = 32;           // columns per partial sum of the head (head_layer<2, 4>: 32-row x 32-column warp tiles)
 constexpr int MAX_UNITS = 32;      // partial sums of the head: one per 32-column unit of the last layer (1024 / 32)
 constexpr int SMEM_BYTES = (BM * S + MAX_UNITS * BM * 4) * 4;
 constexpr int PAD_STEPS = 4;       // k-steps of 8 n-tiles behind the packed weights that the prefetch may touch
@@ -158,7 +150,7 @@ __device__ __forceinline__ void split_a(const float (&a)[4], uint32_t (&hi)[4], 
 template <int MT, int NT, int NTG, bool X3, class ALoad>
 __device__ __forceinline__ void mma_block(float (&acc)[MT][NT][4], ALoad&& aload, int KS, const float2* __restrict__ whi,
                                           const float2* __restrict__ wlo, int nt0, int lane) {
-    constexpr int PF = X3 ? DCP_PF_X3 : DCP_PF_TF32;
+    constexpr int PF = X3 ? 1 : 2;     // 3 and 4 k-steps measured the same as 2 in TF32 mode (profiles/r2av_variants.txt)
     // packed weights: [group of NT n-tiles][k-step][n-tile in group][lane] -- one pointer per operand, immediate offsets
     // (a warp consumes NT n-tiles of a packed group of NTG)
     const float2* ph = whi + (size_t)(nt0 / NTG) * KS * (NTG * 32) + (nt0 % NTG) * 32 + lane;
@@ -336,36 +328,41 @@ __device__ __forceinline__ void head_layer(const float* in, float* red, const La
     }
 }
 
+// A hidden layer with the warp tile for its width: 16 x 32 for 64 and 128 columns, so that the 16 warps all have a tile;
+// 32 x 32 for the wider ones (a B fragment serves two m-tiles: 20 % fewer operand bytes through L1 per MMA than 16 x 64 tiles,
+// profiles/r2av_variants.txt).
+template <bool X3, int LDI, int LDO, bool SERVE = false>
+__device__ __forceinline__ void hidden_layer(const float* in, float* out, const Layer& L, const Params& P, long long env0, int warp,
+                                             int lane, long long inertial_ld = 0) {
+    if (L.N == 128 || L.N == 64) dense_layer<1, 4, X3, LDI, LDO, SERVE>(in, out, L, P, env0, warp, lane, inertial_ld);
+    else dense_layer<2, 4, X3, LDI, LDO, SERVE>(in, out, L, P, env0, warp, lane, inertial_ld);
+}
+
+// Output k of a head for one row: its bias plus head_layer's partial sums of the N-column layer, added in unit order (fixed
+// order: the same bits every run).
+template <int NH>
+__device__ __forceinline__ float head_sum(const float* red, float bias, int N, int row, int k) {
+    float v = bias;
+    const int n_units = N / UNIT;
+    for (int c = 0; c < n_units; ++c) v += red[(c * BM + row) * NH + k];
+    return v;
+}
+
 // The value of each of the block's rows for the actor-critic kernel, returned to the threads (row = tid / 4, any k) of the
 // epilogue; features in the stash (pi != ()) or still to be computed from act (pi == ()); red is free.
 template <bool X3>
 __device__ __forceinline__ float value_branch(const float* act, float* stash, float* red, const Params& P, const ACParams& A,
                                               long long env0, int tid, int warp, int lane) {
-    constexpr int UNIT = DCP_WIDE ? 32 : 64;
-    if (P.n_layers == FINAL_LAYER + 1) {                 // pi == (): the plain kernel never stores the features
-        const Layer& L = P.layers[FINAL_LAYER];
-        if (L.N == 128 || L.N == 64) dense_layer<1, 4, X3, S, SV>(act, stash, L, P, env0, warp, lane);
-        else if (DCP_WIDE) dense_layer<2, 4, X3, S, SV>(act, stash, L, P, env0, warp, lane);
-        else dense_layer<1, 8, X3, S, SV>(act, stash, L, P, env0, warp, lane);
-    }
-    for (int li = 0; li + 1 < A.n_vf; ++li) {
-        const Layer& L = A.vf[li];
-        if (L.N == 128 || L.N == 64) dense_layer<1, 4, X3, SV, SV>(stash, stash, L, P, env0, warp, lane);
-        else if (DCP_WIDE) dense_layer<2, 4, X3, SV, SV>(stash, stash, L, P, env0, warp, lane);
-        else dense_layer<1, 8, X3, SV, SV>(stash, stash, L, P, env0, warp, lane);
-    }
+    if (P.n_layers == FINAL_LAYER + 1)                   // pi == (): the plain kernel never stores the features
+        hidden_layer<X3, S, SV>(act, stash, P.layers[FINAL_LAYER], P, env0, warp, lane);
+    for (int li = 0; li + 1 < A.n_vf; ++li) hidden_layer<X3, SV, SV>(stash, stash, A.vf[li], P, env0, warp, lane);
     const int row = tid >> 2, k = tid & 3;
     float v = 0.f;
     if (A.n_vf > 0) {                                     // the last vf layer, streamed into value_net
         const Layer& L = A.vf[A.n_vf - 1];
-        if (DCP_WIDE) head_layer<2, 4, X3, 1, SV>(stash, red, L, P, A.value_w, warp, lane);
-        else head_layer<1, 8, X3, 1, SV>(stash, red, L, P, A.value_w, warp, lane);
+        head_layer<2, 4, X3, 1, SV>(stash, red, L, P, A.value_w, warp, lane);
         __syncthreads();
-        if (row < BM) {
-            v = __ldg(P.fp + A.value_b);
-            const int n_units = L.N / UNIT;
-            for (int c = 0; c < n_units; ++c) v += red[c * BM + row];              // fixed order
-        }
+        if (row < BM) v = head_sum<1>(red, __ldg(P.fp + A.value_b), L.N, row, 0);
     } else if (row < BM) {                                // vf == (): value_net reads the features; the quad splits the columns
         const int F = P.layers[FINAL_LAYER].N;
         const float* w = P.fp + A.value_w;
@@ -378,10 +375,14 @@ __device__ __forceinline__ float value_branch(const float* act, float* stash, fl
     return v;
 }
 
+enum class Mode { PLAIN, AC, SERVE };
+
 // tid = threadIdx.x, read by the kernel itself: there it carries the range of __launch_bounds__ (the code of policy_kernel is
-// what it was before the actor-critic mode, instruction for instruction).  V: the serve kernel's parameters (SERVE only).
-template <bool X3, bool AC, bool SERVE = false>
-__device__ __forceinline__ void policy_body(const Params& P, const ACParams* A, const int tid, const ServeParams* V = nullptr) {
+// what it was before the actor-critic mode, instruction for instruction).  A: the actor-critic kernel's parameters (Mode::AC
+// only); V: the serve kernel's (Mode::SERVE only).
+template <bool X3, Mode MODE>
+__device__ __forceinline__ void policy_body(const Params& P, const ACParams* A, const ServeParams* V, const int tid) {
+    constexpr bool SERVE = MODE == Mode::SERVE;
     extern __shared__ __align__(16) float smem[];
     float* act = smem;
     float* red = smem + BM * S;
@@ -491,10 +492,8 @@ __device__ __forceinline__ void policy_body(const Params& P, const ACParams* A, 
     if constexpr (SERVE) inertial_ld = (long long)V->n_lw * 15;
     for (int li = 0; li + 1 < P.n_layers; ++li) {
         const Layer& L = P.layers[li];
-        if (L.N == 128 || L.N == 64) dense_layer<1, 4, X3, S, S, SERVE>(act, act, L, P, env0, warp, lane, inertial_ld);
-        else if (DCP_WIDE) dense_layer<2, 4, X3, S, S, SERVE>(act, act, L, P, env0, warp, lane, inertial_ld);
-        else dense_layer<1, 8, X3, S, S, SERVE>(act, act, L, P, env0, warp, lane, inertial_ld);
-        if constexpr (AC) {
+        hidden_layer<X3, S, S, SERVE>(act, act, L, P, env0, warp, lane, inertial_ld);
+        if constexpr (MODE == Mode::AC) {
             // keep the features for the value branch: the next layer overwrites act only after its first barrier
             if (li == FINAL_LAYER) {
                 float* stash = red + MAX_UNITS * BM * 4;
@@ -508,17 +507,13 @@ __device__ __forceinline__ void policy_body(const Params& P, const ACParams* A, 
     // ---- the last hidden layer, streamed into action_net
     {
         const Layer& L = P.layers[P.n_layers - 1];
-        constexpr int UNIT = DCP_WIDE ? 32 : 64;         // columns per partial sum
-        if (DCP_WIDE) head_layer<2, 4, X3>(act, red, L, P, P.head_w, warp, lane);
-        else head_layer<1, 8, X3>(act, red, L, P, P.head_w, warp, lane);
+        head_layer<2, 4, X3>(act, red, L, P, P.head_w, warp, lane);
         __syncthreads();
         const int row = tid >> 2, k = tid & 3;
         const long long env = env0 + row;
-        if constexpr (!AC) {
+        if constexpr (MODE != Mode::AC) {
             if (row < BM && env < E) {
-                float v = __ldg(P.fp + P.head_b + k);
-                const int n_units = L.N / UNIT;
-                for (int c = 0; c < n_units; ++c) v += red[(c * BM + row) * 4 + k];      // fixed order: the same bits every run
+                const float v = head_sum<4>(red, __ldg(P.fp + P.head_b + k), L.N, row, k);
                 const float a = fminf(fmaxf(v, P.low[k]), P.high[k]);
                 if constexpr (SERVE) {
                     // last_action is read (P.last_action, first action-MLP layer) and written (here) in the same launch.
@@ -533,11 +528,7 @@ __device__ __forceinline__ void policy_body(const Params& P, const ACParams* A, 
             }
         } else {
             float mean = 0.f;                             // the Gaussian's mean: action_net's output, unclipped
-            if (row < BM) {
-                mean = __ldg(P.fp + P.head_b + k);
-                const int n_units = L.N / UNIT;
-                for (int c = 0; c < n_units; ++c) mean += red[(c * BM + row) * 4 + k];
-            }
+            if (row < BM) mean = head_sum<4>(red, __ldg(P.fp + P.head_b + k), L.N, row, k);
             __syncthreads();                              // red is free for the value head
             const float value = value_branch<X3>(act, red + MAX_UNITS * BM * 4, red, P, *A, env0, tid, warp, lane);
             if (row < BM) {                               // warps 0-7 whole: the shuffles below see every lane
@@ -572,17 +563,17 @@ __device__ __forceinline__ void policy_body(const Params& P, const ACParams* A, 
 
 template <bool X3>
 __global__ void __launch_bounds__(THREADS, 1) policy_kernel(const __grid_constant__ Params P) {
-    policy_body<X3, false>(P, nullptr, threadIdx.x);
+    policy_body<X3, Mode::PLAIN>(P, nullptr, nullptr, threadIdx.x);
 }
 
 template <bool X3>
 __global__ void __launch_bounds__(THREADS, 1) policy_ac_kernel(const __grid_constant__ ACParams A) {
-    policy_body<X3, true>(A.p, &A, threadIdx.x);
+    policy_body<X3, Mode::AC>(A.p, &A, nullptr, threadIdx.x);
 }
 
 template <bool X3>
 __global__ void __launch_bounds__(THREADS, 1) policy_serve_kernel(const __grid_constant__ ServeParams V) {
-    policy_body<X3, false, true>(V.p, nullptr, threadIdx.x, &V);
+    policy_body<X3, Mode::SERVE>(V.p, nullptr, &V, threadIdx.x);
 }
 
 // Weights [N][K] (torch layout) -> B fragments in consumption order, split into a TF32 head and tail.
@@ -754,16 +745,39 @@ int create(const dc_policy_weights* w, const dc_value_weights* v, int device, dc
     }
     p.w_hi = P->w_hi; p.w_lo = P->w_lo; p.fp = P->fp;
     P->a.p = p;
-    if ((e = cudaFuncSetAttribute(policy_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES)) != cudaSuccess ||
-        (e = cudaFuncSetAttribute(policy_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES)) != cudaSuccess ||
-        (e = cudaFuncSetAttribute(policy_serve_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES)) != cudaSuccess ||
-        (e = cudaFuncSetAttribute(policy_serve_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES)) != cudaSuccess ||
-        (v && (e = cudaFuncSetAttribute(policy_ac_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_AC_BYTES)) != cudaSuccess) ||
-        (v && (e = cudaFuncSetAttribute(policy_ac_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_AC_BYTES)) != cudaSuccess)) {
-        cleanup();
-        return pfail(DC_ERR_CUDA, fn + ": cudaFuncSetAttribute: " + cudaGetErrorString(e));
-    }
+    // the actor-critic kernels last: only a policy made by dc_policy_create_ac launches them
+    const std::pair<const void*, int> smem[] = {
+        {(const void*)policy_kernel<true>, SMEM_BYTES}, {(const void*)policy_kernel<false>, SMEM_BYTES},
+        {(const void*)policy_serve_kernel<true>, SMEM_BYTES}, {(const void*)policy_serve_kernel<false>, SMEM_BYTES},
+        {(const void*)policy_ac_kernel<true>, SMEM_AC_BYTES}, {(const void*)policy_ac_kernel<false>, SMEM_AC_BYTES}};
+    for (int i = 0; i < (v ? 6 : 4); ++i)
+        if ((e = cudaFuncSetAttribute(smem[i].first, cudaFuncAttributeMaxDynamicSharedMemorySize, smem[i].second)) != cudaSuccess) {
+            cleanup();
+            return pfail(DC_ERR_CUDA, fn + ": cudaFuncSetAttribute: " + cudaGetErrorString(e));
+        }
     *out = P;
+    return DC_OK;
+}
+
+// Each entry point checks the precision where it did before its other checks: a call with several bad arguments reports the
+// same one as ever.
+int check_precision(const char* who, int32_t precision) {
+    if (precision == 0 || precision == 1) return DC_OK;
+    return pfail(DC_ERR_ARG, std::string(who) + ": precision must be 0 (3 x TF32, float32-grade) or 1 (TF32)");
+}
+
+// The launch shared by dc_policy_forward, dc_policy_act and dc_policy_serve once their own arguments are checked: kernel x3
+// (precision 0, 3 x TF32) or tf32 (precision 1) over ceil(n_envs / 64) blocks.
+template <class KP>
+int launch(const char* who, void (*x3)(KP), void (*tf32)(KP), const KP& kp, int smem_bytes, int64_t n_envs, int32_t precision,
+           void* stream) {
+    using namespace dcp;
+    if (n_envs == 0) return DC_OK;
+    const long long blocks = (n_envs + BM - 1) / BM;
+    if (blocks > 0x7fffffffLL) return pfail(DC_ERR_ARG, std::string(who) + ": too many envs for one launch");
+    (precision == 0 ? x3 : tf32)<<<(unsigned)blocks, THREADS, smem_bytes, static_cast<cudaStream_t>(stream)>>>(kp);
+    dc_internal_count_launches(1);
+    DCP_CUDA(cudaGetLastError());
     return DC_OK;
 }
 
@@ -784,18 +798,10 @@ int dc_policy_forward(dc_policy* P, const float* lidar, const float* inertial, c
                       float* actions, int32_t precision, void* stream) {
     using namespace dcp;
     if (!P || !lidar || !inertial || !last_action || !actions || n_envs < 0) return pfail(DC_ERR_ARG, "dc_policy_forward: bad argument");
-    if (precision != 0 && precision != 1) return pfail(DC_ERR_ARG, "dc_policy_forward: precision must be 0 (3 x TF32, float32-grade) or 1 (TF32)");
-    if (n_envs == 0) return DC_OK;
-    const long long blocks = (n_envs + BM - 1) / BM;
-    if (blocks > 0x7fffffffLL) return pfail(DC_ERR_ARG, "dc_policy_forward: too many envs for one launch");
+    if (int r = check_precision("dc_policy_forward", precision)) return r;
     Params p = P->p;
     p.lidar = lidar; p.inertial = inertial; p.last_action = last_action; p.actions = actions; p.n_envs = n_envs;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (precision == 0) policy_kernel<true><<<(unsigned)blocks, THREADS, SMEM_BYTES, st>>>(p);
-    else policy_kernel<false><<<(unsigned)blocks, THREADS, SMEM_BYTES, st>>>(p);
-    dc_internal_count_launches(1);
-    DCP_CUDA(cudaGetLastError());
-    return DC_OK;
+    return launch("dc_policy_forward", policy_kernel<true>, policy_kernel<false>, p, SMEM_BYTES, n_envs, precision, stream);
 }
 
 int dc_policy_act(dc_policy* P, const float* lidar, const float* inertial, const float* last_action, int64_t n_envs,
@@ -806,21 +812,13 @@ int dc_policy_act(dc_policy* P, const float* lidar, const float* inertial, const
     if (!P->ac) return pfail(DC_ERR_ARG, "dc_policy_act: the policy was made by dc_policy_create, without a value branch (use dc_policy_create_ac)");
     if (sample != 0 && sample != 1) return pfail(DC_ERR_ARG, "dc_policy_act: sample must be 0 (mean action) or 1");
     if (sample && (!raw_actions || !log_prob)) return pfail(DC_ERR_ARG, "dc_policy_act: sample = 1 needs raw_actions and log_prob");
-    if (precision != 0 && precision != 1) return pfail(DC_ERR_ARG, "dc_policy_act: precision must be 0 (3 x TF32, float32-grade) or 1 (TF32)");
+    if (int r = check_precision("dc_policy_act", precision)) return r;
     if (env_offset < 0 || env_offset + n_envs > (1LL << 32)) return pfail(DC_ERR_ARG, "dc_policy_act: env_offset + n_envs must lie in [0, 2^32]");
-    if (n_envs == 0) return DC_OK;
-    const long long blocks = (n_envs + BM - 1) / BM;
-    if (blocks > 0x7fffffffLL) return pfail(DC_ERR_ARG, "dc_policy_act: too many envs for one launch");
     ACParams a = P->a;
     a.p.lidar = lidar; a.p.inertial = inertial; a.p.last_action = last_action; a.p.actions = env_actions; a.p.n_envs = n_envs;
     a.raw = raw_actions; a.log_prob = log_prob; a.value = value;
     a.k0 = (uint32_t)seed; a.k1 = (uint32_t)(seed >> 32); a.env_offset = (uint32_t)env_offset; a.counter = counter; a.sample = sample;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (precision == 0) policy_ac_kernel<true><<<(unsigned)blocks, THREADS, SMEM_AC_BYTES, st>>>(a);
-    else policy_ac_kernel<false><<<(unsigned)blocks, THREADS, SMEM_AC_BYTES, st>>>(a);
-    dc_internal_count_launches(1);
-    DCP_CUDA(cudaGetLastError());
-    return DC_OK;
+    return launch("dc_policy_act", policy_ac_kernel<true>, policy_ac_kernel<false>, a, SMEM_AC_BYTES, n_envs, precision, stream);
 }
 
 int dc_policy_serve(dc_policy* P, const float* lw_lidar, const float* lw_inertial, const uint8_t* lw_present, int32_t n_lw,
@@ -829,7 +827,7 @@ int dc_policy_serve(dc_policy* P, const float* lw_lidar, const float* lw_inertia
     if (n_lw < 1 || slot < 0 || slot >= n_lw) return pfail(DC_ERR_ARG, "dc_policy_serve: slot must lie in [0, n_lw), n_lw >= 1");
     if (!lw_lidar || !lw_inertial || !lw_present || !last_action || !lw_actions || n_envs < 0)
         return pfail(DC_ERR_ARG, "dc_policy_serve: bad argument (null pointer or n_envs < 0)");
-    if (precision != 0 && precision != 1) return pfail(DC_ERR_ARG, "dc_policy_serve: precision must be 0 (3 x TF32, float32-grade) or 1 (TF32)");
+    if (int r = check_precision("dc_policy_serve", precision)) return r;
     // every float the kernel touches is a 4-byte access (conv1 too: its A fragments are single words)
     if ((reinterpret_cast<uintptr_t>(lw_lidar) | reinterpret_cast<uintptr_t>(lw_inertial) | reinterpret_cast<uintptr_t>(last_action) |
          reinterpret_cast<uintptr_t>(lw_actions)) & 3)
@@ -838,9 +836,6 @@ int dc_policy_serve(dc_policy* P, const float* lw_lidar, const float* lw_inertia
     if (P->p.C != 3)
         return pfail(DC_ERR_ARG, "dc_policy_serve: the policy reads " + std::to_string(P->p.C) +
                                  " lidar channels; the wingman sphere lw_lidar has 3 (lidar_channels must be 3)");
-    if (n_envs == 0) return DC_OK;
-    const long long blocks = (n_envs + BM - 1) / BM;
-    if (blocks > 0x7fffffffLL) return pfail(DC_ERR_ARG, "dc_policy_serve: too many envs for one launch");
     ServeParams v{};
     v.p = P->p;
     v.p.lidar = lw_lidar + (size_t)slot * 3 * 338;
@@ -851,12 +846,7 @@ int dc_policy_serve(dc_policy* P, const float* lw_lidar, const float* lw_inertia
     v.present = lw_present + slot;
     v.last_action = last_action;
     v.n_lw = n_lw;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (precision == 0) policy_serve_kernel<true><<<(unsigned)blocks, THREADS, SMEM_BYTES, st>>>(v);
-    else policy_serve_kernel<false><<<(unsigned)blocks, THREADS, SMEM_BYTES, st>>>(v);
-    dc_internal_count_launches(1);
-    DCP_CUDA(cudaGetLastError());
-    return DC_OK;
+    return launch("dc_policy_serve", policy_serve_kernel<true>, policy_serve_kernel<false>, v, SMEM_BYTES, n_envs, precision, stream);
 }
 
 void dc_policy_destroy(dc_policy* P) {

@@ -277,26 +277,34 @@ class FusedPolicy:
         self._handle, self.device = h, dev
         return self
 
+    def _is_f32(self, *ts: torch.Tensor) -> bool:
+        """Every tensor is contiguous float32 on the policy's device: what the kernels read and write."""
+        return all(t.dtype == torch.float32 and t.is_contiguous() and t.device == self.device for t in ts)
+
+    def _call(self, fn: str, *args):
+        """``fn(handle, *args, precision, stream)`` of the C library on the current stream of the policy's device; tensors in
+        ``args`` are passed as their data pointers."""
+        C = self._C
+        args = [C.c_void_p(a.data_ptr()) if isinstance(a, torch.Tensor) else a for a in args]
+        with torch.cuda.device(self.device):
+            self._lib.check(getattr(self._lib.lib(), fn)(self._handle, *args, self._prec,
+                                                          C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)), fn)
+
     def _check_obs(self, obs: Dict[str, torch.Tensor]):
         lidar, inertial, last = obs["lidar"], obs["inertial_data"], obs["last_action"]
         E = lidar.shape[0]
-        for t in (lidar, inertial, last):
-            if t.dtype != torch.float32 or not t.is_contiguous() or t.device != self.device:
-                raise ValueError("FusedPolicy: observations must be contiguous float32 tensors on the policy's device")
+        if not self._is_f32(lidar, inertial, last):
+            raise ValueError("FusedPolicy: observations must be contiguous float32 tensors on the policy's device")
         if tuple(lidar.shape[1:]) != (self.module.lidar_feature_extractor[0].in_channels, 13, 26) or inertial.numel() != E * 15 \
                 or last.numel() != E * 4:
             raise ValueError("FusedPolicy: observation shapes must be lidar [E,C,13,26], inertial_data [E,15], last_action [E,4]")
         return lidar, inertial, last, E
 
     def __call__(self, obs: Dict[str, torch.Tensor], out: Optional[torch.Tensor] = None) -> torch.Tensor:
-        C = self._C
         lidar, inertial, last, E = self._check_obs(obs)
         if out is None:
             out = torch.empty(E, 4, dtype=torch.float32, device=self.device)
-        with torch.cuda.device(self.device):
-            self._lib.check(self._lib.lib().dc_policy_forward(
-                self._handle, C.c_void_p(lidar.data_ptr()), C.c_void_p(inertial.data_ptr()), C.c_void_p(last.data_ptr()), E,
-                C.c_void_p(out.data_ptr()), self._prec, C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)), "dc_policy_forward")
+        self._call("dc_policy_forward", lidar, inertial, last, E, out)
         return out
 
     def serve(self, lw: Dict[str, torch.Tensor], slot: int, last_action: torch.Tensor, lw_actions: torch.Tensor) -> torch.Tensor:
@@ -306,12 +314,10 @@ class FusedPolicy:
         env, and ``last_action`` ([E,4], the task's shared chain, which is also the policy's input) is overwritten with it
         where ``present[:, slot]``.  Bit for bit ``self`` on contiguous copies of the slot followed by ``torch.where``.
         Needs a 3-channel policy.  Returns ``lw_actions``."""
-        C = self._C
         lidar, inertial, present = lw["lidar"], lw["inertial_data"], lw["present"]
-        for t in (lidar, inertial, last_action, lw_actions):
-            if t.dtype != torch.float32 or not t.is_contiguous() or t.device != self.device:
-                raise ValueError("FusedPolicy.serve: the wingman slabs, last_action and lw_actions must be contiguous float32 "
-                                 "tensors on the policy's device")
+        if not self._is_f32(lidar, inertial, last_action, lw_actions):
+            raise ValueError("FusedPolicy.serve: the wingman slabs, last_action and lw_actions must be contiguous float32 "
+                             "tensors on the policy's device")
         if present.dtype not in (torch.bool, torch.uint8) or not present.is_contiguous() or present.device != self.device:
             raise ValueError("FusedPolicy.serve: present must be a contiguous bool or uint8 tensor on the policy's device")
         E, n_lw = lidar.shape[:2] if lidar.dim() == 5 else (-1, -1)
@@ -319,35 +325,25 @@ class FusedPolicy:
                 or tuple(last_action.shape) != (E, 4) or tuple(lw_actions.shape) != (E, n_lw, 4)):
             raise ValueError("FusedPolicy.serve: shapes must be lidar [E,n_lw,3,13,26], inertial_data [E,n_lw,15], present [E,n_lw], "
                              "last_action [E,4], lw_actions [E,n_lw,4]")
-        p = lambda t: C.c_void_p(t.data_ptr())      # noqa: E731
-        with torch.cuda.device(self.device):
-            self._lib.check(self._lib.lib().dc_policy_serve(
-                self._handle, p(lidar), p(inertial), p(present), n_lw, int(slot), E, p(last_action), p(lw_actions), self._prec,
-                C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)), "dc_policy_serve")
+        self._call("dc_policy_serve", lidar, inertial, present, n_lw, int(slot), E, last_action, lw_actions)
         return lw_actions
 
     def _run_act(self, obs, counter: int, seed: int, env_offset: int, sample: int, env_actions, raw_actions, log_prob, value):
         if not isinstance(self.module, LidarInertialActorCritic):
             raise self._lib.DroneChaseError("FusedPolicy.act / values need a LidarInertialActorCritic module (value branch, log_std)")
-        C = self._C
         lidar, inertial, last, E = self._check_obs(obs)
 
         def buf(t, shape):
             if t is None:
                 return torch.empty(shape, dtype=torch.float32, device=self.device)
-            if t.dtype != torch.float32 or not t.is_contiguous() or t.device != self.device or tuple(t.shape) != shape:
+            if not self._is_f32(t) or tuple(t.shape) != shape:
                 raise ValueError(f"FusedPolicy: outputs must be contiguous float32 tensors of shape {shape} on the policy's device")
             return t
         env_actions, value = buf(env_actions, (E, 4)), buf(value, (E,))
         if sample:
             raw_actions, log_prob = buf(raw_actions, (E, 4)), buf(log_prob, (E,))
-        p = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None      # noqa: E731
-        with torch.cuda.device(self.device):
-            self._lib.check(self._lib.lib().dc_policy_act(
-                self._handle, p(lidar), p(inertial), p(last), E, int(seed) & 0xFFFFFFFFFFFFFFFF, int(env_offset),
-                int(counter) & 0xFFFFFFFF, sample, p(env_actions), p(raw_actions) if sample else None,
-                p(log_prob) if sample else None, p(value), self._prec,
-                C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)), "dc_policy_act")
+        self._call("dc_policy_act", lidar, inertial, last, E, int(seed) & 0xFFFFFFFFFFFFFFFF, int(env_offset), int(counter) & 0xFFFFFFFF,
+                   sample, env_actions, raw_actions if sample else None, log_prob if sample else None, value)
         return env_actions, raw_actions, log_prob, value
 
     def act(self, obs: Dict[str, torch.Tensor], counter: int, *, seed: int = 0, env_offset: int = 0,

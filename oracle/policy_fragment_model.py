@@ -17,6 +17,8 @@ from __future__ import annotations
 import numpy as np
 
 BM, WARPS, S = 64, 16, 452
+SV, MAX_UNITS, FINAL_LAYER = 260, 32, 6                      # stash row stride, head partial sums, layers[6] = final_layer
+RED, STASH = BM * S, BM * S + MAX_UNITS * BM * 4            # offsets of red and the stash in the flat shared memory
 LANE = np.arange(32)
 G, T = LANE >> 2, LANE & 3
 
@@ -64,12 +66,92 @@ def _act(x, act):
     return np.maximum(x, 0) if act == 1 else np.tanh(x) if act == 2 else x
 
 
-def forward(weights: dict, lidar, inertial, last_action, low, high, activation=2):
-    """weights: conv1_w [32][C*16], conv1_b, conv2_w [64][128], conv2_b, inertial_w/b[3], action_w/b[3], final_w/b, pi_w/b lists,
-    head_w [4][N], head_b (float64 arrays in torch layout, convs flattened).  One block of <= 64 envs."""
+def _dense(src, ldi, dst, ldo, W, b, in_off, out_off, a_fn, sel, inputs):
+    """dense_layer<MT, NT, X3, LDI, LDO> as hidden_layer picks the tile: rows of `src` / `dst` (flat shared-memory arrays) at
+    stride ldi / ldo; sel 1 / 2 reads the rows of inputs[sel] (inertial vector / last action) instead."""
+    N, K = W.shape
+    KS, w = (K + 7) // 8, pack(W)
+    MT, NT = (1, 4) if N in (128, 64) else (2, 4)              # 16 x 32 warp tiles for 64 and 128 columns, 32 x 32 otherwise
+    RG = BM // (16 * MT)
+    results = {}
+    for warp in range(WARPS):
+        rg, cc = warp % RG, warp // RG
+        row0, nt0 = rg * 16 * MT, cc * NT
+        if nt0 * 8 >= N:
+            continue
+
+        def aload(mt, ks, row0=row0):
+            ra, rb = row0 + mt * 16 + G, row0 + mt * 16 + G + 8
+            k0, k1 = ks * 8 + T, ks * 8 + T + 4
+            if sel == 0:
+                return np.stack([src[ra * ldi + in_off + k0], src[rb * ldi + in_off + k0], src[ra * ldi + in_off + k1],
+                                 src[rb * ldi + in_off + k1]], axis=1)
+            x = inputs[sel]
+            a = np.zeros((32, 4))
+            for i, (rows, k) in enumerate(((ra, k0), (rb, k0), (ra, k1), (rb, k1))):
+                ok = (rows < len(x)) & (k < K)
+                a[ok, i] = x[rows[ok], k[ok]]
+            return a
+        results[warp] = (mma_block(MT, NT, aload, KS, w, nt0), row0, nt0)
+    for warp, (acc, row0, nt0) in results.items():            # after the barrier
+        for mt in range(MT):
+            for j in range(NT):
+                col = (nt0 + j) * 8 + 2 * T
+                r = row0 + mt * 16 + G
+                dst[r * ldo + out_off + col] = _act(acc[mt, j][:, 0] + b[col], a_fn)
+                dst[r * ldo + out_off + col + 1] = _act(acc[mt, j][:, 1] + b[col + 1], a_fn)
+                dst[(r + 8) * ldo + out_off + col] = _act(acc[mt, j][:, 2] + b[col], a_fn)
+                dst[(r + 8) * ldo + out_off + col + 1] = _act(acc[mt, j][:, 3] + b[col + 1], a_fn)
+
+
+def _head(src, ld, W, b, in_off, a_fn, hw, red):
+    """head_layer<2, 4, X3, NH, LD> + head_sum<NH>: the last hidden layer streamed into the NH = len(hw) outputs, partial sums
+    into red[unit][row][k] (a flat view of the kernel's red array), then added over the units.  Returns [BM][NH], no bias."""
+    N, K = W.shape
+    NH = hw.shape[0]
+    KS, w = (K + 7) // 8, pack(W)
+    MT, NT, RG = 2, 4, 2                                       # units of 32 columns, 8 per pass
+    CP = WARPS // RG
+    n_units = N // (NT * 8)
+    for p4 in range((n_units + CP - 1) // CP):
+        for warp in range(WARPS):
+            rg, cc = warp % RG, warp // RG
+            unit, row0 = p4 * CP + cc, rg * 16 * MT
+            if unit >= n_units:
+                continue
+
+            def aload(mt, ks, row0=row0):
+                ra = row0 + mt * 16 + G
+                k0 = in_off + ks * 8 + T
+                return np.stack([src[ra * ld + k0], src[(ra + 8) * ld + k0], src[ra * ld + k0 + 4], src[(ra + 8) * ld + k0 + 4]], axis=1)
+            acc = mma_block(MT, NT, aload, KS, w, unit * NT)
+            for mt in range(MT):
+                part = np.zeros((2, 32, NH))
+                for j in range(NT):
+                    col = (unit * NT + j) * 8 + 2 * T
+                    h = [_act(acc[mt, j][:, 0] + b[col], a_fn), _act(acc[mt, j][:, 1] + b[col + 1], a_fn),
+                         _act(acc[mt, j][:, 2] + b[col], a_fn), _act(acc[mt, j][:, 3] + b[col + 1], a_fn)]
+                    for k in range(NH):
+                        part[0, :, k] += h[0] * hw[k, col] + h[1] * hw[k, col + 1]
+                        part[1, :, k] += h[2] * hw[k, col] + h[3] * hw[k, col + 1]
+                for hh in range(2):
+                    quad = part[hh].reshape(8, 4, NH).sum(axis=1)           # the two shfl_xor steps: sum over t
+                    rows = row0 + mt * 16 + hh * 8 + np.arange(8)
+                    for k in range(NH):
+                        red[(unit * BM + rows) * NH + k] = quad[:, k]
+    return red[:n_units * BM * NH].reshape(n_units, BM, NH).sum(axis=0)
+
+
+def _trunk(weights: dict, lidar, inertial, last_action, activation=2, stash=False):
+    """conv1, conv2 and every dense layer but the last hidden one, in place in act, over one block of <= 64 envs.  The
+    shared memory is ONE flat array act | red | stash (the actor-critic kernel's layout; the plain kernel stops after red),
+    filled with NaN so that a read at a wrong row stride or base shows up.  stash: copy the features (final_layer's output)
+    into the stash at row stride SV, as the actor-critic kernel does.  Returns (smem, layers, inputs): layers are
+    (W, b, in_off, out_off, activation, source) of every dense layer, the last one included; inputs the arrays of sources 1, 2."""
     E, C = lidar.shape[0], lidar.shape[1]
     lid = lidar.reshape(E, -1)
-    act = np.zeros((BM, S))
+    smem = np.full(STASH + BM * SV, np.nan)
+    act = smem[:RED].reshape(BM, S)
     # ---- conv1
     w1, KS1 = pack(weights["conv1_w"], ntg=4), 2 * C
     for warp in range(WARPS):
@@ -122,69 +204,20 @@ def forward(weights: dict, lidar, inertial, last_action, low, high, activation=2
     layers.append((weights["final_w"], weights["final_b"], 0, 0, 1, 0))
     for W, b in zip(weights["pi_w"], weights["pi_b"]):
         layers.append((W, b, 0, 0, activation, 0))
-    for W, b, in_off, out_off, a_fn, src in layers[:-1]:
-        N, K = W.shape
-        KS, w = (K + 7) // 8, pack(W)
-        MT, NT = (1, 4) if N in (128, 64) else (2, 4)          # DCP_WIDE = 1: 32 x 32 warp tiles for the wide layers
-        RG = BM // (16 * MT)
-        results = {}
-        for warp in range(WARPS):
-            rg, cc = warp % RG, warp // RG
-            row0, nt0 = rg * 16 * MT, cc * NT
-            if nt0 * 8 >= N:
-                continue
+    inputs = {1: inertial, 2: last_action}
+    for li, layer in enumerate(layers[:-1]):
+        _dense(smem, S, smem, S, *layer, inputs)
+        if stash and li == FINAL_LAYER:                        # the features -> the stash
+            F = layer[0].shape[0]
+            for r in range(BM):
+                smem[STASH + r * SV:STASH + r * SV + F] = smem[r * S:r * S + F]
+    return smem, layers, inputs
 
-            def aload(mt, ks, row0=row0):
-                ra, rb = row0 + mt * 16 + G, row0 + mt * 16 + G + 8
-                k0, k1 = ks * 8 + T, ks * 8 + T + 4
-                if src == 0:
-                    return np.stack([act[ra, in_off + k0], act[rb, in_off + k0], act[ra, in_off + k1], act[rb, in_off + k1]], axis=1)
-                x = inertial if src == 1 else last_action
-                a = np.zeros((32, 4))
-                for i, (rows, k) in enumerate(((ra, k0), (rb, k0), (ra, k1), (rb, k1))):
-                    ok = (rows < E) & (k < K)
-                    a[ok, i] = x[rows[ok], k[ok]]
-                return a
-            results[warp] = (mma_block(MT, NT, aload, KS, w, nt0), row0, nt0, MT)
-        for warp, (acc, row0, nt0, MT) in results.items():
-            for mt in range(MT):
-                for j in range(NT):
-                    col = (nt0 + j) * 8 + 2 * T
-                    r = row0 + mt * 16 + G
-                    act[r, out_off + col] = _act(acc[mt, j][:, 0] + b[col], a_fn); act[r, out_off + col + 1] = _act(acc[mt, j][:, 1] + b[col + 1], a_fn)
-                    act[r + 8, out_off + col] = _act(acc[mt, j][:, 2] + b[col], a_fn); act[r + 8, out_off + col + 1] = _act(acc[mt, j][:, 3] + b[col + 1], a_fn)
-    # ---- last layer + head
+
+def forward(weights: dict, lidar, inertial, last_action, low, high, activation=2):
+    """weights: conv1_w [32][C*16], conv1_b, conv2_w [64][128], conv2_b, inertial_w/b[3], action_w/b[3], final_w/b, pi_w/b lists,
+    head_w [4][N], head_b (float64 arrays in torch layout, convs flattened).  One block of <= 64 envs."""
+    smem, layers, _ = _trunk(weights, lidar, inertial, last_action, activation)
     W, b, in_off, _, a_fn, _ = layers[-1]
-    N, K = W.shape
-    KS, w = (K + 7) // 8, pack(W)
-    MT, NT, RG = 2, 4, 2                                       # head_layer<2, 4>: units of 32 columns, 8 per pass
-    CP = WARPS // RG
-    n_units = N // (NT * 8)
-    red = np.zeros((n_units, BM, 4))
-    hw = weights["head_w"]
-    for p4 in range((n_units + CP - 1) // CP):
-        for warp in range(WARPS):
-            rg, cc = warp % RG, warp // RG
-            unit, row0 = p4 * CP + cc, rg * 16 * MT
-            if unit >= n_units:
-                continue
-
-            def aload(mt, ks, row0=row0):
-                ra = row0 + mt * 16 + G
-                k0 = in_off + ks * 8 + T
-                return np.stack([act[ra, k0], act[ra + 8, k0], act[ra, k0 + 4], act[ra + 8, k0 + 4]], axis=1)
-            acc = mma_block(MT, NT, aload, KS, w, unit * NT)
-            for mt in range(MT):
-                part = np.zeros((2, 32, 4))
-                for j in range(NT):
-                    col = (unit * NT + j) * 8 + 2 * T
-                    h = [_act(acc[mt, j][:, 0] + b[col], a_fn), _act(acc[mt, j][:, 1] + b[col + 1], a_fn),
-                         _act(acc[mt, j][:, 2] + b[col], a_fn), _act(acc[mt, j][:, 3] + b[col + 1], a_fn)]
-                    for k in range(4):
-                        part[0, :, k] += h[0] * hw[k, col] + h[1] * hw[k, col + 1]
-                        part[1, :, k] += h[2] * hw[k, col] + h[3] * hw[k, col + 1]
-                for hh in range(2):
-                    quad = part[hh].reshape(8, 4, 4).sum(axis=1)           # the two shfl_xor steps: sum over t
-                    red[unit, row0 + mt * 16 + hh * 8 + np.arange(8)] = quad
-    out = weights["head_b"][None, :] + red.sum(axis=0)
-    return np.clip(out, low, high)[:E]
+    out = weights["head_b"][None, :] + _head(smem, S, W, b, in_off, a_fn, weights["head_w"], smem[RED:STASH])
+    return np.clip(out, low, high)[:lidar.shape[0]]
