@@ -151,6 +151,7 @@ template <typename R> struct StepArgs {
     int epb;                 // envs per block of env_kernel
     int epw;                 // envs per warp of env_kernel (<= 32)
     uint32_t div_m;          // slot / D == (slot * div_m) >> 20 for every slot index of a block (checked by dc_create)
+    __device__ int env_of(int s) const { return (int)(((uint32_t)s * div_m) >> 20); }     // block slot -> block env
     int tl_slot;             // profiling builds (DC_PROFILE_PHASES): row of g_tl this launch stamps
     alignas(16) uint32_t rk[20];   // Philox round keys of (t.k0, t.k1) for philox4x32_10_rk (dyn_kernel's motor noise)
 };
@@ -505,6 +506,7 @@ template <typename R, int FAM, int GS = 1> struct EnvCtx {
     int b, le;
     uint32_t env_id;         // global env index (Philox counter word)
     int32_t* w;              // env scalar words (local copy)
+    double inv_dome;         // 1 / dome radius: the position scale of normalize_inertial_data
     // level5: Gun.current_step == Task.current_step (gun.py:44-47, level5_c1_fusion_task.py:74-76).  The env
     // broadcasts the step as publisher 0 (level5_envrionment.py:276-281) and the first munition is body 0 (spawned
     // before the ground plane), so every disarm of that munition makes MessageHub.terminate(0) re-broadcast
@@ -512,6 +514,7 @@ template <typename R, int FAM, int GS = 1> struct EnvCtx {
     // next broadcast.
     int agent = 0, gun_step = 0;
     bool registered = false;
+    int32_t* w5 = nullptr;           // level5: this env's row of SimPtrs::env5
     int32_t* kills = nullptr;        // FAM_DRIVEN: this env's row of SimPtrs::lw_kills
     int g = 0;                       // lane within the env's group, and the group's lane mask (GS > 1)
     unsigned gmask = 0xffffffffu;
@@ -530,7 +533,7 @@ template <typename R, int FAM, int GS = 1> struct EnvCtx {
         }
     }
     __device__ EnvCtx(const TaskParams& t, Smem<R>& s, int base, int local_env, uint32_t id, int32_t* words)
-        : T(t), S(s), b(base), le(local_env), env_id(id), w(words) {}
+        : T(t), S(s), b(base), le(local_env), env_id(id), w(words), inv_dome(1.0 / t.dome) {}
     __device__ int gstep() const { return fam_l5(FAM) ? gun_step : w[W_STEP]; }
     __device__ void broadcast_step() { gun_step = w[W_STEP]; registered = true; }
 
@@ -581,10 +584,13 @@ template <typename R, int FAM, int GS = 1> struct EnvCtx {
         replace(lm, p[0], p[1], p[2]);
         S.ev[b + lm] |= (S.ev[b + lm] & EV_PENDING) ? EV_PENDING2 : EV_PENDING;   // caught on the terminal step: two owed
     }
-    __device__ void reset_env_stage01() {                 // pyflyt_level2_environment_modified_v2.py:70-104
+    __device__ void reset_words() {                       // the episode counters of Env.reset
         w[W_STEP] = 0; w[W_MAX_STEP] = T.max_step;
         w[W_AGENT_KILLS] = w[W_ALLIES_KILLS] = w[W_DEADS] = 0; w[W_BUILDING] = 1;
         w[W_EP_RETURN] = __float_as_int(0.0f); w[W_EP_STEPS] = 0;
+    }
+    __device__ void reset_env_stage01() {                 // pyflyt_level2_environment_modified_v2.py:70-104
+        reset_words();
         const int lm = T.n_lw;
         double p[3];
         u3(p); replace_invader_stage01(lm, p);
@@ -616,28 +622,24 @@ template <typename R, int FAM, int GS = 1> struct EnvCtx {
                                  (double)S.newpos[3 * a + 2] - (double)S.newpos[3 * c + 2]);
         }
     }
-    __device__ void env_init_stage02(double* last_dist) {  // stages.py:96-100,378-397
+    // stage02 placement: munitions on r in U(r0, r1), wingmen on r in U(1, 1), then Stage.on_episode_start
+    __device__ void place_stage02(double r0, double r1, double* last_dist) {
         uint32_t base = (uint32_t)w[W_SPAWN_CTR];
-        for (int i = 0; i < T.n_lm; ++i) { double p[3]; gen3(base, T.n_lm, i, 2.0, 0.0, p); replace(T.n_lw + i, p[0], p[1], p[2]); }
+        for (int i = 0; i < T.n_lm; ++i) { double p[3]; gen3(base, T.n_lm, i, r0, r1, p); replace(T.n_lw + i, p[0], p[1], p[2]); }
         w[W_SPAWN_CTR] += 3 * T.n_lm;
         base = (uint32_t)w[W_SPAWN_CTR];
         for (int j = 0; j < T.n_lw; ++j) { double p[3]; gen3(base, T.n_lw, j, 1.0, 0.0, p); replace(j, p[0], p[1], p[2]); }
         w[W_SPAWN_CTR] += 3 * T.n_lw;
         episode_start_stage02(last_dist);
+    }
+    __device__ void env_init_stage02(double* last_dist) {  // stages.py:96-100,378-397
+        place_stage02(2.0, 0.0, last_dist);
         w[W_INIT] = 1;
     }
     __device__ void reset_env_stage02(double* last_dist) { // stages.py:102-135
-        w[W_STEP] = 0; w[W_MAX_STEP] = T.max_step;
-        w[W_AGENT_KILLS] = w[W_ALLIES_KILLS] = w[W_DEADS] = 0; w[W_BUILDING] = 1;
-        w[W_EP_RETURN] = __float_as_int(0.0f); w[W_EP_STEPS] = 0;
+        reset_words();
         for (int d = 0; d < T.D; ++d) disarm(d);
-        uint32_t base = (uint32_t)w[W_SPAWN_CTR];
-        for (int i = 0; i < T.n_lm; ++i) { double p[3]; gen3(base, T.n_lm, i, T.respawn_r0, T.respawn_r1, p); replace(T.n_lw + i, p[0], p[1], p[2]); }
-        w[W_SPAWN_CTR] += 3 * T.n_lm;
-        base = (uint32_t)w[W_SPAWN_CTR];
-        for (int j = 0; j < T.n_lw; ++j) { double p[3]; gen3(base, T.n_lw, j, 1.0, 0.0, p); replace(j, p[0], p[1], p[2]); }
-        w[W_SPAWN_CTR] += 3 * T.n_lw;
-        episode_start_stage02(last_dist);
+        place_stage02(T.respawn_r0, T.respawn_r1, last_dist);
     }
     __device__ void setup_round(int k) {                  // exp02_vFinal_task.py:179-195
         for (int i = g; i < T.n_lm; i += GS) disarm(T.n_lw + i);
@@ -650,6 +652,14 @@ template <typename R, int FAM, int GS = 1> struct EnvCtx {
         gsync();
         w[W_SPAWN_CTR] += 2 * k;
     }
+    // advance_round (stage03 :154-174, level5 :139-152): the next wave once the munitions of this one are gone
+    __device__ void advance_round() {
+        const int last = fam_l5(FAM) ? T.max_rounds : T.n_lm;
+        w[W_ROUND] += (w[W_ROUND] < last) ? 1 : last;
+        if (fam_l5(FAM)) setup_round5(w[W_ROUND]); else setup_round(w[W_ROUND]);
+        refresh_offsets();
+        S.envflag[le] |= EF_NAV_RESET;
+    }
     __device__ void refresh_offsets() {                   // OffsetHandler.on_episode_start: snapshot := live set
         gsync();
         for (int d = g; d < T.D; d += GS) {
@@ -658,22 +668,24 @@ template <typename R, int FAM, int GS = 1> struct EnvCtx {
         }
         gsync();
     }
-    __device__ void episode_start(double* lw_init) {      // exp02_vFinal_task.py:258-267
+    __device__ void episode_start(double* lw_init) {      // exp02_vFinal_task.py:258-267, level5 :262-273
         w[W_ROUND] = T.initial_round;
-        setup_round(T.initial_round);
+        if (fam_l5(FAM)) setup_round5(T.initial_round); else setup_round(T.initial_round);
         for (int j = g; j < T.n_lw; j += GS) arm(j);
         gsync();
+        const bool fixed = !fam_l5(FAM) && T.fixed_lw_spawn;
         const uint32_t base = (uint32_t)w[W_SPAWN_CTR];
         for (int j = g; j < T.n_lw; j += GS) {
             double p[3];
-            if (T.fixed_lw_spawn) { p[0] = lw_init[3 * j]; p[1] = lw_init[3 * j + 1]; p[2] = lw_init[3 * j + 2]; }
+            if (fixed) { p[0] = lw_init[3 * j]; p[1] = lw_init[3 * j + 1]; p[2] = lw_init[3 * j + 2]; }
             else gen_position(base, T.n_lw, j, T.lw_spawn, p);
             replace(j, p[0], p[1], p[2]);
         }
         gsync();
-        if (!T.fixed_lw_spawn) w[W_SPAWN_CTR] += 2 * T.n_lw;
+        if (!fixed) w[W_SPAWN_CTR] += 2 * T.n_lw;
     }
     // Env.__init__: Task.on_env_init + on_episode_start  exp02_vFinal_environment.py:62-63, task :248-252,622-646
+    // (level5: on_env_init :253-257,609-660 + set_agent())
     __device__ void env_init(double* lw_init) {
         uint32_t base = (uint32_t)w[W_SPAWN_CTR];
         for (int i = g; i < T.n_lm; i += GS) {
@@ -686,28 +698,37 @@ template <typename R, int FAM, int GS = 1> struct EnvCtx {
         for (int j = g; j < T.n_lw; j += GS) {
             double p[3];
             gen_position(base, T.n_lw, j, T.lw_spawn, p);
-            lw_init[3 * j] = p[0]; lw_init[3 * j + 1] = p[1]; lw_init[3 * j + 2] = p[2];
+            if (!fam_l5(FAM)) { lw_init[3 * j] = p[0]; lw_init[3 * j + 1] = p[1]; lw_init[3 * j + 2] = p[2]; }
             replace(j, p[0], p[1], p[2]);
         }
         if (GS > 1) __threadfence_block();                 // episode_start of the other lanes reads lw_init (fixed spawn)
         gsync();
         w[W_SPAWN_CTR] += 2 * T.n_lw;
+        if (fam_l5(FAM)) {
+            if (FAM == FAM_L5_MULTI && T.l5_eval) agent = 0;                        // Teacher_Student=False: no agent is chosen, no draw
+            else {
+                agent = (int)(spawn_u((uint32_t)w[W_SPAWN_CTR]) * T.n_lw); // entities_manager.py:350-383, randomness as data
+                w[W_SPAWN_CTR] += 1;
+            }
+            registered = false;
+        }
         episode_start(lw_init);
         w[W_INIT] = 1;
     }
-    // Env.reset -> Task.on_reset  exp02_vFinal_environment.py:133-151, task :254-273
+    // Env.reset -> Task.on_reset  exp02_vFinal_environment.py:133-151, task :254-273 (level5_envrionment.py:203-231,
+    // task on_reset :275-283)
     __device__ void reset_env(double* lw_init) {
         if (FAM == FAM_DRIVEN && kills) for (int j = 0; j < T.n_lw; ++j) kills[j] = 0;      // on_episode_start evaluation_task.py:360-364
-        w[W_STEP] = 0; w[W_MAX_STEP] = T.max_step;
-        w[W_AGENT_KILLS] = w[W_ALLIES_KILLS] = w[W_DEADS] = 0; w[W_BUILDING] = 1;
+        reset_words();
         set_last_closest(T.dome);
-        w[W_EP_RETURN] = __float_as_int(0.0f); w[W_EP_STEPS] = 0;
         for (int d = g; d < T.D; d += GS) disarm(d);
         gsync();
         episode_start(lw_init);
         refresh_offsets();
         S.envflag[le] |= EF_NAV_RESET;
+        if (fam_l5(FAM)) broadcast_step();                 // reset_step_counter: step 0
     }
+    // ---- level5 (Level5C1FusionTask) ----
     // ---- level5 (Level5C1FusionTask) ----
     __device__ int n_active(int k) const {                // setup_round :158-160
         const int n = (k - 1) * T.invaders_per_round + T.initial_invaders;
@@ -723,52 +744,18 @@ template <typename R, int FAM, int GS = 1> struct EnvCtx {
         }
         w[W_SPAWN_CTR] += 2 * n;
     }
-    __device__ void episode_start5() {                    // :262-273
-        w[W_ROUND] = T.initial_round;
-        setup_round5(T.initial_round);
-        for (int j = 0; j < T.n_lw; ++j) arm(j);
-        const uint32_t base = (uint32_t)w[W_SPAWN_CTR];
-        for (int j = 0; j < T.n_lw; ++j) {
-            double p[3];
-            gen_position(base, T.n_lw, j, T.lw_spawn, p);
-            replace(j, p[0], p[1], p[2]);
+    // ---- the family's Env.__init__ and Env.reset ----
+    __device__ void init_task(double* lw_init, double* last_dist) {
+        for (int k = 0; k < ENV_WORDS; ++k) w[k] = 0;
+        if (fam_l5(FAM)) {
+            for (int k = 0; k < ENV5_WORDS; ++k) w5[k] = 0;
+            w5[W5_LAST_DIST_LO] = 0; w5[W5_LAST_DIST_HI] = 0x7ff80000;     // NaN: last_distance not set yet
         }
-        w[W_SPAWN_CTR] += 2 * T.n_lw;
+        if (FAM == FAM_STAGE01) env_init_stage01(); else if (FAM == FAM_STAGE02) env_init_stage02(last_dist); else env_init(lw_init);
     }
-    __device__ void env_init5() {                         // on_env_init :253-257,609-660 + set_agent()
-        uint32_t base = (uint32_t)w[W_SPAWN_CTR];
-        for (int i = 0; i < T.n_lm; ++i) {
-            double p[3];
-            gen_position(base, T.n_lm, i, T.born, p);
-            replace(T.n_lw + i, p[0], p[1], p[2]);
-        }
-        w[W_SPAWN_CTR] += 2 * T.n_lm;
-        base = (uint32_t)w[W_SPAWN_CTR];
-        for (int j = 0; j < T.n_lw; ++j) {
-            double p[3];
-            gen_position(base, T.n_lw, j, T.lw_spawn, p);
-            replace(j, p[0], p[1], p[2]);
-        }
-        w[W_SPAWN_CTR] += 2 * T.n_lw;
-        if (FAM == FAM_L5_MULTI && T.l5_eval) agent = 0;                            // Teacher_Student=False: no agent is chosen, no draw
-        else {
-            agent = (int)(spawn_u((uint32_t)w[W_SPAWN_CTR]) * T.n_lw);     // entities_manager.py:350-383, randomness as data
-            w[W_SPAWN_CTR] += 1;
-        }
-        registered = false;
-        episode_start5();
-        w[W_INIT] = 1;
-    }
-    __device__ void reset_env5() {                        // level5_envrionment.py:203-231, task on_reset :275-283
-        w[W_STEP] = 0; w[W_MAX_STEP] = T.max_step;
-        w[W_AGENT_KILLS] = w[W_ALLIES_KILLS] = w[W_DEADS] = 0; w[W_BUILDING] = 1;
-        set_last_closest(T.dome);
-        w[W_EP_RETURN] = __float_as_int(0.0f); w[W_EP_STEPS] = 0;
-        for (int d = 0; d < T.D; ++d) disarm(d);
-        episode_start5();
-        refresh_offsets();
-        S.envflag[le] |= EF_NAV_RESET;
-        broadcast_step();                                  // reset_step_counter: step 0
+    __device__ void reset_task(double* lw_init, double* last_dist) {
+        if (FAM == FAM_STAGE01) reset_env_stage01(); else if (FAM == FAM_STAGE02) reset_env_stage02(last_dist); else reset_env(lw_init);
+        if (fam_l5(FAM)) { w5[W5_STACK_MODE] = STACK_EMPTY; w5[W5_OBS_CALL] += T.l5_base ? 3 : 1; }
     }
     __device__ void set_last_closest(double v) {
         long long bits = __double_as_longlong(v);
@@ -786,6 +773,13 @@ template <typename R, int FAM, int GS = 1> struct EnvCtx {
     __device__ bool gun_available(int j) const {
         if (S.ammo[b + j] <= 0) return true;
         return T.cooldown <= (double)gstep() - (double)S.last[b + j];
+    }
+    __device__ void gun_state(int j, float* g) const {      // Gun.get_state gun.py:101-113
+        const double wait = fmax(T.cooldown - ((double)gstep() - (double)S.last[b + j]), 0.0);
+        const int mx = T.munition > 0 ? T.munition : 1;
+        g[0] = (float)((double)S.ammo[b + j] / (double)mx);
+        g[1] = (float)(wait / T.cooldown);
+        g[2] = gun_available(j) ? 1.f : 0.f;
     }
     // identify_invaders_in_range(...)[j][0] (offsets_handler.py:283-309: ascending stable sort -> first index wins ties; sqrt is
     // monotone, so squared distances pick the same winner).
@@ -822,6 +816,25 @@ template <typename R, int FAM, int GS = 1> struct EnvCtx {
         gargmin(best, bd);
         return best;
     }
+    // identify_closest_ally(as) on the offsets snapshot (the agent itself when it flies alone), then that ally's nearest
+    // invader; -1 when the agent is not in the snapshot
+    __device__ int ally_target(int as) const {
+        int src = -1;
+        if (off(as)) {
+            int n_all = 0;
+            for (int j = 0; j < T.n_lw; ++j) n_all += off(j) ? 1 : 0;
+            if (n_all <= 1) src = as;
+            else {
+                double bd = 0;
+                for (int j = 0; j < T.n_lw; ++j) {
+                    if (j == as || !off(j)) continue;
+                    const double dd = dist2(j, as);
+                    if (src < 0 || dd < bd) { src = j; bd = dd; }
+                }
+            }
+        }
+        return src >= 0 ? nearest_invader(src) : -1;
+    }
     __device__ int count_outside_dome(int lo, int hi) const {
         int n = 0;
         const double r2 = T.dome * T.dome;
@@ -841,10 +854,604 @@ __device__ __forceinline__ int warp_compact(bool pred, int value, int* list, int
 
 #ifdef DC_PROFILE_PHASES      // per-warp clock stamps at the phase borders of env_kernel (profiles/phase_clocks.py)
 __device__ long long g_phase_clk[8192 * 8];
-#define DC_STAMP(k) do { if (MODE == MODE_STEP && lane == 0) { const int gw = blockIdx.x * (blockDim.x >> 5) + (tid >> 5); if (gw < 8192) g_phase_clk[gw * 8 + (k)] = clock64(); } } while (0)
+#define DC_STAMP_STEP(k) do { if ((threadIdx.x & 31) == 0) { const int gw = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); if (gw < 8192) g_phase_clk[gw * 8 + (k)] = clock64(); } } while (0)
 #else
-#define DC_STAMP(k) do { } while (0)
+#define DC_STAMP_STEP(k) do { } while (0)
 #endif
+#define DC_STAMP(k) do { if (MODE == MODE_STEP) DC_STAMP_STEP(k); } while (0)      // reset launches stamp nothing
+
+// ------------------------------------------------------------------------------------------------
+// P3 per family: what each reference task does in Task.on_step_middle (engagement, reward, termination) and
+// Task.on_step_end.  env_kernel's env loop calls the family's pair and writes the outputs common to all families.
+// ------------------------------------------------------------------------------------------------
+// normalize_inertial_data's clip(v / scale, -1, 1).  The float32 build multiplies in float32 (its inputs are float32
+// state; one rounding of difference at most), the float64 build keeps the reference's float64 arithmetic.
+template <typename R> __device__ __forceinline__ float nrm(double v, double inv_scale) {
+    if constexpr (sizeof(R) == 4) return fminf(fmaxf((float)v * (float)inv_scale, -1.0f), 1.0f);
+    else return (float)fmin(fmax(v * inv_scale, -1.0), 1.0);
+}
+// the scales of normalize_inertial_data normalization.py:6-110 (the position scale is the dome radius)
+constexpr double INV_SPEED = 1.0 / (1 * 10 * (1000.0 / 3600.0));
+constexpr double INV_PI = 1.0 / 3.141592653589793, INV_2PI = 1.0 / (2 * 3.141592653589793);
+
+// What on_step_middle hands to the rest of the step.
+struct StepMiddle {
+    double reward = 0.0;
+    bool done = false, lm_alive = false, lw_alive = false, all_over = false;
+    bool caught = false;     // stage01: the munition was caught
+    float g[3];              // the agent's Gun.get_state
+};
+
+// ================= stage01: compute_reward / compute_termination (level2 modified_v2 :157-191) =================
+template <typename R, int FAM, int GS> __device__ __forceinline__ StepMiddle stage01_on_step_middle(EnvCtx<R, FAM, GS>& C, const R* ag, const double* ap) {
+    const TaskParams& T = C.T;
+    int32_t* w = C.w;
+    StepMiddle m;
+    const int lm = T.n_lw;
+    const double dcur = sqrt(C.dist2(lm, 0));
+    double bonus = 0, penalty = 0;
+    if (dcur < C.last_closest()) bonus += 10.0 * norm3((double)ag[AG_UB], (double)ag[AG_VB], (double)ag[AG_WB]);
+    m.caught = dcur < 0.4;                           // CATCH_DISTANCE (:34)
+    if (m.caught) bonus += 1000.0;
+    if (dcur > T.dome) penalty += 1000.0;
+    m.reward = -dcur + bonus - penalty;
+    m.done = w[W_STEP] > w[W_MAX_STEP];
+    m.done |= norm3(ap[0], ap[1], ap[2]) > T.dome;
+    m.done |= norm3(C.pos(lm, 0), C.pos(lm, 1), C.pos(lm, 2)) > T.dome;
+    C.gun_state(C.agent, m.g);
+    C.set_last_closest(dcur);
+    return m;
+}
+// replace_invader_if_close + update_last_distance (:148-155,193-198)
+template <typename R, int FAM, int GS> __device__ __forceinline__ void stage01_on_step_end(EnvCtx<R, FAM, GS>& C, const StepMiddle& m, const double* ap) {
+    if (m.caught) {
+        const int lm = C.T.n_lw, b = C.b;
+        double p[3];
+        C.w[W_AGENT_KILLS] += 1;
+        C.u3(p);
+        C.replace_invader_stage01(lm, p);
+        C.set_last_closest(norm3((double)C.S.newpos[3 * (b + lm)] - ap[0], (double)C.S.newpos[3 * (b + lm) + 1] - ap[1],
+                                 (double)C.S.newpos[3 * (b + lm) + 2] - ap[2]));
+    }
+}
+
+// ================= stage02: L3Stage1.on_step_middle (level3/components/stages.py:144-179) =================
+template <typename R, int FAM, int GS> __device__ __forceinline__ StepMiddle stage02_on_step_middle(EnvCtx<R, FAM, GS>& C, const R* ag, const double* last_dist) {
+    const TaskParams& T = C.T;
+    Smem<R>& S = C.S;
+    int32_t* w = C.w;
+    const int b = C.b, D = T.D;
+    StepMiddle m;
+    int shots = 0, exploded = 0;
+    C.nearest_all();
+    for (int j = 0; j < T.n_lw; ++j) {              // process_shoot_range_invaders + shoot_by_ids (quadcopter_manager.py:155-169)
+        if (!C.off(j)) continue;
+        const int tgt = C.nearest_shoot(j);
+        if (tgt < 0) continue;
+        if (S.ammo[b + j] == 0) { C.disarm(tgt); ++shots; continue; }      // "LW suicided to kill LM"
+        if (!C.gun_available(j)) continue;
+        S.ammo[b + j] -= 1; S.last[b + j] = (R)w[W_STEP];
+        const double u = hit_uniform(T.k0, T.k1, C.env_id, (uint32_t)w[W_HIT_CTR]);
+        w[W_HIT_CTR] += 1;
+        if (u < T.fire_p) { C.disarm(tgt); ++shots; }
+    }
+    for (int j = 0; j < T.n_lw; ++j) {              // process_explosion_range_invaders
+        if (!C.off(j)) continue;
+        const int tgt = C.nearest_expl(j);
+        if (tgt < 0) continue;
+        C.disarm(j); C.disarm(tgt); ++exploded;
+    }
+    w[W_AGENT_KILLS] += shots; w[W_DEADS] += exploded;
+    C.gun_state(C.agent, m.g);
+    // compute_reward stages.py:234-296 with the closest distances of OffsetHandler (row 0)
+    const int j0 = C.row0();
+    double cur2 = -1.0, last = -1.0;
+    for (int i = T.n_lw; i < D; ++i) {
+        if (!C.off(i) || j0 < 0) continue;
+        const double d2 = C.dist2(j0, i);
+        if (cur2 < 0 || d2 < cur2) cur2 = d2;
+        const double ld = last_dist[i - T.n_lw];
+        if (ld == ld && (last < 0 || ld < last)) last = ld;
+    }
+    const double current = sqrt(fmax(cur2, 0.0));
+    const double munition = (double)m.g[0], reload = (double)fmax(T.cooldown - ((double)w[W_STEP] - (double)S.last[b]), 0.0) / T.cooldown;
+    const bool avail = m.g[2] == 1.f;
+    double score = (avail || munition == 0.0) ? -current : current * (2 * reload - 1);
+    double bonus = 0, penalty = 0;
+    if (0.01 < last - current && (avail || munition == 0.0))
+        bonus += 10.0 * norm3((double)ag[AG_UB], (double)ag[AG_VB], (double)ag[AG_WB]);
+    bonus += 1000.0 * shots;
+    penalty += 1000.0 * exploded;
+    const int lw_out = C.count_outside_dome(0, T.n_lw);
+    if (lw_out > 0) penalty += 1000.0;
+    m.reward = score + bonus - penalty;
+    int n_armed_lw = 0;
+    for (int j = 0; j < T.n_lw; ++j) n_armed_lw += C.live(j) ? 1 : 0;
+    m.done = w[W_STEP] > w[W_MAX_STEP];             // compute_termination stages.py:298-344
+    m.done |= lw_out > 0;
+    m.done |= C.count_outside_dome(T.n_lw, D) > 0;
+    m.done |= n_armed_lw < T.n_lw;
+    return m;
+}
+// disarmed munitions reappear at once (stages.py:170-174,370-376); on_step_end: last offsets := current
+template <typename R, int FAM, int GS> __device__ __forceinline__ void stage02_on_step_end(EnvCtx<R, FAM, GS>& C, double* last_dist) {
+    const TaskParams& T = C.T;
+    int32_t* w = C.w;
+    const int D = T.D;
+    int n_dead = 0;
+    for (int i = T.n_lw; i < D; ++i) n_dead += C.live(i) ? 0 : 1;
+    if (n_dead > 0) {
+        const uint32_t base = (uint32_t)w[W_SPAWN_CTR];
+        int k = 0;
+        for (int i = T.n_lw; i < D; ++i) {
+            if (C.live(i)) continue;
+            double p[3];
+            C.gen3(base, n_dead, k++, T.respawn_r0, T.respawn_r1, p);
+            C.replace(i, p[0], p[1], p[2]);
+            C.arm(i);
+        }
+        w[W_SPAWN_CTR] += 3 * n_dead;
+    }
+    const int j0 = C.row0();
+    const double qnan = __longlong_as_double(0x7ff8000000000000LL);
+    for (int i = T.n_lw; i < D; ++i)
+        last_dist[i - T.n_lw] = (C.off(i) && j0 >= 0) ? sqrt(C.dist2(j0, i)) : qnan;
+}
+
+// ================= level5: Level5C1FusionTask.on_step_middle (level5_c1_fusion_task.py:298-336) =================
+template <typename R, int FAM, int GS> __device__ __forceinline__ StepMiddle level5_on_step_middle(EnvCtx<R, FAM, GS>& C, const R* ag, const double* ap) {
+    const TaskParams& T = C.T;
+    Smem<R>& S = C.S;
+    int32_t* w = C.w;
+    int32_t* w5 = C.w5;
+    const int b = C.b, D = T.D;
+    const double apx = ap[0], apy = ap[1], apz = ap[2];
+    StepMiddle m;
+    const int as = C.agent;
+    int agent_shots = 0, ally_shots = 0;
+    C.nearest_all();
+    for (int j = 0; j < T.n_lw; ++j) {              // process_shoot_range_invaders :399-424
+        if (!C.off(j)) continue;
+        const int tgt = C.nearest_shoot(j);
+        if (tgt < 0) continue;
+        if (!(C.gun_available(j) && S.ammo[b + j] > 0)) continue;
+        S.ammo[b + j] -= 1; S.last[b + j] = (R)C.gstep();
+        const double u = hit_uniform(T.k0, T.k1, C.env_id, (uint32_t)w[W_HIT_CTR]);
+        w[W_HIT_CTR] += 1;
+        if (u < T.fire_p) { C.disarm(tgt); if (j == as) ++agent_shots; else ++ally_shots; }
+    }
+    int exploded = 0, agent_suicide = 0, ally_suicide = 0;
+    for (int j = 0; j < T.n_lw; ++j) {              // process_explosion_range_invaders :366-397
+        if (!C.off(j)) continue;
+        const int tgt = C.nearest_expl(j);
+        if (tgt < 0) continue;
+        C.disarm(j); C.disarm(tgt);
+        if (S.ammo[b + j] == 0 && j == as) ++agent_suicide;
+        else if (S.ammo[b + j] == 0) ++ally_suicide;
+        else ++exploded;
+    }
+    w[W_AGENT_KILLS] += agent_shots; w[W_ALLIES_KILLS] += ally_shots; w[W_DEADS] += exploded;
+    for (int i = T.n_lw; i < D; ++i)                   // process_invaders_in_origin
+        if (C.off(i) && sq3(C.pos(i, 0), C.pos(i, 1), C.pos(i, 2)) < 0.2 * 0.2) C.disarm(i);
+    if (FAM == FAM_L5_MULTI && T.l5_eval) m.reward = 0.0;                 // "EVALUATION TASK DO NOT USES REWARD" (level5_2bt_evaluation_task.py:418-427)
+    else if (T.reward == 2) {
+        // Level5FusionTask.compute_reward (level5_fusion_task.py:448-555; allies_dead is never passed)
+        double score, bonus = 0, penalty = 0;
+        const bool avail = C.gun_available(as);
+        const int ammo = S.ammo[b + as];
+        const int target = C.ally_target(as);
+        double tpx = 0, tpy = 0, tpz = 0;
+        if (target >= 0) { tpx = C.pos(target, 0); tpy = C.pos(target, 1); tpz = C.pos(target, 2); }
+        const double current = norm3(apx - tpx, apy - tpy, apz - tpz);
+        if (avail || ammo == 0) score = -current;
+        else {
+            score = current;
+            if (current < 5.0) penalty += ((5.0 - current) / 5.0) * (0.50 * 1000.0);
+        }
+        if (!avail && ammo > 0 && (current - C.last_closest()) > 0.01) bonus += 0.10 * 1000.0;
+        if (agent_shots > 0) bonus += 1.0 * agent_shots * 1000.0;
+        if (ally_shots > 0 || ally_suicide > 0) bonus += 0.5 * (ally_shots + ally_suicide) * 1000.0;
+        if (agent_suicide > 0) penalty += 2.0 * agent_suicide * 1000.0;
+        if (exploded > 0) penalty += 1000.0 * exploded;
+        if (apz < -5.0) penalty += fmin((-5.0 - apz) / 1.0, 1.0) * 1000.0;
+        if (C.count_outside_dome(0, T.n_lw) > 0) penalty += 1000.0;
+        const double d0 = norm3(apx, apy, apz);
+        if (d0 > T.born - 2) penalty += fmin((d0 - (T.born - 2)) * 1.0, 1000.0);
+        C.set_last_closest(current);
+        m.reward = fmin(fmax(score + bonus - penalty, -3000.0), 3000.0);
+    } else {
+        // compute_reward :434-484: one-shot last_distance, clipped
+        const int target = C.off(as) ? C.nearest_invader(as) : -1;
+        double tpx = 0, tpy = 0, tpz = 0;
+        if (target >= 0) { tpx = C.pos(target, 0); tpy = C.pos(target, 1); tpz = C.pos(target, 2); }
+        const double distance = norm3(apx - tpx, apy - tpy, apz - tpz);
+        double last_distance = __longlong_as_double(((long long)w5[W5_LAST_DIST_HI] << 32) | (unsigned int)w5[W5_LAST_DIST_LO]);
+        if (last_distance != last_distance) {          // ``hasattr(self, 'last_distance')``: set once per env object
+            last_distance = distance;
+            const long long bits = __double_as_longlong(distance);
+            w5[W5_LAST_DIST_LO] = (int32_t)(bits & 0xffffffffLL); w5[W5_LAST_DIST_HI] = (int32_t)(bits >> 32);
+        }
+        if (distance < last_distance) m.reward += 10.0 * norm3((double)ag[AG_UB], (double)ag[AG_VB], (double)ag[AG_WB]);
+        if (agent_shots > 0) m.reward += 1.0 * agent_shots * 1000.0;
+        if (agent_suicide > 0) m.reward -= 2.0 * agent_suicide * 1000.0;
+        m.reward = fmin(fmax(m.reward, -3000.0), 3000.0);
+    }
+    if (agent_shots + ally_shots > 0) w[W_MAX_STEP] += T.step_increment;
+    // compute_termination :488-545
+    const int lw_out = C.count_outside_dome(0, T.n_lw);
+    for (int i = T.n_lw; i < D; ++i) m.lm_alive |= C.live(i);
+    for (int j = 0; j < T.n_lw; ++j) m.lw_alive |= C.live(j);
+    m.all_over = !m.lm_alive && w[W_ROUND] >= T.max_rounds;
+    m.done = C.gstep() > w[W_MAX_STEP];
+    m.done |= m.all_over;
+    m.done |= lw_out > 0;
+    m.done |= C.count_outside_dome(T.n_lw, D) > 0;
+    m.done |= !m.lw_alive;
+    if (FAM != FAM_L5_MULTI) m.done |= !C.live(as);
+    if (!(FAM == FAM_L5_MULTI && T.l5_eval)) m.done |= apz < -5.99;
+    C.gun_state(C.agent, m.g);
+    return m;
+}
+// Task.on_step_end :338-350 + advance_round :139-152 (setup_round disarms every munition first: the id clash zeroes the
+// guns' step until the next broadcast)
+template <typename R, int FAM, int GS> __device__ __forceinline__ void level5_on_step_end(EnvCtx<R, FAM, GS>& C, const StepMiddle& m) {
+    const TaskParams& T = C.T;
+    Smem<R>& S = C.S;
+    int32_t* w = C.w;
+    int32_t* w5 = C.w5;
+    if (!m.all_over && !m.lm_alive && m.lw_alive) C.advance_round();
+    if (T.l5_base) {
+        // base env: a dead agent still runs read_data -> six empty spheres; the candidates of
+        // get_random_neighborhood are the wingmen with an open buffer in the agent's ring at ITS read_data of
+        // the first compute_observation call: the armed ones, the ones that died before this step (their LiDAR
+        // broadcasts re-opened it) and, of those that died in this step, the ones in front of the agent
+        int cand = 0;
+        for (int P = 0; P < T.n_lw; ++P)
+            if (C.live(P) || !(S.ev[C.b + P] & EV_WAS_ARMED) || P < C.agent) cand |= 1 << P;
+        w5[W5_STACK_MODE] = (C.live(C.agent) ? STACK_BUILD : STACK_EMPTY) | (cand << 8);
+        w5[W5_OBS_CALL] += 3;
+    } else {
+        w5[W5_STACK_MODE] = (FAM == FAM_L5_MULTI || C.live(C.agent)) ? STACK_BUILD : STACK_KEEP;   // a dead agent's flight state keeps its last stack
+        w5[W5_OBS_CALL] += 1;
+    }
+    S.envflag[C.le] |= (w[W_STEP] % RING) << 8;     // ring slot of this step for the feature pass
+}
+// Level5DumbMultiObs.compute_info (level5_dumb_multiobs.py:112-150): inertial + gun vector of every ARMED wingman, at the
+// point between on_step_middle and on_step_end
+template <typename R, int FAM, int GS> __device__ __forceinline__ void write_multi_info(const EnvCtx<R, FAM, GS>& C, const StepArgs<R>& A, int env) {
+    const TaskParams& T = C.T;
+    for (int P = 0; P < T.n_lw; ++P) {
+        const bool here = C.live(P);
+        A.mo_present[(long long)env * T.n_lw + P] = here ? 1 : 0;
+        if (!here) continue;
+        const V4<R>* rp = reinterpret_cast<const V4<R>*>(A.p.agent + ((long long)env * T.n_rec + P) * AG_WORDS);
+        const V4<R> r0 = ld4(rp), r1 = ld4(rp + 1), r2 = ld4(rp + 2);
+        float gp3[3]; C.gun_state(P, gp3);
+        float* o = A.mo_inertial + ((long long)env * T.n_lw + P) * 15;
+        o[0] = nrm<R>(C.pos(P, 0), C.inv_dome); o[1] = nrm<R>(C.pos(P, 1), C.inv_dome); o[2] = nrm<R>(C.pos(P, 2), C.inv_dome);
+        o[3] = nrm<R>(r0.x, INV_SPEED); o[4] = nrm<R>(r0.y, INV_SPEED); o[5] = nrm<R>(r0.z, INV_SPEED);
+        o[6] = nrm<R>(r0.w, INV_PI); o[7] = nrm<R>(r1.x, INV_PI); o[8] = nrm<R>(r1.y, INV_PI);
+        o[9] = nrm<R>(r1.z, INV_2PI); o[10] = nrm<R>(r1.w, INV_2PI); o[11] = nrm<R>(r2.x, INV_2PI);
+        o[12] = gp3[0]; o[13] = gp3[1]; o[14] = gp3[2];
+    }
+}
+// ================= stage03 (level4 tasks, FAM_DRIVEN too): Task.on_step_middle exp02_vFinal_task.py:284-318 =================
+template <typename R, int FAM, int GS> __device__ __forceinline__ StepMiddle stage03_on_step_middle(EnvCtx<R, FAM, GS>& C, const StepArgs<R>& A, int env, const R* ag, const double* ap) {
+    const TaskParams& T = C.T;
+    Smem<R>& S = C.S;
+    int32_t* w = C.w;
+    const int b = C.b, D = T.D, gl = C.g;
+    const double apx = ap[0], apy = ap[1], apz = ap[2];
+    StepMiddle m;
+    if (T.reward == 1) {                               // update_building_life (exp02_v2_full_task.py)
+        int cnt = 0;
+        for (int i = T.n_lw + gl; i < D; i += GS)
+            if (C.off(i) && sq3(C.pos(i, 0), C.pos(i, 1), C.pos(i, 2)) < 0.2 * 0.2) ++cnt;
+        w[W_BUILDING] = max(w[W_BUILDING] - C.gsum(cnt), 0);
+    }
+    // process_shoot_range_invaders :391-412 -> shoot_by_ids -> Gun.shoot
+    int agent_shots = 0, ally_shots = 0;
+    C.nearest_all();
+    for (int j = 0; j < T.n_lw; ++j) {
+        if (!C.off(j)) continue;
+        const int tgt = C.nearest_shoot(j);
+        if (tgt < 0) continue;
+        if (!(C.gun_available(j) && S.ammo[b + j] > 0)) continue;
+        { const int am = S.ammo[b + j]; C.gsync(); S.ammo[b + j] = am - 1; }      // every lane of the group stores the same value
+        S.last[b + j] = (R)w[W_STEP];
+        const double u = hit_uniform(T.k0, T.k1, C.env_id, (uint32_t)w[W_HIT_CTR]);
+        w[W_HIT_CTR] += 1;
+        if (u < T.fire_p) {
+            C.disarm(tgt); if (j == 0) ++agent_shots; else ++ally_shots;
+            if (FAM == FAM_DRIVEN) A.p.lw_kills[(long long)env * T.n_lw + j] += 1;       // Evaluation_Task.lw_kills :491-494
+        }
+    }
+    // process_explosion_range_invaders :358-389 (same, now stale, distance matrix)
+    int exploded = 0, ally_suicide = 0, agent_suicide = 0;
+    for (int j = 0; j < T.n_lw; ++j) {
+        if (!C.off(j)) continue;
+        const int tgt = C.nearest_expl(j);
+        if (tgt < 0) continue;
+        C.disarm(j); C.disarm(tgt);
+        if (T.reward == 1) ++exploded;
+        else if (S.ammo[b + j] == 0 && j == 0) ++agent_suicide;
+        else if (S.ammo[b + j] == 0) ++ally_suicide;
+        else ++exploded;
+    }
+    const bool EVAL = FAM == FAM_DRIVEN && T.eval_task;     // Evaluation_Task.on_step_middle evaluation_task.py:383-407
+    if (!EVAL) {
+        w[W_AGENT_KILLS] += agent_shots; w[W_ALLIES_KILLS] += ally_shots; w[W_DEADS] += exploded;
+        C.gsync();
+        for (int i = T.n_lw + gl; i < D; i += GS)       // process_invaders_in_origin :656-659
+            if (C.off(i) && sq3(C.pos(i, 0), C.pos(i, 1), C.pos(i, 2)) < 0.2 * 0.2) C.disarm(i);
+        C.gsync();
+    }
+
+    // ---- reward ----
+    C.gun_state(C.agent, m.g);
+    const int lw_out = C.count_outside_dome(0, T.n_lw);
+    if (EVAL) m.reward = 0.0;                        // "Reward will be deactivated" (evaluation_task.py:512-516)
+    else if (T.reward == 0) {                        // exp02_vFinal_task.py:422-514
+        double bonus = 0, penalty = 0, score;
+        const double munition = (double)S.ammo[b] / (double)(T.munition > 0 ? T.munition : 1);
+        const double reload = fmax(T.cooldown - ((double)w[W_STEP] - (double)S.last[b]), 0.0) / T.cooldown;
+        const bool avail = C.gun_available(0);
+        const int target = C.ally_target(0);
+        double tpx = 0, tpy = 0, tpz = 0;
+        if (target >= 0) { tpx = C.pos(target, 0); tpy = C.pos(target, 1); tpz = C.pos(target, 2); }
+        const double current = norm3(apx - tpx, apy - tpy, apz - tpz);
+        if (0.01 < C.last_closest() - current && (avail || munition == 0.0))
+            bonus += T.vel_bonus * norm3((double)ag[AG_UB], (double)ag[AG_VB], (double)ag[AG_WB]);
+        C.set_last_closest(current);
+        score = (avail || munition == 0.0) ? -current : current * (2 * reload - 1);
+        if (agent_shots > 0 || agent_suicide > 0) bonus += (agent_shots + agent_suicide) * 1000.0;
+        if (ally_shots > 0 || ally_suicide > 0) bonus += 0.5 * (ally_shots + ally_suicide) * 1000.0;
+        else if (exploded > 0) penalty += 1000.0 * exploded;
+        if (apz < -5.0) penalty += (-5.0 - apz) / (-5.0 + 6.0) * 1000.0;
+        if (lw_out > 0) penalty += 1000.0;
+        const double d0 = norm3(apx, apy, apz);
+        if (d0 > T.born - 2) penalty += d0 - T.born - 2;
+        m.reward = score + bonus - penalty;
+    } else {                                         // exp02_v2_full_task.py compute_reward
+        double bonus = 0, penalty = 0;
+        const int shots = agent_shots + ally_shots;
+        const double kills = (double)(w[W_AGENT_KILLS] + w[W_ALLIES_KILLS]);
+        if (shots > 0) bonus += (shots + kills / 10) * 1000.0;
+        if (S.ammo[b] == 0 && exploded > 0) bonus += (shots + kills / 10) * 1000.0;
+        else if (exploded > 0) penalty += 1000.0 * exploded;
+        if (apz < 0.01) penalty += 1000.0;
+        if (lw_out > 0) penalty += 1000.0;
+        if (w[W_BUILDING] < 1) penalty += 1000.0 * (1 - w[W_BUILDING]);
+        const double d0 = norm3(apx, apy, apz);
+        if (d0 > T.born) penalty += d0 - T.born;
+        m.reward = 0 + bonus - penalty;
+    }
+    if (agent_shots + ally_shots > 0) w[W_MAX_STEP] += T.step_increment;   // increment_max_step :149-152
+
+    // ---- termination :516-568 ----
+    for (int i = T.n_lw + gl; i < D; i += GS) m.lm_alive |= C.live(i);
+    m.lm_alive = C.gany(m.lm_alive);
+    for (int j = 0; j < T.n_lw; ++j) m.lw_alive |= C.live(j);
+    m.all_over = !m.lm_alive && w[W_ROUND] >= T.n_lm;
+    m.done = w[W_STEP] > w[W_MAX_STEP] && !(EVAL && !T.time_limited);      // evaluation_task.py:522
+    m.done |= m.all_over;
+    if (T.reward == 1) m.done |= w[W_BUILDING] <= 0;
+    m.done |= lw_out > 0;
+    m.done |= C.count_outside_dome(T.n_lw, D) > 0;
+    m.done |= !m.lw_alive;
+    if (!EVAL) {                                     // a training env stops when its agent dies; the evaluation goes on
+        m.done |= !C.live(0);
+        m.done |= apz < (T.reward == 1 ? 0.01 : -5.99);
+    }
+    if (FAM == FAM_DRIVEN && A.lw_info) {            // compute_info (evaluation_task.py:554-574), between middle and end
+        for (int j = 0; j < T.n_lw; ++j)
+            reinterpret_cast<int4*>(A.lw_info)[(long long)env * T.n_lw + j] =
+                make_int4(A.p.lw_kills[(long long)env * T.n_lw + j], C.live(j) ? 1 : 0, S.ammo[b + j], 0);
+    }
+    return m;
+}
+// The inertial observation of wingman P right after Env.reset: its new position, zero velocities and attitude, a fresh
+// gun.  Wingman C.agent gives the agent's vector; write_multi_reset gives those of the multi-observer rows.
+template <typename R, int FAM, int GS> __device__ __forceinline__ void reset_inertial(const EnvCtx<R, FAM, GS>& C, int P, float* o) {
+    const int rp = 3 * (C.b + P);
+    o[0] = nrm<R>(C.S.newpos[rp], C.inv_dome); o[1] = nrm<R>(C.S.newpos[rp + 1], C.inv_dome); o[2] = nrm<R>(C.S.newpos[rp + 2], C.inv_dome);
+    for (int k = 3; k < 12; ++k) o[k] = 0.f;
+    float g[3]; C.gun_state(P, g);
+    o[12] = g[0]; o[13] = g[1]; o[14] = g[2];
+}
+// multi-observer reset observation: every wingman re-armed at its new position
+template <typename R, int FAM, int GS> __device__ __forceinline__ void write_multi_reset(const EnvCtx<R, FAM, GS>& C, const StepArgs<R>& A, int env) {
+    for (int P = 0; P < C.T.n_lw; ++P) {
+        A.mo_present[(long long)env * C.T.n_lw + P] = 1;
+        reset_inertial(C, P, A.mo_inertial + ((long long)env * C.T.n_lw + P) * 15);
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
+// P4: the LiDAR passes of one warp over its envs [LE_LO, LE_HI) and slots [S_LO, S_HI) of the block.
+// ------------------------------------------------------------------------------------------------
+// a cell of the agent's sphere given back (LIDARSpec.empty_sphere), and a cell marked by entity d (EntityType value / 5,
+// normalised age 1/10: lidar_buffer.py:98-99)
+__device__ __forceinline__ void sphere_clear(float* sph, int c, int ch) {
+    sph[c] = 1.0f; sph[N_CELLS + c] = 1.0f;
+    if (ch == 3) sph[2 * N_CELLS + c] = 1.0f;
+}
+__device__ __forceinline__ void sphere_mark(float* sph, int c, float rn, bool is_lw, int ch) {
+    sph[c] = rn;
+    sph[N_CELLS + c] = (float)((is_lw ? 3.0 : 1.0) / 5.0);
+    if (ch == 3) sph[2 * N_CELLS + c] = 0.1f;
+}
+// (cell, r_n) of the entity at imu position e in the frame of the agent at o with the attitude of its record ag.
+// F32 (float32 build, fused flavour): float32 projection, exact cell (lidar_cell_fused_f32).  Otherwise the fused flavour
+// projects in float64 from the float32 snapshot (perception_snapshot.py:91-110), the classic one in float64.
+template <typename R, bool F32> __device__ __forceinline__ void project_agent(const TaskParams& T, const R* o, const R* ag, const R* e, int* cell, double* rn) {
+    if (F32 && T.lidar == 0 && sizeof(R) == 4) {
+        int c; float r;
+        lidar_cell_fused_f32((float)(2 * T.dome), (float)o[0], (float)o[1], (float)o[2],
+                             (float)ag[AG_QX], (float)ag[AG_QY], (float)ag[AG_QZ], (float)ag[AG_QW],
+                             (float)e[0], (float)e[1], (float)e[2], &c, &r);
+        *cell = c; *rn = (double)r;
+    } else if (T.lidar == 0) {
+        int c; double r;
+        lidar_cell_fused(2 * T.dome, (double)(float)o[0], (double)(float)o[1], (double)(float)o[2],
+                         (double)(float)ag[AG_QX], (double)(float)ag[AG_QY], (double)(float)ag[AG_QZ], (double)(float)ag[AG_QW],
+                         (double)(float)e[0], (double)(float)e[1], (double)(float)e[2], &c, &r);
+        *cell = c; *rn = r;
+    } else {
+        const LidarHit h = lidar_project_one(1, 2 * T.dome, (double)o[0], (double)o[1], (double)o[2],
+                                             (double)ag[AG_QX], (double)ag[AG_QY], (double)ag[AG_QZ], (double)ag[AG_QW],
+                                             (double)e[0], (double)e[1], (double)e[2]);
+        *cell = h.cell; *rn = h.rn;
+    }
+}
+
+// level5: every armed wingman P runs FusedLIDAR.update_data (level5_c1_fusion_environment.py:25-26); what the agent's
+// ring keeps of it -- P's float32 pose and the kept features (r_n, theta, phi float64, type, id) -- goes to ring slot
+// step % 10.  stack_kernel assembles the observation from the ring afterwards.
+template <typename R> __device__ __forceinline__ void level5_ring_pass(const StepArgs<R>& A, const Smem<R>& S, int env0, int S_LO, int S_HI, int lane) {
+    const TaskParams& T = A.t;
+    const int D = T.D;
+    int* s_list = S.list + S_LO;
+    for (int P = 0; P < T.n_lw; ++P) {
+        for (int s = S_LO + lane; s < S_HI; s += 32) { S.cell[s] = -1; S.rn[s] = 1.0; }
+        int n_proj = 0;
+        for (int s = S_LO + lane; s < S_HI + lane; s += 32) {
+            bool pred = false;
+            if (s < S_HI) {
+                const int le = A.env_of(s), d = s - le * D;
+                pred = d != P && (S.ev[s] & EV_MID) && (S.ev[le * D + P] & EV_MID) && (S.envflag[le] & EF_LIDAR);
+            }
+            n_proj = warp_compact(pred, s, s_list, n_proj);
+        }
+        __syncwarp();
+        for (int i = lane; i < n_proj; i += 32) {
+            const int s = s_list[i];
+            const int le = A.env_of(s), o = le * D + P;
+            const R* rec = A.p.agent + ((long long)(env0 + le) * T.n_rec + P) * AG_WORDS;
+            const LidarHit h = lidar_project_one(0, 2 * T.dome, (double)(float)S.imu[3 * o], (double)(float)S.imu[3 * o + 1],
+                                                 (double)(float)S.imu[3 * o + 2], (double)(float)rec[AG_QX], (double)(float)rec[AG_QY],
+                                                 (double)(float)rec[AG_QZ], (double)(float)rec[AG_QW],
+                                                 (double)(float)S.imu[3 * s], (double)(float)S.imu[3 * s + 1], (double)(float)S.imu[3 * s + 2]);
+            S.cell[s] = h.cell; S.rn[s] = h.rn; S.ang[2 * s] = h.theta; S.ang[2 * s + 1] = h.phi;
+        }
+        __syncwarp();
+        for (int s = S_LO + lane; s < S_HI; s += 32) {
+            const int le = A.env_of(s), d = s - le * D, b = le * D;
+            if (!(S.envflag[le] & EF_LIDAR) || !(S.ev[b + P] & EV_MID)) continue;
+            const long long entry = ((long long)(env0 + le) * T.n_lw + P) * RING + ((S.envflag[le] >> 8) & 15);
+            const bool win = lidar_wins(0, d, D, S.cell + b, S.rn + b);
+            A.p.ring_meta[entry * D + d] = win ? (S.cell[s] | ((d < T.n_lw ? 3 : 1) << 16)) : -1;
+            if (win) {
+                double* f = A.p.ring_feat + (entry * D + d) * 3;
+                f[0] = S.rn[s]; f[1] = S.ang[2 * s]; f[2] = S.ang[2 * s + 1];
+            }
+            if (d == P) {
+                const R* rec = A.p.agent + ((long long)(env0 + le) * T.n_rec + P) * AG_WORDS;
+                float4* pp = reinterpret_cast<float4*>(A.p.ring_pose + entry * 8);
+                pp[0] = make_float4((float)S.imu[3 * s], (float)S.imu[3 * s + 1], (float)S.imu[3 * s + 2], (float)rec[AG_QX]);
+                pp[1] = make_float4((float)rec[AG_QY], (float)rec[AG_QZ], (float)rec[AG_QW], 0.f);
+            }
+        }
+        __syncwarp();
+    }
+}
+
+// The agent's sphere (wingman 0 observes).  It lives in the caller's obs_lidar buffer across steps and is maintained
+// INCREMENTALLY: the cells held by the previous step's hits (remembered in sphere_desc, parked in S.rn by P0) go back to
+// 1.0, then the new hits are written -- bit-identical to rebuilding LIDARSpec.empty_sphere() + add_features, at a few
+// dozen bytes per env instead of 4 KB.  When the agent is no longer a publisher nothing is touched: the reference keeps
+// the previous sphere (fused_lidar.py:160-166).
+// SYNC0 (FAM_DRIVEN, wingman 0 flown by a policy): its FusedLIDAR keeps ONE sphere that the step-start update
+// (lw_obs_kernel, dc_buffers.lw_lidar[:,0], SimPtrs::lw_desc) and this end-of-step update both overwrite.  When this
+// update is skipped (wingman 0 is no publisher any more) the observation shows that object as the step-start update left
+// it.  SYNC0 projects in float64 from the float32 snapshot in both builds.
+template <typename R, bool SYNC0> __device__ __forceinline__ void agent_sphere_pass(const StepArgs<R>& A, const Smem<R>& S, int env0, int LE_LO, int LE_HI, int S_LO, int S_HI, int lane) {
+    const TaskParams& T = A.t;
+    const int D = T.D;
+    const long long slot0 = (long long)env0 * D;
+    const int ch = T.lidar == 0 ? 3 : 2;
+    const int per_env = ch * N_CELLS;
+    int* s_list = S.list + S_LO;
+    if (A.lidar_ids) {
+        int32_t* idp = A.lidar_ids + (long long)(env0 + LE_LO) * N_CELLS;
+        for (int i = lane; i < (LE_HI - LE_LO) * N_CELLS; i += 32) idp[i] = -1;   // features = [] when skipped
+    }
+    // One pass over the warp's slots: a slot whose entity held a cell of the previous sphere gives it back (cell and,
+    // without SYNC0, remembered-hit record; SYNC0 gives back the cells of every env), and the entities that can mark a
+    // cell now -- alive after the engagement, not the observer, observer still a publisher -- are compacted so that the
+    // float64 projection runs on full warps.
+    int n_proj = 0;
+    for (int s = S_LO + lane; s < S_HI + lane; s += 32) {
+        bool pred = false;
+        if (s < S_HI) {
+            const int le = A.env_of(s), d = s - le * D;
+            const bool on = S.envflag[le] & EF_LIDAR;
+            const int oc = (int)reinterpret_cast<const long long*>(S.rn)[s];
+            if ((on || SYNC0) && oc >= 0) {
+                sphere_clear(A.obs_lidar + (long long)(env0 + le) * per_env, oc, ch);
+                if (!SYNC0) A.p.sphere_desc[slot0 + s] = make_int2(-1, __float_as_int(1.0f));
+            }
+            pred = d != 0 && (S.ev[s] & EV_MID) && on;
+            S.cell[s] = -1;
+        }
+        n_proj = warp_compact(pred, s, s_list, n_proj);
+    }
+    __syncwarp();                                 // un-write before write: two slots of an env may name the same cell
+    if (SYNC0) {                                  // the envs without this update show the step-start sphere of wingman 0
+        for (int s = S_LO + lane; s < S_HI; s += 32) {
+            const int le = A.env_of(s), d = s - le * D;
+            if (S.envflag[le] & EF_LIDAR) continue;
+            const int2 h = A.p.lw_desc[((long long)(env0 + le) * T.n_lw + 0) * D + d];
+            A.p.sphere_desc[slot0 + s] = make_int2(h.x >= 0 ? h.x : -1, h.x >= 0 ? h.y : __float_as_int(1.0f));
+            if (h.x >= 0) sphere_mark(A.obs_lidar + (long long)(env0 + le) * per_env, h.x, __int_as_float(h.y), d < T.n_lw, ch);
+        }
+    }
+    DC_STAMP_STEP(6);
+    for (int i = lane; i < n_proj; i += 32) {
+        const int s = s_list[i];
+        const int b = A.env_of(s) * D;
+        const R* ag = A.p.agent + (long long)(env0 + A.env_of(s)) * T.n_rec * AG_WORDS;      // record of wingman 0
+        project_agent<R, !SYNC0>(T, S.imu + 3 * b, ag, S.imu + 3 * s, S.cell + s, S.rn + s);
+    }
+    __syncwarp();
+    DC_STAMP_STEP(7);
+    // winners among the projected entities (full warps): into the sphere, and remembered for the next step's
+    // un-write (and for the sparse host transfer)
+    for (int i = lane; i < n_proj; i += 32) {
+        const int s = s_list[i];
+        const int le = A.env_of(s), d = s - le * D, b = le * D;
+        if (!lidar_wins(T.lidar, d, D, S.cell + b, S.rn + b)) continue;
+        if (SYNC0) S.ev[s] |= EV_LWIN;
+        const int c = S.cell[s];
+        const float rnf = (float)S.rn[s];
+        sphere_mark(A.obs_lidar + (long long)(env0 + le) * per_env, c, rnf, d < T.n_lw, ch);
+        if (A.lidar_ids) A.lidar_ids[(long long)(env0 + le) * N_CELLS + c] = d;
+        if (!SYNC0) A.p.sphere_desc[slot0 + s] = make_int2(c, __float_as_int(rnf));
+    }
+    if (SYNC0) {                                  // the record of every slot of an env with this update
+        __syncwarp();
+        for (int s = S_LO + lane; s < S_HI; s += 32) {
+            if (!(S.envflag[A.env_of(s)] & EF_LIDAR)) continue;
+            const bool win = S.ev[s] & EV_LWIN;
+            A.p.sphere_desc[slot0 + s] = make_int2(win ? S.cell[s] : -1, __float_as_int(win ? (float)S.rn[s] : 1.0f));
+        }
+    }
+}
+
+// MODE_RESET, first use of an env: an empty sphere (level5: stack of spheres) and no remembered hits
+template <typename R, int FAM> __device__ __forceinline__ void first_use_sphere(const StepArgs<R>& A, const Smem<R>& S, int env0, int LE_LO, int LE_HI, int lane) {
+    const TaskParams& T = A.t;
+    const int D = T.D;
+    const long long slot0 = (long long)env0 * D;
+    const int per_env = (fam_l5(FAM) ? N_STACK * 3 : (T.lidar == 0 ? 3 : 2)) * N_CELLS;
+    for (int e = LE_LO; e < LE_HI; ++e) {
+        if (!(S.envflag[e] & EF_FIRST)) continue;
+        float* sph = A.obs_lidar + (long long)(env0 + e) * per_env;
+        for (int f = lane; f < per_env; f += 32) sph[f] = 1.0f;
+        if (A.lidar_ids) for (int f = lane; f < N_CELLS; f += 32) A.lidar_ids[(long long)(env0 + e) * N_CELLS + f] = -1;
+        for (int f = lane; f < D; f += 32) A.p.sphere_desc[slot0 + (long long)e * D + f] = make_int2(-1, 0);
+    }
+}
 
 template <typename R, int MODE, int FAM, int GS = 1>
 __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOCKS : 1)) env_kernel(const StepArgs<R> A) {
@@ -884,7 +1491,6 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
     DC_STAMP(0);
     if (MODE == MODE_STEP) DC_TL_BEGIN(A.tl_slot);
     constexpr bool STASH_DESC = MODE == MODE_STEP && !fam_l5(FAM);
-    auto env_of = [&](int s) { return (int)(((uint32_t)s * A.div_m) >> 20); };
     {
         constexpr int U = 4;
         for (int s0 = S_LO + lane; s0 < S_HI; s0 += 32 * U) {
@@ -897,7 +1503,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
                 // Evaluation_Task: the episode goes on after wingman 0 died and the env keeps observing it
                 // (EvaluationEnvironment.compute_observation: get_all_pursuers()[0]): its last imu position / last_fired
                 // live on in the snapshot buffer of the previous step (P5 carries them forward)
-                const bool KEEP0 = FAM == FAM_DRIVEN && MODE == MODE_STEP && T.eval_task && ok && !(fwv[u] & F_ARMED) && s - env_of(s) * D == 0;
+                const bool KEEP0 = FAM == FAM_DRIVEN && MODE == MODE_STEP && T.eval_task && ok && !(fwv[u] & F_ARMED) && s - A.env_of(s) * D == 0;
                 qv[u] = ok ? ld4((KEEP0 ? A.p.imu[A.parity] : imu_g) + slot0 + s) : V4<R>{0, 0, 0, 0};
                 if (STASH_DESC) dv[u] = ok ? *reinterpret_cast<const long long*>(A.p.sphere_desc + slot0 + s) : -1LL;
             }
@@ -909,7 +1515,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
                 const bool armed = fw & F_ARMED;
                 S.ammo[s] = fw >> F_AMMO_SHIFT;
                 V4<R> q = qv[u];
-                const bool keep0 = FAM == FAM_DRIVEN && MODE == MODE_STEP && T.eval_task && s - env_of(s) * D == 0;
+                const bool keep0 = FAM == FAM_DRIVEN && MODE == MODE_STEP && T.eval_task && s - A.env_of(s) * D == 0;
                 if (!(armed || keep0 || (MODE == MODE_RESET && (fw & F_OFF)))) q = V4<R>{0, 0, 0, (R)(-T.cooldown)};
                 S.imu[3 * s] = q.x; S.imu[3 * s + 1] = q.y; S.imu[3 * s + 2] = q.z; S.last[s] = q.w;
                 S.ev[s] = MODE == MODE_STEP ? (armed ? (EV_LIVE | EV_OFF | EV_WAS_ARMED | EV_SNAP) : 0)     // on_middle_step: snapshot := armed set
@@ -937,38 +1543,14 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
         if (GS > 1) { C.g = gl; C.gmask = ((1u << GS) - 1u) << (lane & ~(GS - 1)); }
         if (FAM == FAM_DRIVEN) C.kills = A.p.lw_kills + (long long)env * T.n_lw;
         double* lw_init = A.p.lw_init + (long long)env * T.n_lw * 3;
-        int32_t* w5 = fam_l5(FAM) ? A.p.env5 + (long long)env * ENV5_WORDS : nullptr;
-        if (fam_l5(FAM)) { C.agent = w5[W5_AGENT]; C.gun_step = w5[W5_GUN_STEP]; C.registered = w5[W5_REGISTERED] != 0; }
+        double* last_dist = A.p.last_dist + (long long)env * T.n_lm;
+        if (fam_l5(FAM)) {
+            C.w5 = A.p.env5 + (long long)env * ENV5_WORDS;
+            C.agent = C.w5[W5_AGENT]; C.gun_step = C.w5[W5_GUN_STEP]; C.registered = C.w5[W5_REGISTERED] != 0;
+        }
         float inertial[15];
         float act[4] = {0.f, 0.f, 0.f, 0.f};
-        auto gun_state_of = [&](int as, float* g) {       // Gun.get_state gun.py:101-113
-            const double wait = fmax(T.cooldown - ((double)C.gstep() - (double)S.last[b + as]), 0.0);
-            const int mx = T.munition > 0 ? T.munition : 1;
-            g[0] = (float)((double)S.ammo[b + as] / (double)mx);
-            g[1] = (float)(wait / T.cooldown);
-            g[2] = C.gun_available(as) ? 1.f : 0.f;
-        };
-        auto gun_state = [&](float* g) { gun_state_of(C.agent, g); };      // of the agent
-        // normalize_inertial_data's clip(v / scale, -1, 1).  The float32 build multiplies in float32 (its inputs are float32
-        // state; one rounding of difference at most), the float64 build keeps the reference's float64 arithmetic.
-        auto nrm = [](double v, double inv_scale) {
-            if constexpr (sizeof(R) == 4) return fminf(fmaxf((float)v * (float)inv_scale, -1.0f), 1.0f);
-            else return (float)fmin(fmax(v * inv_scale, -1.0), 1.0);
-        };
-        const double inv_dome = 1.0 / T.dome;
         bool write_obs = false;
-        // multi-observer reset observation: every wingman re-armed at its new position, velocities/attitude zero
-        auto write_multi_reset = [&]() {
-            for (int P = 0; P < T.n_lw; ++P) {
-                A.mo_present[(long long)env * T.n_lw + P] = 1;
-                float gp3[3]; gun_state_of(P, gp3);
-                float* o = A.mo_inertial + ((long long)env * T.n_lw + P) * 15;
-                const int rp = 3 * (b + P);
-                o[0] = nrm(S.newpos[rp], inv_dome); o[1] = nrm(S.newpos[rp + 1], inv_dome); o[2] = nrm(S.newpos[rp + 2], inv_dome);
-                for (int k = 3; k < 12; ++k) o[k] = 0.f;
-                o[12] = gp3[0]; o[13] = gp3[1]; o[14] = gp3[2];
-            }
-        };
         if (MODE == MODE_STEP) {
             R ag[AG_WORDS];
             {
@@ -982,335 +1564,30 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
             }
             w[W_STEP] += 1; w[W_PHYS_CTR] += T.substeps; w[W_EP_STEPS] += 1;
             C.broadcast_step();                            // advance_step_counter -> AGENT_STEP_BROADCAST
-            double reward = 0.0;
-            bool done = false, lm_alive = false, lw_alive = false, all_over = false;
-            float g[3];
-            const double apx = C.pos(C.agent, 0), apy = C.pos(C.agent, 1), apz = C.pos(C.agent, 2);
-            double* last_dist = A.p.last_dist + (long long)env * T.n_lm;
-            bool caught = false;
-            if (FAM == FAM_STAGE01) {
-                // ================= stage01: compute_reward / compute_termination (level2 modified_v2 :157-191) =================
-                const int lm = T.n_lw;
-                const double dcur = sqrt(C.dist2(lm, 0));
-                double bonus = 0, penalty = 0;
-                if (dcur < C.last_closest()) bonus += 10.0 * norm3((double)ag[AG_UB], (double)ag[AG_VB], (double)ag[AG_WB]);
-                caught = dcur < 0.4;                         // CATCH_DISTANCE (:34)
-                if (caught) bonus += 1000.0;
-                if (dcur > T.dome) penalty += 1000.0;
-                reward = -dcur + bonus - penalty;
-                done = w[W_STEP] > w[W_MAX_STEP];
-                done |= norm3(apx, apy, apz) > T.dome;
-                done |= norm3(C.pos(lm, 0), C.pos(lm, 1), C.pos(lm, 2)) > T.dome;
-                gun_state(g);
-                C.set_last_closest(dcur);
-            } else if (FAM == FAM_STAGE02) {
-                // ================= stage02: L3Stage1.on_step_middle (level3/components/stages.py:144-179) =================
-                int shots = 0, exploded = 0;
-                C.nearest_all();
-                for (int j = 0; j < T.n_lw; ++j) {          // process_shoot_range_invaders + shoot_by_ids (quadcopter_manager.py:155-169)
-                    if (!C.off(j)) continue;
-                    const int tgt = C.nearest_shoot(j);
-                    if (tgt < 0) continue;
-                    if (S.ammo[b + j] == 0) { C.disarm(tgt); ++shots; continue; }      // "LW suicided to kill LM"
-                    if (!C.gun_available(j)) continue;
-                    S.ammo[b + j] -= 1; S.last[b + j] = (R)w[W_STEP];
-                    const double u = hit_uniform(T.k0, T.k1, C.env_id, (uint32_t)w[W_HIT_CTR]);
-                    w[W_HIT_CTR] += 1;
-                    if (u < T.fire_p) { C.disarm(tgt); ++shots; }
-                }
-                for (int j = 0; j < T.n_lw; ++j) {          // process_explosion_range_invaders
-                    if (!C.off(j)) continue;
-                    const int tgt = C.nearest_expl(j);
-                    if (tgt < 0) continue;
-                    C.disarm(j); C.disarm(tgt); ++exploded;
-                }
-                w[W_AGENT_KILLS] += shots; w[W_DEADS] += exploded;
-                gun_state(g);
-                // compute_reward stages.py:234-296 with the closest distances of OffsetHandler (row 0)
-                const int j0 = C.row0();
-                double cur2 = -1.0, last = -1.0;
-                for (int i = T.n_lw; i < D; ++i) {
-                    if (!C.off(i) || j0 < 0) continue;
-                    const double d2 = C.dist2(j0, i);
-                    if (cur2 < 0 || d2 < cur2) cur2 = d2;
-                    const double ld = last_dist[i - T.n_lw];
-                    if (ld == ld && (last < 0 || ld < last)) last = ld;
-                }
-                const double current = sqrt(fmax(cur2, 0.0));
-                const double munition = (double)g[0], reload = (double)fmax(T.cooldown - ((double)w[W_STEP] - (double)S.last[b]), 0.0) / T.cooldown;
-                const bool avail = g[2] == 1.f;
-                double score = (avail || munition == 0.0) ? -current : current * (2 * reload - 1);
-                double bonus = 0, penalty = 0;
-                if (0.01 < last - current && (avail || munition == 0.0))
-                    bonus += 10.0 * norm3((double)ag[AG_UB], (double)ag[AG_VB], (double)ag[AG_WB]);
-                bonus += 1000.0 * shots;
-                penalty += 1000.0 * exploded;
-                const int lw_out = C.count_outside_dome(0, T.n_lw);
-                if (lw_out > 0) penalty += 1000.0;
-                reward = score + bonus - penalty;
-                int n_armed_lw = 0;
-                for (int j = 0; j < T.n_lw; ++j) n_armed_lw += C.live(j) ? 1 : 0;
-                done = w[W_STEP] > w[W_MAX_STEP];            // compute_termination stages.py:298-344
-                done |= lw_out > 0;
-                done |= C.count_outside_dome(T.n_lw, D) > 0;
-                done |= n_armed_lw < T.n_lw;
-            } else if (fam_l5(FAM)) {
-                // ================= level5: Level5C1FusionTask.on_step_middle (level5_c1_fusion_task.py:298-336) =================
-                const int as = C.agent;
-                int agent_shots = 0, ally_shots = 0;
-                C.nearest_all();
-                for (int j = 0; j < T.n_lw; ++j) {          // process_shoot_range_invaders :399-424
-                    if (!C.off(j)) continue;
-                    const int tgt = C.nearest_shoot(j);
-                    if (tgt < 0) continue;
-                    if (!(C.gun_available(j) && S.ammo[b + j] > 0)) continue;
-                    S.ammo[b + j] -= 1; S.last[b + j] = (R)C.gstep();
-                    const double u = hit_uniform(T.k0, T.k1, C.env_id, (uint32_t)w[W_HIT_CTR]);
-                    w[W_HIT_CTR] += 1;
-                    if (u < T.fire_p) { C.disarm(tgt); if (j == as) ++agent_shots; else ++ally_shots; }
-                }
-                int exploded = 0, agent_suicide = 0, ally_suicide = 0;
-                for (int j = 0; j < T.n_lw; ++j) {          // process_explosion_range_invaders :366-397
-                    if (!C.off(j)) continue;
-                    const int tgt = C.nearest_expl(j);
-                    if (tgt < 0) continue;
-                    C.disarm(j); C.disarm(tgt);
-                    if (S.ammo[b + j] == 0 && j == as) ++agent_suicide;
-                    else if (S.ammo[b + j] == 0) ++ally_suicide;
-                    else ++exploded;
-                }
-                w[W_AGENT_KILLS] += agent_shots; w[W_ALLIES_KILLS] += ally_shots; w[W_DEADS] += exploded;
-                for (int i = T.n_lw; i < D; ++i)               // process_invaders_in_origin
-                    if (C.off(i) && sq3(C.pos(i, 0), C.pos(i, 1), C.pos(i, 2)) < 0.2 * 0.2) C.disarm(i);
-                if (FAM == FAM_L5_MULTI && T.l5_eval) reward = 0.0;                   // "EVALUATION TASK DO NOT USES REWARD" (level5_2bt_evaluation_task.py:418-427)
-                else if (T.reward == 2) {
-                    // Level5FusionTask.compute_reward (level5_fusion_task.py:448-555; allies_dead is never passed)
-                    double score, bonus = 0, penalty = 0;
-                    const bool avail = C.gun_available(as);
-                    const int ammo = S.ammo[b + as];
-                    int src = -1;                            // identify_closest_ally on the offsets snapshot
-                    if (C.off(as)) {
-                        int n_all = 0;
-                        for (int j = 0; j < T.n_lw; ++j) n_all += C.off(j) ? 1 : 0;
-                        if (n_all <= 1) src = as;
-                        else {
-                            double bd = 0;
-                            for (int j = 0; j < T.n_lw; ++j) {
-                                if (j == as || !C.off(j)) continue;
-                                const double dd = C.dist2(j, as);
-                                if (src < 0 || dd < bd) { src = j; bd = dd; }
-                            }
-                        }
-                    }
-                    const int target = src >= 0 ? C.nearest_invader(src) : -1;
-                    double tpx = 0, tpy = 0, tpz = 0;
-                    if (target >= 0) { tpx = C.pos(target, 0); tpy = C.pos(target, 1); tpz = C.pos(target, 2); }
-                    const double current = norm3(apx - tpx, apy - tpy, apz - tpz);
-                    if (avail || ammo == 0) score = -current;
-                    else {
-                        score = current;
-                        if (current < 5.0) penalty += ((5.0 - current) / 5.0) * (0.50 * 1000.0);
-                    }
-                    if (!avail && ammo > 0 && (current - C.last_closest()) > 0.01) bonus += 0.10 * 1000.0;
-                    if (agent_shots > 0) bonus += 1.0 * agent_shots * 1000.0;
-                    if (ally_shots > 0 || ally_suicide > 0) bonus += 0.5 * (ally_shots + ally_suicide) * 1000.0;
-                    if (agent_suicide > 0) penalty += 2.0 * agent_suicide * 1000.0;
-                    if (exploded > 0) penalty += 1000.0 * exploded;
-                    if (apz < -5.0) penalty += fmin((-5.0 - apz) / 1.0, 1.0) * 1000.0;
-                    if (C.count_outside_dome(0, T.n_lw) > 0) penalty += 1000.0;
-                    const double d0 = norm3(apx, apy, apz);
-                    if (d0 > T.born - 2) penalty += fmin((d0 - (T.born - 2)) * 1.0, 1000.0);
-                    C.set_last_closest(current);
-                    reward = fmin(fmax(score + bonus - penalty, -3000.0), 3000.0);
-                } else {
-                // compute_reward :434-484: one-shot last_distance, clipped
-                const int target = C.off(as) ? C.nearest_invader(as) : -1;
-                double tpx = 0, tpy = 0, tpz = 0;
-                if (target >= 0) { tpx = C.pos(target, 0); tpy = C.pos(target, 1); tpz = C.pos(target, 2); }
-                const double distance = norm3(apx - tpx, apy - tpy, apz - tpz);
-                double last_distance = __longlong_as_double(((long long)w5[W5_LAST_DIST_HI] << 32) | (unsigned int)w5[W5_LAST_DIST_LO]);
-                if (last_distance != last_distance) {      // ``hasattr(self, 'last_distance')``: set once per env object
-                    last_distance = distance;
-                    const long long bits = __double_as_longlong(distance);
-                    w5[W5_LAST_DIST_LO] = (int32_t)(bits & 0xffffffffLL); w5[W5_LAST_DIST_HI] = (int32_t)(bits >> 32);
-                }
-                if (distance < last_distance) reward += 10.0 * norm3((double)ag[AG_UB], (double)ag[AG_VB], (double)ag[AG_WB]);
-                if (agent_shots > 0) reward += 1.0 * agent_shots * 1000.0;
-                if (agent_suicide > 0) reward -= 2.0 * agent_suicide * 1000.0;
-                reward = fmin(fmax(reward, -3000.0), 3000.0);
-                }
-                if (agent_shots + ally_shots > 0) w[W_MAX_STEP] += T.step_increment;
-                // compute_termination :488-545
-                const int lw_out = C.count_outside_dome(0, T.n_lw);
-                for (int i = T.n_lw; i < D; ++i) lm_alive |= C.live(i);
-                for (int j = 0; j < T.n_lw; ++j) lw_alive |= C.live(j);
-                all_over = !lm_alive && w[W_ROUND] >= T.max_rounds;
-                done = C.gstep() > w[W_MAX_STEP];
-                done |= all_over;
-                done |= lw_out > 0;
-                done |= C.count_outside_dome(T.n_lw, D) > 0;
-                done |= !lw_alive;
-                if (FAM != FAM_L5_MULTI) done |= !C.live(as);
-                if (!(FAM == FAM_L5_MULTI && T.l5_eval)) done |= apz < -5.99;
-                gun_state(g);
-            } else {
-            if (T.reward == 1) {                           // update_building_life (exp02_v2_full_task.py)
-                int cnt = 0;
-                for (int i = T.n_lw + gl; i < D; i += GS)
-                    if (C.off(i) && sq3(C.pos(i, 0), C.pos(i, 1), C.pos(i, 2)) < 0.2 * 0.2) ++cnt;
-                w[W_BUILDING] = max(w[W_BUILDING] - C.gsum(cnt), 0);
-            }
-            // process_shoot_range_invaders :391-412 -> shoot_by_ids -> Gun.shoot
-            int agent_shots = 0, ally_shots = 0;
-            C.nearest_all();
-            for (int j = 0; j < T.n_lw; ++j) {
-                if (!C.off(j)) continue;
-                const int tgt = C.nearest_shoot(j);
-                if (tgt < 0) continue;
-                if (!(C.gun_available(j) && S.ammo[b + j] > 0)) continue;
-                { const int am = S.ammo[b + j]; C.gsync(); S.ammo[b + j] = am - 1; }      // every lane of the group stores the same value
-                S.last[b + j] = (R)w[W_STEP];
-                const double u = hit_uniform(T.k0, T.k1, C.env_id, (uint32_t)w[W_HIT_CTR]);
-                w[W_HIT_CTR] += 1;
-                if (u < T.fire_p) {
-                    C.disarm(tgt); if (j == 0) ++agent_shots; else ++ally_shots;
-                    if (FAM == FAM_DRIVEN) A.p.lw_kills[(long long)env * T.n_lw + j] += 1;       // Evaluation_Task.lw_kills :491-494
-                }
-            }
-            // process_explosion_range_invaders :358-389 (same, now stale, distance matrix)
-            int exploded = 0, ally_suicide = 0, agent_suicide = 0;
-            for (int j = 0; j < T.n_lw; ++j) {
-                if (!C.off(j)) continue;
-                const int tgt = C.nearest_expl(j);
-                if (tgt < 0) continue;
-                C.disarm(j); C.disarm(tgt);
-                if (T.reward == 1) ++exploded;
-                else if (S.ammo[b + j] == 0 && j == 0) ++agent_suicide;
-                else if (S.ammo[b + j] == 0) ++ally_suicide;
-                else ++exploded;
-            }
-            const bool EVAL = FAM == FAM_DRIVEN && T.eval_task;     // Evaluation_Task.on_step_middle evaluation_task.py:383-407
-            if (!EVAL) {
-            w[W_AGENT_KILLS] += agent_shots; w[W_ALLIES_KILLS] += ally_shots; w[W_DEADS] += exploded;
-            C.gsync();
-            for (int i = T.n_lw + gl; i < D; i += GS)       // process_invaders_in_origin :656-659
-                if (C.off(i) && sq3(C.pos(i, 0), C.pos(i, 1), C.pos(i, 2)) < 0.2 * 0.2) C.disarm(i);
-            C.gsync();
-            }
+            const double ap[3] = {C.pos(C.agent, 0), C.pos(C.agent, 1), C.pos(C.agent, 2)};
+            StepMiddle m;
+            if constexpr (FAM == FAM_STAGE01) m = stage01_on_step_middle(C, ag, ap);
+            else if constexpr (FAM == FAM_STAGE02) m = stage02_on_step_middle(C, ag, last_dist);
+            else if constexpr (fam_l5(FAM)) m = level5_on_step_middle(C, ag, ap);
+            else m = stage03_on_step_middle(C, A, env, ag, ap);
 
-            // ---- reward ----
-            gun_state(g);
-            const int lw_out = C.count_outside_dome(0, T.n_lw);
-            if (EVAL) reward = 0.0;                        // "Reward will be deactivated" (evaluation_task.py:512-516)
-            else if (T.reward == 0) {                      // exp02_vFinal_task.py:422-514
-                double bonus = 0, penalty = 0, score;
-                const double munition = (double)S.ammo[b] / (double)(T.munition > 0 ? T.munition : 1);
-                const double reload = fmax(T.cooldown - ((double)w[W_STEP] - (double)S.last[b]), 0.0) / T.cooldown;
-                const bool avail = C.gun_available(0);
-                int src = -1;
-                if (C.off(0)) {
-                    int n_all = 0;
-                    for (int j = 0; j < T.n_lw; ++j) n_all += C.off(j) ? 1 : 0;
-                    if (n_all <= 1) src = 0;
-                    else {
-                        double bd = 0;
-                        for (int j = 1; j < T.n_lw; ++j) {
-                            if (!C.off(j)) continue;
-                            const double dd = C.dist2(j, 0);
-                            if (src < 0 || dd < bd) { src = j; bd = dd; }
-                        }
-                    }
-                }
-                const int target = src >= 0 ? C.nearest_invader(src) : -1;
-                double tpx = 0, tpy = 0, tpz = 0;
-                if (target >= 0) { tpx = C.pos(target, 0); tpy = C.pos(target, 1); tpz = C.pos(target, 2); }
-                const double current = norm3(apx - tpx, apy - tpy, apz - tpz);
-                if (0.01 < C.last_closest() - current && (avail || munition == 0.0))
-                    bonus += T.vel_bonus * norm3((double)ag[AG_UB], (double)ag[AG_VB], (double)ag[AG_WB]);
-                C.set_last_closest(current);
-                score = (avail || munition == 0.0) ? -current : current * (2 * reload - 1);
-                if (agent_shots > 0 || agent_suicide > 0) bonus += (agent_shots + agent_suicide) * 1000.0;
-                if (ally_shots > 0 || ally_suicide > 0) bonus += 0.5 * (ally_shots + ally_suicide) * 1000.0;
-                else if (exploded > 0) penalty += 1000.0 * exploded;
-                if (apz < -5.0) penalty += (-5.0 - apz) / (-5.0 + 6.0) * 1000.0;
-                if (lw_out > 0) penalty += 1000.0;
-                const double d0 = norm3(apx, apy, apz);
-                if (d0 > T.born - 2) penalty += d0 - T.born - 2;
-                reward = score + bonus - penalty;
-            } else {                                       // exp02_v2_full_task.py compute_reward
-                double bonus = 0, penalty = 0;
-                const int shots = agent_shots + ally_shots;
-                const double kills = (double)(w[W_AGENT_KILLS] + w[W_ALLIES_KILLS]);
-                if (shots > 0) bonus += (shots + kills / 10) * 1000.0;
-                if (S.ammo[b] == 0 && exploded > 0) bonus += (shots + kills / 10) * 1000.0;
-                else if (exploded > 0) penalty += 1000.0 * exploded;
-                if (apz < 0.01) penalty += 1000.0;
-                if (lw_out > 0) penalty += 1000.0;
-                if (w[W_BUILDING] < 1) penalty += 1000.0 * (1 - w[W_BUILDING]);
-                const double d0 = norm3(apx, apy, apz);
-                if (d0 > T.born) penalty += d0 - T.born;
-                reward = 0 + bonus - penalty;
-            }
-            if (agent_shots + ally_shots > 0) w[W_MAX_STEP] += T.step_increment;   // increment_max_step :149-152
-
-            // ---- termination :516-568 ----
-            for (int i = T.n_lw + gl; i < D; i += GS) lm_alive |= C.live(i);
-            lm_alive = C.gany(lm_alive);
-            for (int j = 0; j < T.n_lw; ++j) lw_alive |= C.live(j);
-            all_over = !lm_alive && w[W_ROUND] >= T.n_lm;
-            done = w[W_STEP] > w[W_MAX_STEP] && !(EVAL && !T.time_limited);      // evaluation_task.py:522
-            done |= all_over;
-            if (T.reward == 1) done |= w[W_BUILDING] <= 0;
-            done |= lw_out > 0;
-            done |= C.count_outside_dome(T.n_lw, D) > 0;
-            done |= !lw_alive;
-            if (!EVAL) {                                   // a training env stops when its agent dies; the evaluation goes on
-                done |= !C.live(0);
-                done |= apz < (T.reward == 1 ? 0.01 : -5.99);
-            }
-            if (FAM == FAM_DRIVEN && A.lw_info) {                   // compute_info (evaluation_task.py:554-574), between middle and end
-                for (int j = 0; j < T.n_lw; ++j)
-                    reinterpret_cast<int4*>(A.lw_info)[(long long)env * T.n_lw + j] =
-                        make_int4(A.p.lw_kills[(long long)env * T.n_lw + j], C.live(j) ? 1 : 0, S.ammo[b + j], 0);
-            }
-            }   // family
-
-            w[W_EP_RETURN] = __float_as_int(__int_as_float(w[W_EP_RETURN]) + (float)reward);
+            w[W_EP_RETURN] = __float_as_int(__int_as_float(w[W_EP_RETURN]) + (float)m.reward);
             if (lead) {
-                A.reward[env] = (float)reward;
-                A.done[env] = done ? 1 : 0;
+                A.reward[env] = (float)m.reward;
+                A.done[env] = m.done ? 1 : 0;
                 int32_t* info = A.info + (long long)env * INFO_WORDS;
                 reinterpret_cast<int4*>(info)[0] = make_int4(w[W_AGENT_KILLS], w[W_ALLIES_KILLS], w[W_DEADS], w[W_ROUND]);
                 reinterpret_cast<int4*>(info)[1] = make_int4(w[W_BUILDING], w[W_STEP], w[W_MAX_STEP], w[W_EP_STEPS]);
             }
 
-            // ---- observation vector: normalize_inertial_data normalization.py:6-110 + gun_state ----
-            const double i_speed = 1.0 / (1 * 10 * (1000.0 / 3600.0));
-            const double i_pi = 1.0 / 3.141592653589793, i_2pi = 1.0 / (2 * 3.141592653589793);
-            inertial[0] = nrm(apx, inv_dome); inertial[1] = nrm(apy, inv_dome); inertial[2] = nrm(apz, inv_dome);
-            inertial[3] = nrm(ag[AG_UB], i_speed); inertial[4] = nrm(ag[AG_VB], i_speed); inertial[5] = nrm(ag[AG_WB], i_speed);
-            inertial[6] = nrm(ag[AG_ROLL], i_pi); inertial[7] = nrm(ag[AG_PITCH], i_pi); inertial[8] = nrm(ag[AG_YAW], i_pi);
-            inertial[9] = nrm(ag[AG_P], i_2pi); inertial[10] = nrm(ag[AG_Q], i_2pi); inertial[11] = nrm(ag[AG_R], i_2pi);
-            inertial[12] = g[0]; inertial[13] = g[1]; inertial[14] = g[2];
+            // ---- observation vector: normalize_inertial_data + gun_state ----
+            inertial[0] = nrm<R>(ap[0], C.inv_dome); inertial[1] = nrm<R>(ap[1], C.inv_dome); inertial[2] = nrm<R>(ap[2], C.inv_dome);
+            inertial[3] = nrm<R>(ag[AG_UB], INV_SPEED); inertial[4] = nrm<R>(ag[AG_VB], INV_SPEED); inertial[5] = nrm<R>(ag[AG_WB], INV_SPEED);
+            inertial[6] = nrm<R>(ag[AG_ROLL], INV_PI); inertial[7] = nrm<R>(ag[AG_PITCH], INV_PI); inertial[8] = nrm<R>(ag[AG_YAW], INV_PI);
+            inertial[9] = nrm<R>(ag[AG_P], INV_2PI); inertial[10] = nrm<R>(ag[AG_Q], INV_2PI); inertial[11] = nrm<R>(ag[AG_R], INV_2PI);
+            inertial[12] = m.g[0]; inertial[13] = m.g[1]; inertial[14] = m.g[2];
             write_obs = true;
-            if (FAM == FAM_L5_MULTI && !T.l5_eval) {
-                // Level5DumbMultiObs.compute_info (level5_dumb_multiobs.py:112-150): inertial + gun vector of every ARMED
-                // wingman, at the point between on_step_middle and on_step_end
-                for (int P = 0; P < T.n_lw; ++P) {
-                    const bool here = C.live(P);
-                    A.mo_present[(long long)env * T.n_lw + P] = here ? 1 : 0;
-                    if (!here) continue;
-                    const V4<R>* rp = reinterpret_cast<const V4<R>*>(A.p.agent + ((long long)env * T.n_rec + P) * AG_WORDS);
-                    const V4<R> r0 = ld4(rp), r1 = ld4(rp + 1), r2 = ld4(rp + 2);
-                    float gp3[3]; gun_state_of(P, gp3);
-                    float* o = A.mo_inertial + ((long long)env * T.n_lw + P) * 15;
-                    o[0] = nrm(C.pos(P, 0), inv_dome); o[1] = nrm(C.pos(P, 1), inv_dome); o[2] = nrm(C.pos(P, 2), inv_dome);
-                    o[3] = nrm(r0.x, i_speed); o[4] = nrm(r0.y, i_speed); o[5] = nrm(r0.z, i_speed);
-                    o[6] = nrm(r0.w, i_pi); o[7] = nrm(r1.x, i_pi); o[8] = nrm(r1.y, i_pi);
-                    o[9] = nrm(r1.z, i_2pi); o[10] = nrm(r1.w, i_2pi); o[11] = nrm(r2.x, i_2pi);
-                    o[12] = gp3[0]; o[13] = gp3[1]; o[14] = gp3[2];
-                }
-            }
+            if (FAM == FAM_L5_MULTI && !T.l5_eval) write_multi_info(C, A, env);
 
             // LiDAR is rebuilt only while the agent is still a publisher (fused_lidar.py:160-166)
             C.gsync();
@@ -1318,71 +1595,12 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
             C.gsync();
             if (C.live(C.agent)) S.envflag[le] |= EF_LIDAR;
 
-            if (FAM == FAM_STAGE01) {
-                // replace_invader_if_close + update_last_distance (:148-155,193-198)
-                if (caught) {
-                    const int lm = T.n_lw;
-                    double p[3];
-                    w[W_AGENT_KILLS] += 1;
-                    C.u3(p);
-                    C.replace_invader_stage01(lm, p);
-                    C.set_last_closest(norm3((double)S.newpos[3 * (b + lm)] - apx, (double)S.newpos[3 * (b + lm) + 1] - apy,
-                                             (double)S.newpos[3 * (b + lm) + 2] - apz));
-                }
-            } else if (FAM == FAM_STAGE02) {
-                // disarmed munitions reappear at once (stages.py:170-174,370-376); on_step_end: last offsets := current
-                int n_dead = 0;
-                for (int i = T.n_lw; i < D; ++i) n_dead += C.live(i) ? 0 : 1;
-                if (n_dead > 0) {
-                    const uint32_t base = (uint32_t)w[W_SPAWN_CTR];
-                    int k = 0;
-                    for (int i = T.n_lw; i < D; ++i) {
-                        if (C.live(i)) continue;
-                        double p[3];
-                        C.gen3(base, n_dead, k++, T.respawn_r0, T.respawn_r1, p);
-                        C.replace(i, p[0], p[1], p[2]);
-                        C.arm(i);
-                    }
-                    w[W_SPAWN_CTR] += 3 * n_dead;
-                }
-                const int j0 = C.row0();
-                const double qnan = __longlong_as_double(0x7ff8000000000000LL);
-                for (int i = T.n_lw; i < D; ++i)
-                    last_dist[i - T.n_lw] = (C.off(i) && j0 >= 0) ? sqrt(C.dist2(j0, i)) : qnan;
-            } else if (fam_l5(FAM)) {
-                // Task.on_step_end :338-350 + advance_round :139-152 (setup_round disarms every munition first: the id
-                // clash zeroes the guns' step until the next broadcast)
-                if (!all_over && !lm_alive && lw_alive) {
-                    w[W_ROUND] += (w[W_ROUND] < T.max_rounds) ? 1 : T.max_rounds;
-                    C.setup_round5(w[W_ROUND]);
-                    C.refresh_offsets();
-                    S.envflag[le] |= EF_NAV_RESET;
-                }
-                if (T.l5_base) {
-                    // base env: a dead agent still runs read_data -> six empty spheres; the candidates of
-                    // get_random_neighborhood are the wingmen with an open buffer in the agent's ring at ITS read_data of
-                    // the first compute_observation call: the armed ones, the ones that died before this step (their LiDAR
-                    // broadcasts re-opened it) and, of those that died in this step, the ones in front of the agent
-                    int cand = 0;
-                    for (int P = 0; P < T.n_lw; ++P)
-                        if (C.live(P) || !(S.ev[b + P] & EV_WAS_ARMED) || P < C.agent) cand |= 1 << P;
-                    w5[W5_STACK_MODE] = (C.live(C.agent) ? STACK_BUILD : STACK_EMPTY) | (cand << 8);
-                    w5[W5_OBS_CALL] += 3;
-                } else {
-                    w5[W5_STACK_MODE] = (FAM == FAM_L5_MULTI || C.live(C.agent)) ? STACK_BUILD : STACK_KEEP;   // a dead agent's flight state keeps its last stack
-                    w5[W5_OBS_CALL] += 1;
-                }
-                S.envflag[le] |= (w[W_STEP] % RING) << 8;     // ring slot of this step for the feature pass
-            } else
-            // ---- Task.on_step_end :320-332 + advance_round :154-174 ----
-            if (!all_over && !lm_alive && lw_alive) {
-                w[W_ROUND] += (w[W_ROUND] < T.n_lm) ? 1 : T.n_lm;
-                C.setup_round(w[W_ROUND]);
-                C.refresh_offsets();
-                S.envflag[le] |= EF_NAV_RESET;
-            }
+            if constexpr (FAM == FAM_STAGE01) stage01_on_step_end(C, m, ap);
+            else if constexpr (FAM == FAM_STAGE02) stage02_on_step_end(C, last_dist);
+            else if constexpr (fam_l5(FAM)) level5_on_step_end(C, m);
+            else if (!m.all_over && !m.lm_alive && m.lw_alive) C.advance_round();    // Task.on_step_end :320-332
             // ---- VecEnv auto-reset (SB3 DummyVecEnv.step_wait semantics) ----
-            if (done && T.auto_reset) {
+            if (m.done && T.auto_reset) {
                 if (A.term_inertial && lead) for (int k = 0; k < 15; ++k) A.term_inertial[(long long)env * 15 + k] = inertial[k];
                 if (A.term_last_action && lead) reinterpret_cast<float4*>(A.term_last_action)[env] = make_float4(act[0], act[1], act[2], act[3]);
                 if (A.stats && lead) {
@@ -1391,44 +1609,28 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
                     atomicAdd(A.stats + 4, (double)w[W_ALLIES_KILLS]); atomicAdd(A.stats + 5, (double)w[W_DEADS]);
                     atomicAdd(A.stats + 6, (double)w[W_ROUND]);
                 }
-                if (fam_l5(FAM)) { C.reset_env5(); w5[W5_STACK_MODE] = STACK_EMPTY; w5[W5_OBS_CALL] += T.l5_base ? 3 : 1; S.envflag[le] &= ~EF_LIDAR; }
-                else if (FAM == FAM_STAGE01) C.reset_env_stage01(); else if (FAM == FAM_STAGE02) C.reset_env_stage02(last_dist); else C.reset_env(lw_init);
+                C.reset_task(lw_init, last_dist);
+                if (fam_l5(FAM)) S.envflag[le] &= ~EF_LIDAR;
                 // level5 C1 reports agent.last_action, the command the drone keeps across the reset (quadcopter.py:415-419);
                 // the base level5 env reports its own last_action, zeroed by init_globals (level5_envrionment.py:153-155)
                 if (!fam_l5(FAM) || T.l5_base) act[0] = act[1] = act[2] = act[3] = 0.f;
-                const int ra = 3 * (b + C.agent);
-                inertial[0] = nrm(S.newpos[ra], inv_dome); inertial[1] = nrm(S.newpos[ra + 1], inv_dome);
-                inertial[2] = nrm(S.newpos[ra + 2], inv_dome);
-                for (int k = 3; k < 12; ++k) inertial[k] = 0.f;
-                gun_state(g); inertial[12] = g[0]; inertial[13] = g[1]; inertial[14] = g[2];
-                if (FAM == FAM_L5_MULTI && !T.l5_eval) write_multi_reset();
+                reset_inertial(C, C.agent, inertial);
+                if (FAM == FAM_L5_MULTI && !T.l5_eval) write_multi_reset(C, A, env);
             }
         } else {
             // ---- MODE_RESET: Env.__init__ on first use, then Env.reset for the masked envs ----
             const bool masked = A.reset_mask == nullptr || A.reset_mask[env] != 0;
             const bool first = w[W_INIT] == 0;
-            double* last_dist = A.p.last_dist + (long long)env * T.n_lm;
             if (first) {
-                for (int k = 0; k < ENV_WORDS; ++k) w[k] = 0;
-                if (fam_l5(FAM)) {
-                    for (int k = 0; k < ENV5_WORDS; ++k) w5[k] = 0;
-                    w5[W5_LAST_DIST_LO] = 0; w5[W5_LAST_DIST_HI] = 0x7ff80000;     // NaN: last_distance not set yet
-                    C.env_init5();
-                } else if (FAM == FAM_STAGE01) C.env_init_stage01(); else if (FAM == FAM_STAGE02) C.env_init_stage02(last_dist); else C.env_init(lw_init);
+                C.init_task(lw_init, last_dist);
                 S.envflag[le] |= EF_FIRST;                  // first use: start from an empty sphere
             }
-            if (fam_l5(FAM)) w5[W5_STACK_MODE] = STACK_KEEP;
+            if (fam_l5(FAM)) C.w5[W5_STACK_MODE] = STACK_KEEP;
             if (masked || first) {
-                if (fam_l5(FAM)) { C.reset_env5(); w5[W5_STACK_MODE] = STACK_EMPTY; w5[W5_OBS_CALL] += T.l5_base ? 3 : 1; }
-                else if (FAM == FAM_STAGE01) C.reset_env_stage01(); else if (FAM == FAM_STAGE02) C.reset_env_stage02(last_dist); else C.reset_env(lw_init);
-                float g[3]; gun_state(g);
-                const int ra = 3 * (b + C.agent);
-                inertial[0] = nrm(S.newpos[ra], inv_dome); inertial[1] = nrm(S.newpos[ra + 1], inv_dome);
-                inertial[2] = nrm(S.newpos[ra + 2], inv_dome);
-                for (int k = 3; k < 12; ++k) inertial[k] = 0.f;
-                inertial[12] = g[0]; inertial[13] = g[1]; inertial[14] = g[2];
+                C.reset_task(lw_init, last_dist);
+                reset_inertial(C, C.agent, inertial);
                 write_obs = true;
-                if (FAM == FAM_L5_MULTI && !T.l5_eval) write_multi_reset();
+                if (FAM == FAM_L5_MULTI && !T.l5_eval) write_multi_reset(C, A, env);
             }
         }
         if (write_obs && lead) {
@@ -1437,7 +1639,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
             if (!(MODE == MODE_RESET && fam_l5(FAM) && !T.l5_base && !(S.envflag[le] & EF_FIRST)))      // level5 C1 reset keeps agent.last_action
                 reinterpret_cast<float4*>(A.obs_last_action)[env] = make_float4(act[0], act[1], act[2], act[3]);
         }
-        if (fam_l5(FAM)) { w5[W5_AGENT] = C.agent; w5[W5_GUN_STEP] = C.gun_step; w5[W5_REGISTERED] = C.registered ? 1 : 0; }
+        if (fam_l5(FAM)) { C.w5[W5_AGENT] = C.agent; C.w5[W5_GUN_STEP] = C.gun_step; C.w5[W5_REGISTERED] = C.registered ? 1 : 0; }
         int4* wp = reinterpret_cast<int4*>(A.p.env + (long long)env * ENV_WORDS);
 #pragma unroll
         for (int k = 0; k < 4; ++k) if (lead) wp[k] = make_int4(w[4 * k], w[4 * k + 1], w[4 * k + 2], w[4 * k + 3]);
@@ -1462,7 +1664,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
                 const uint32_t base = (uint32_t)jp[0];
                 const int n = jp[1], i = jp[2];
                 double p[3];
-                spawn_point(T, T.env_offset + (uint32_t)(env0 + env_of(s)), base, n, i, T.born, p);
+                spawn_point(T, T.env_offset + (uint32_t)(env0 + A.env_of(s)), base, n, i, T.born, p);
                 S.newpos[3 * s] = (R)p[0]; S.newpos[3 * s + 1] = (R)p[1]; S.newpos[3 * s + 2] = (R)p[2];
             }
         }
@@ -1478,7 +1680,7 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
     // imu[parity] / items[parity], whose count the host zeroed before this launch.
     for (int s = S_LO + lane; s < S_HI; s += 32) {
         {
-            const int le = env_of(s);
+            const int le = A.env_of(s);
             const int ev = S.ev[s];
             const bool live = ev & EV_LIVE;
             V4<R>* gp = A.p.state + slot0 + s;
@@ -1509,223 +1711,18 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
 
     DC_STAMP(4);
     if (MODE == MODE_STEP) asm volatile("griddepcontrol.launch_dependents;");     // the next step's dyn_kernel waits for the whole grid
-    // ---- P4: projection LiDAR of the agent (slot 0) over the entities alive after engagement --------
-    const int ch = T.lidar == 0 ? 3 : 2;
-    const int per_env = (fam_l5(FAM) ? N_STACK * 3 : ch) * N_CELLS;
-    double* s_rn = S.rn;
-    int* s_cell = S.cell;
+    // ---- P4: LiDAR over the entities alive after engagement --------
     if (MODE == MODE_STEP && fam_l5(FAM)) {
-        // level5: every armed wingman P runs FusedLIDAR.update_data (level5_c1_fusion_environment.py:25-26); what the
-        // agent's ring keeps of it -- P's float32 pose and the kept features (r_n, theta, phi float64, type, id) -- goes
-        // to ring slot step % 10.  stack_kernel assembles the observation from the ring afterwards.
-        for (int P = 0; P < T.n_lw; ++P) {
-            for (int s = S_LO + lane; s < S_HI; s += 32) { s_cell[s] = -1; s_rn[s] = 1.0; }
-            int n_proj = 0;
-            for (int s = S_LO + lane; s < S_HI + lane; s += 32) {
-                bool pred = false;
-                if (s < S_HI) {
-                    const int le = env_of(s), d = s - le * D;
-                    pred = d != P && (S.ev[s] & EV_MID) && (S.ev[le * D + P] & EV_MID) && (S.envflag[le] & EF_LIDAR);
-                }
-                n_proj = warp_compact(pred, s, s_list, n_proj);
-            }
-            __syncwarp();
-            for (int i = lane; i < n_proj; i += 32) {
-                const int s = s_list[i];
-                const int le = env_of(s), o = le * D + P;
-                const R* rec = A.p.agent + ((long long)(env0 + le) * T.n_rec + P) * AG_WORDS;
-                const LidarHit h = lidar_project_one(0, 2 * T.dome, (double)(float)S.imu[3 * o], (double)(float)S.imu[3 * o + 1],
-                                                     (double)(float)S.imu[3 * o + 2], (double)(float)rec[AG_QX], (double)(float)rec[AG_QY],
-                                                     (double)(float)rec[AG_QZ], (double)(float)rec[AG_QW],
-                                                     (double)(float)S.imu[3 * s], (double)(float)S.imu[3 * s + 1], (double)(float)S.imu[3 * s + 2]);
-                s_cell[s] = h.cell; s_rn[s] = h.rn; S.ang[2 * s] = h.theta; S.ang[2 * s + 1] = h.phi;
-            }
-            __syncwarp();
-            for (int s = S_LO + lane; s < S_HI; s += 32) {
-                const int le = env_of(s), d = s - le * D, b = le * D;
-                if (!(S.envflag[le] & EF_LIDAR) || !(S.ev[b + P] & EV_MID)) continue;
-                const long long entry = ((long long)(env0 + le) * T.n_lw + P) * RING + ((S.envflag[le] >> 8) & 15);
-                const bool win = lidar_wins(0, d, D, s_cell + b, s_rn + b);
-                A.p.ring_meta[entry * D + d] = win ? (s_cell[s] | ((d < T.n_lw ? 3 : 1) << 16)) : -1;
-                if (win) {
-                    double* f = A.p.ring_feat + (entry * D + d) * 3;
-                    f[0] = s_rn[s]; f[1] = S.ang[2 * s]; f[2] = S.ang[2 * s + 1];
-                }
-                if (d == P) {
-                    const R* rec = A.p.agent + ((long long)(env0 + le) * T.n_rec + P) * AG_WORDS;
-                    float4* pp = reinterpret_cast<float4*>(A.p.ring_pose + entry * 8);
-                    pp[0] = make_float4((float)S.imu[3 * s], (float)S.imu[3 * s + 1], (float)S.imu[3 * s + 2], (float)rec[AG_QX]);
-                    pp[1] = make_float4((float)rec[AG_QY], (float)rec[AG_QZ], (float)rec[AG_QW], 0.f);
-                }
-            }
-            __syncwarp();
-        }
+        level5_ring_pass(A, S, env0, S_LO, S_HI, lane);
     } else if (MODE == MODE_STEP) {
-        if (A.lidar_ids) {
-            int32_t* idp = A.lidar_ids + (long long)(env0 + LE_LO) * N_CELLS;
-            for (int i = lane; i < (LE_HI - LE_LO) * N_CELLS; i += 32) idp[i] = -1;   // features = [] when skipped
-        }
-        // The sphere lives in the caller's obs_lidar buffer across steps and is maintained INCREMENTALLY:
-        // the cells held by the previous step's hits (remembered in sphere_desc, parked in S.rn by P0) go back to
-        // 1.0, then the new hits are written -- bit-identical to rebuilding LIDARSpec.empty_sphere() + add_features,
-        // at a few dozen bytes per env instead of 4 KB.  When the agent is no longer a publisher nothing is
-        // touched: the reference keeps the previous sphere (fused_lidar.py:160-166).
-        // FAM_DRIVEN, wingman 0 flown by a policy: its FusedLIDAR keeps ONE sphere that the step-start update (lw_obs_kernel,
-        // dc_buffers.lw_lidar[:,0], SimPtrs::lw_desc) and this end-of-step update both overwrite.  When this update is
-        // skipped (wingman 0 is no publisher any more) the observation shows that object as the step-start update left it.
-        const bool SYNC0 = FAM == FAM_DRIVEN && A.lw_lidar && (T.lw_driver[0] == DRV_NN || T.lw_driver[0] == DRV_NN_ALLY);
-        if (!SYNC0) {
-            // One pass over the warp's slots: a slot whose entity held a cell of the previous sphere gives it back (cell and
-            // remembered-hit record), and the entities that can mark a cell now -- alive after the engagement, not the
-            // observer, observer still a publisher -- are compacted so that the float64 projection runs on full warps.
-            int n_proj = 0;
-            for (int s = S_LO + lane; s < S_HI + lane; s += 32) {
-                bool pred = false;
-                if (s < S_HI) {
-                    const int le = env_of(s), d = s - le * D;
-                    const bool on = S.envflag[le] & EF_LIDAR;
-                    const int oc = (int)reinterpret_cast<const long long*>(S.rn)[s];
-                    if (on && oc >= 0) {
-                        float* sph = A.obs_lidar + (long long)(env0 + le) * per_env;
-                        sph[oc] = 1.0f; sph[N_CELLS + oc] = 1.0f;
-                        if (ch == 3) sph[2 * N_CELLS + oc] = 1.0f;
-                        A.p.sphere_desc[slot0 + s] = make_int2(-1, __float_as_int(1.0f));
-                    }
-                    pred = d != 0 && (S.ev[s] & EV_MID) && on;
-                    s_cell[s] = -1;
-                }
-                n_proj = warp_compact(pred, s, s_list, n_proj);
-            }
-            __syncwarp();                                 // un-write before write: two slots of an env may name the same cell
-            DC_STAMP(6);
-            for (int i = lane; i < n_proj; i += 32) {
-                const int s = s_list[i];
-                const int b = env_of(s) * D;
-                const R* ag = A.p.agent + (long long)(env0 + env_of(s)) * T.n_rec * AG_WORDS;      // record of wingman 0
-                if (T.lidar == 0 && sizeof(R) == 4) {    // float32 build: float32 projection, exact cell (lidar_cell_fused_f32)
-                    int c; float rn;
-                    lidar_cell_fused_f32((float)(2 * T.dome), (float)S.imu[3 * b], (float)S.imu[3 * b + 1], (float)S.imu[3 * b + 2],
-                                         (float)ag[AG_QX], (float)ag[AG_QY], (float)ag[AG_QZ], (float)ag[AG_QW],
-                                         (float)S.imu[3 * s], (float)S.imu[3 * s + 1], (float)S.imu[3 * s + 2], &c, &rn);
-                    s_cell[s] = c; s_rn[s] = (double)rn;
-                } else if (T.lidar == 0) {    // float32 snapshot (perception_snapshot.py:91-110)
-                    int c; double rn;
-                    lidar_cell_fused(2 * T.dome, (double)(float)S.imu[3 * b], (double)(float)S.imu[3 * b + 1],
-                                     (double)(float)S.imu[3 * b + 2], (double)(float)ag[AG_QX], (double)(float)ag[AG_QY],
-                                     (double)(float)ag[AG_QZ], (double)(float)ag[AG_QW],
-                                     (double)(float)S.imu[3 * s], (double)(float)S.imu[3 * s + 1], (double)(float)S.imu[3 * s + 2], &c, &rn);
-                    s_cell[s] = c; s_rn[s] = rn;
-                } else {
-                    const LidarHit h = lidar_project_one(1, 2 * T.dome, (double)S.imu[3 * b], (double)S.imu[3 * b + 1], (double)S.imu[3 * b + 2],
-                                                         (double)ag[AG_QX], (double)ag[AG_QY], (double)ag[AG_QZ], (double)ag[AG_QW],
-                                                         (double)S.imu[3 * s], (double)S.imu[3 * s + 1], (double)S.imu[3 * s + 2]);
-                    s_cell[s] = h.cell; s_rn[s] = h.rn;
-                }
-            }
-            __syncwarp();
-            DC_STAMP(7);
-            // winners among the projected entities (full warps): into the sphere, and remembered for the next step's
-            // un-write (and for the sparse host transfer)
-            for (int i = lane; i < n_proj; i += 32) {
-                const int s = s_list[i];
-                const int le = env_of(s), d = s - le * D, b = le * D;
-                if (!lidar_wins(T.lidar, d, D, s_cell + b, s_rn + b)) continue;
-                const int c = s_cell[s];
-                const float rnf = (float)s_rn[s];
-                float* sph = A.obs_lidar + (long long)(env0 + le) * per_env;
-                sph[c] = rnf;
-                sph[N_CELLS + c] = (float)((d < T.n_lw ? 3.0 : 1.0) / 5.0);  // EntityType value / 5
-                if (ch == 3) sph[2 * N_CELLS + c] = 0.1f;                     // normalised age 1/10 (lidar_buffer.py:98-99)
-                if (A.lidar_ids) A.lidar_ids[(long long)(env0 + le) * N_CELLS + c] = d;
-                A.p.sphere_desc[slot0 + s] = make_int2(c, __float_as_int(rnf));
-            }
-        } else {
-            for (int s = S_LO + lane; s < S_HI; s += 32) {
-                const int le = env_of(s);
-                if (!(S.envflag[le] & EF_LIDAR) && !SYNC0) continue;
-                const int oc = (int)reinterpret_cast<const long long*>(S.rn)[s];
-                if (oc < 0) continue;
-                float* sph = A.obs_lidar + (long long)(env0 + le) * per_env;
-                sph[oc] = 1.0f; sph[N_CELLS + oc] = 1.0f;
-                if (ch == 3) sph[2 * N_CELLS + oc] = 1.0f;
-            }
-            __syncwarp();                                     // un-write before write: two slots of an env may name the same cell
-            if (SYNC0) {
-                for (int s = S_LO + lane; s < S_HI; s += 32) {
-                    const int le = env_of(s), d = s - le * D;
-                    if (S.envflag[le] & EF_LIDAR) continue;
-                    const int2 h = A.p.lw_desc[((long long)(env0 + le) * T.n_lw + 0) * D + d];
-                    A.p.sphere_desc[slot0 + s] = make_int2(h.x >= 0 ? h.x : -1, h.x >= 0 ? h.y : __float_as_int(1.0f));
-                    if (h.x < 0) continue;
-                    float* sph = A.obs_lidar + (long long)(env0 + le) * per_env;
-                    sph[h.x] = __int_as_float(h.y);
-                    sph[N_CELLS + h.x] = (float)((d < T.n_lw ? 3.0 : 1.0) / 5.0);
-                    if (ch == 3) sph[2 * N_CELLS + h.x] = 0.1f;
-                }
-            }
-            // entities that can mark a cell: alive after the engagement, not the observer, observer still a
-            // publisher.  They are compacted so that the float64 projection runs on full warps.
-            int n_proj = 0;
-            for (int s = S_LO + lane; s < S_HI + lane; s += 32) {
-                bool pred = false;
-                if (s < S_HI) {
-                    const int le = env_of(s), d = s - le * D;
-                    pred = d != 0 && (S.ev[s] & EV_MID) && (S.envflag[le] & EF_LIDAR);
-                    s_cell[s] = -1;
-                }
-                n_proj = warp_compact(pred, s, s_list, n_proj);
-            }
-            __syncwarp();
-            for (int i = lane; i < n_proj; i += 32) {
-                const int s = s_list[i];
-                const int le = env_of(s), b = le * D;
-                const R* ag = A.p.agent + (long long)(env0 + le) * T.n_rec * AG_WORDS;      // record of wingman 0 (n_rec = n_lw in FAM_DRIVEN)
-                if (T.lidar == 0) {    // float32 snapshot (perception_snapshot.py:91-110)
-                    int c; double rn;
-                    lidar_cell_fused(2 * T.dome, (double)(float)S.imu[3 * b], (double)(float)S.imu[3 * b + 1],
-                                     (double)(float)S.imu[3 * b + 2], (double)(float)ag[AG_QX], (double)(float)ag[AG_QY],
-                                     (double)(float)ag[AG_QZ], (double)(float)ag[AG_QW],
-                                     (double)(float)S.imu[3 * s], (double)(float)S.imu[3 * s + 1], (double)(float)S.imu[3 * s + 2], &c, &rn);
-                    s_cell[s] = c; s_rn[s] = rn;
-                } else {
-                    const LidarHit h = lidar_project_one(1, 2 * T.dome, (double)S.imu[3 * b], (double)S.imu[3 * b + 1], (double)S.imu[3 * b + 2],
-                                                         (double)ag[AG_QX], (double)ag[AG_QY], (double)ag[AG_QZ], (double)ag[AG_QW],
-                                                         (double)S.imu[3 * s], (double)S.imu[3 * s + 1], (double)S.imu[3 * s + 2]);
-                    s_cell[s] = h.cell; s_rn[s] = h.rn;
-                }
-            }
-            __syncwarp();
-            // winners among the projected entities (full warps), written into the sphere
-            for (int i = lane; i < n_proj; i += 32) {
-                const int s = s_list[i];
-                const int le = env_of(s), d = s - le * D, b = le * D;
-                if (!lidar_wins(T.lidar, d, D, s_cell + b, s_rn + b)) continue;
-                S.ev[s] |= EV_LWIN;
-                const int c = s_cell[s];
-                float* sph = A.obs_lidar + (long long)(env0 + le) * per_env;
-                sph[c] = (float)s_rn[s];
-                sph[N_CELLS + c] = (float)((d < T.n_lw ? 3.0 : 1.0) / 5.0);  // EntityType value / 5
-                if (ch == 3) sph[2 * N_CELLS + c] = 0.1f;                     // normalised age 1/10 (lidar_buffer.py:98-99)
-                if (A.lidar_ids) A.lidar_ids[(long long)(env0 + le) * N_CELLS + c] = d;
-            }
-            __syncwarp();
-            // what the sphere now holds, per slot, for the next step's un-write (and for the sparse host transfer)
-            for (int s = S_LO + lane; s < S_HI; s += 32) {
-                if (!(S.envflag[env_of(s)] & EF_LIDAR)) continue;
-                const bool win = S.ev[s] & EV_LWIN;
-                A.p.sphere_desc[slot0 + s] = make_int2(win ? s_cell[s] : -1, __float_as_int(win ? (float)s_rn[s] : 1.0f));
-            }
-        }
+        if (FAM == FAM_DRIVEN && A.lw_lidar && (T.lw_driver[0] == DRV_NN || T.lw_driver[0] == DRV_NN_ALLY))
+            agent_sphere_pass<R, true>(A, S, env0, LE_LO, LE_HI, S_LO, S_HI, lane);
+        else
+            agent_sphere_pass<R, false>(A, S, env0, LE_LO, LE_HI, S_LO, S_HI, lane);
         DC_STAMP(5);
         DC_TL_END(A.tl_slot);
     } else {
-        for (int e = LE_LO; e < LE_HI; ++e) {               // first use of an env: empty sphere
-            if (!(S.envflag[e] & EF_FIRST)) continue;
-            float* sph = A.obs_lidar + (long long)(env0 + e) * per_env;
-            for (int f = lane; f < per_env; f += 32) sph[f] = 1.0f;
-            if (A.lidar_ids) for (int f = lane; f < N_CELLS; f += 32) A.lidar_ids[(long long)(env0 + e) * N_CELLS + f] = -1;
-            for (int f = lane; f < D; f += 32) A.p.sphere_desc[slot0 + (long long)e * D + f] = make_int2(-1, 0);
-        }
+        first_use_sphere<R, FAM>(A, S, env0, LE_LO, LE_HI, lane);
     }
 }
 
