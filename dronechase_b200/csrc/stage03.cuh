@@ -172,6 +172,49 @@ __device__ __forceinline__ double sq3(double x, double y, double z) { return x *
 // ================================================================================================
 // dyn_kernel
 // ================================================================================================
+// The state words a drone carries through dyn_kernel's substeps, listed once in move(): quads 0-4 (position, quaternion,
+// velocity, body rate, throttle), then the PID words.  load() and store() are move(); the prefetch skips what move() skips.
+template <typename R, int FAM, bool BUILTIN> struct DroneWords {
+    static constexpr int NPID = FAM == FAM_STAGE01 ? 6 : 5;                       // quad 10 holds the mode-7 words
+    // The folded cf2x model (BUILTIN) has ki = kd = 0 in the angle loop and kd = 0 in the yaw-rate loop: of the 20 mode-6
+    // controller words only 11 are ever read -- ang_vel integrators 0..2 and previous errors 3, 4, lin_vel 12..15, z_vel 16, 17.
+    // The others are neither loaded nor written back (they keep what the last reset left): 9 registers less across the
+    // substep loop and 56 bytes less traffic per drone and direction.
+    static constexpr bool PID_DIET = BUILTIN && sizeof(R) == 4 && FAM != FAM_STAGE01;
+    __device__ __forceinline__ static void prefetch(const V4<R>* gp, long long stride) {
+#pragma unroll
+        for (int q = 0; q < 10; ++q)                         // quad 10 is loaded but not prefetched
+            if (!(PID_DIET && q == 7)) asm volatile("prefetch.global.L2 [%0];" :: "l"(gp + q * stride));
+    }
+    // one 16-byte quad (d == nullptr: its fourth word is not carried, stored as 0), or one word on its own
+    template <bool ST> __device__ __forceinline__ static void quad(V4<R>* p, R& a, R& b, R& c, R* d) {
+        if constexpr (ST) st4(p, V4<R>{a, b, c, d ? *d : (R)0});
+        else { const V4<R> v = ld4(p); a = v.x; b = v.y; c = v.z; if (d) *d = v.w; }
+    }
+    template <bool ST> __device__ __forceinline__ static void word(R* p, R& a) { if constexpr (ST) *p = a; else a = *p; }
+    template <bool ST> __device__ __forceinline__ static void move(Drone<R>& st, V4<R>* gp, long long stride) {
+        quad<ST>(gp, st.px, st.py, st.pz, nullptr);
+        quad<ST>(gp + stride, st.qx, st.qy, st.qz, &st.qw);
+        quad<ST>(gp + 2 * stride, st.vx, st.vy, st.vz, nullptr);
+        quad<ST>(gp + 3 * stride, st.wx, st.wy, st.wz, nullptr);
+        quad<ST>(gp + 4 * stride, st.thr[0], st.thr[1], st.thr[2], &st.thr[3]);
+        if constexpr (PID_DIET) {
+            if constexpr (!ST)
+#pragma unroll
+                for (int k = 0; k < 24; ++k) st.pid[k] = 0;
+            quad<ST>(gp + 5 * stride, st.pid[0], st.pid[1], st.pid[2], &st.pid[3]);
+            word<ST>(reinterpret_cast<R*>(gp + 6 * stride), st.pid[4]);
+            quad<ST>(gp + 8 * stride, st.pid[12], st.pid[13], st.pid[14], &st.pid[15]);
+            word<ST>(reinterpret_cast<R*>(gp + 9 * stride), st.pid[16]); word<ST>(reinterpret_cast<R*>(gp + 9 * stride) + 1, st.pid[17]);
+        } else {
+#pragma unroll
+            for (int k = 0; k < NPID; ++k) quad<ST>(gp + (5 + k) * stride, st.pid[4 * k], st.pid[4 * k + 1], st.pid[4 * k + 2], &st.pid[4 * k + 3]);
+        }
+    }
+    __device__ __forceinline__ static void load(Drone<R>& st, V4<R>* gp, long long stride) { move<false>(st, gp, stride); }
+    __device__ __forceinline__ static void store(Drone<R>& st, V4<R>* gp, long long stride) { move<true>(st, gp, stride); }
+};
+
 // FAM: FAM_* above.  BUILTIN (float32 only): the drone model is the built-in cf2x, folded into the code (quad_dynamics.cuh Cf2x).
 template <typename R, bool NOISE, int FAM, bool BUILTIN = false>
 __global__ void __launch_bounds__(DYN_THREADS, (sizeof(R) == 4 ? DC_DYN_MIN_BLOCKS : 2)) dyn_kernel(const StepArgs<R> A) {
@@ -194,14 +237,9 @@ __global__ void __launch_bounds__(DYN_THREADS, (sizeof(R) == 4 ? DC_DYN_MIN_BLOC
     const V4<R>* snap = A.p.imu[par];
     // The pilots below walk a chain of dependent loads (flags -> neighbour snapshots -> formation point) before the drone's
     // own state is touched: ask for the state lines now so that they arrive under that chain (no registers held).
-    {
-        const V4<R>* pp = A.p.state + s;
-#pragma unroll
-        for (int q = 0; q < 10; ++q)
-            if (!(BUILTIN && sizeof(R) == 4 && FAM != FAM_STAGE01 && q == 7))
-                asm volatile("prefetch.global.L2 [%0];" :: "l"(pp + q * stride));
-        asm volatile("prefetch.global.L2 [%0];" :: "l"(A.p.env + (long long)env * ENV_WORDS));
-    }
+    using Words = DroneWords<R, FAM, BUILTIN>;
+    Words::prefetch(A.p.state + s, stride);
+    asm volatile("prefetch.global.L2 [%0];" :: "l"(A.p.env + (long long)env * ENV_WORDS));
     const V4<R> own = ld4(snap + s);                  // imu position of the previous step | last_fired
     const double mx = own.x, my = own.y, mz = own.z;
 
@@ -343,31 +381,7 @@ __global__ void __launch_bounds__(DYN_THREADS, (sizeof(R) == 4 ? DC_DYN_MIN_BLOC
     // ---- dynamic state: 16-byte loads (quads 0..9), 16 substeps in registers, write-back ------------
     Drone<R> st;
     V4<R>* gp = A.p.state + s;
-    V4<R> v = ld4(gp); st.px = v.x; st.py = v.y; st.pz = v.z;
-    v = ld4(gp + stride); st.qx = v.x; st.qy = v.y; st.qz = v.z; st.qw = v.w;
-    v = ld4(gp + 2 * stride); st.vx = v.x; st.vy = v.y; st.vz = v.z;
-    v = ld4(gp + 3 * stride); st.wx = v.x; st.wy = v.y; st.wz = v.z;
-    v = ld4(gp + 4 * stride); st.thr[0] = v.x; st.thr[1] = v.y; st.thr[2] = v.z; st.thr[3] = v.w;
-    constexpr int NPID = FAM == FAM_STAGE01 ? 6 : 5;                              // quad 10 holds the mode-7 words
-    // The folded cf2x model (BUILTIN) has ki = kd = 0 in the angle loop and kd = 0 in the yaw-rate loop: of the 20 mode-6
-    // controller words only 11 are ever read -- ang_vel integrators 0..2 and previous errors 3, 4, lin_vel 12..15, z_vel 16, 17.
-    // The others are neither loaded nor written back (they keep what the last reset left): 9 registers less across the
-    // substep loop and 56 bytes less traffic per drone and direction.
-    constexpr bool PID_DIET = BUILTIN && sizeof(R) == 4 && FAM != FAM_STAGE01;
-    if constexpr (PID_DIET) {
-#pragma unroll
-        for (int k = 0; k < 24; ++k) st.pid[k] = 0;
-        v = ld4(gp + 5 * stride); st.pid[0] = v.x; st.pid[1] = v.y; st.pid[2] = v.z; st.pid[3] = v.w;
-        st.pid[4] = reinterpret_cast<const R*>(gp + 6 * stride)[0];
-        v = ld4(gp + 8 * stride); st.pid[12] = v.x; st.pid[13] = v.y; st.pid[14] = v.z; st.pid[15] = v.w;
-        st.pid[16] = reinterpret_cast<const R*>(gp + 9 * stride)[0]; st.pid[17] = reinterpret_cast<const R*>(gp + 9 * stride)[1];
-    } else {
-#pragma unroll
-    for (int k = 0; k < NPID; ++k) {
-        v = ld4(gp + (5 + k) * stride);
-        st.pid[4 * k] = v.x; st.pid[4 * k + 1] = v.y; st.pid[4 * k + 2] = v.z; st.pid[4 * k + 3] = v.w;
-    }
-    }
+    Words::load(st, gp, stride);
     Imu<R> imu;
     const uint32_t env_id = T.env_offset + (uint32_t)env;
     const uint32_t phys0 = (uint32_t)A.p.env[(long long)env * ENV_WORDS + W_PHYS_CTR];
@@ -409,21 +423,7 @@ __global__ void __launch_bounds__(DYN_THREADS, (sizeof(R) == 4 ? DC_DYN_MIN_BLOC
         st4(ag + 2, V4<R>{imu.r, imu.qx, imu.qy, imu.qz});
         st4(ag + 3, V4<R>{imu.qw, 0, 0, 0});
     }
-    st4(gp, V4<R>{st.px, st.py, st.pz, (R)0});
-    st4(gp + stride, V4<R>{st.qx, st.qy, st.qz, st.qw});
-    st4(gp + 2 * stride, V4<R>{st.vx, st.vy, st.vz, (R)0});
-    st4(gp + 3 * stride, V4<R>{st.wx, st.wy, st.wz, (R)0});
-    st4(gp + 4 * stride, V4<R>{st.thr[0], st.thr[1], st.thr[2], st.thr[3]});
-    if constexpr (PID_DIET) {
-        st4(gp + 5 * stride, V4<R>{st.pid[0], st.pid[1], st.pid[2], st.pid[3]});
-        reinterpret_cast<R*>(gp + 6 * stride)[0] = st.pid[4];
-        st4(gp + 8 * stride, V4<R>{st.pid[12], st.pid[13], st.pid[14], st.pid[15]});
-        reinterpret_cast<R*>(gp + 9 * stride)[0] = st.pid[16]; reinterpret_cast<R*>(gp + 9 * stride)[1] = st.pid[17];
-    } else {
-#pragma unroll
-    for (int k = 0; k < NPID; ++k)
-        st4(gp + (5 + k) * stride, V4<R>{st.pid[4 * k], st.pid[4 * k + 1], st.pid[4 * k + 2], st.pid[4 * k + 3]});
-    }
+    Words::store(st, gp, stride);
     DC_TL_END(A.tl_slot);
 }
 
