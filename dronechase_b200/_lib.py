@@ -83,6 +83,8 @@ def lib():
     L.dc_lw_observe.restype = C.c_int
     L.dc_note_graph_replay.argtypes = [C.c_void_p]
     L.dc_note_graph_replay.restype = C.c_int
+    L.dc_set_ray_radii.argtypes = [C.c_void_p, C.c_float, C.c_float]
+    L.dc_set_ray_radii.restype = C.c_int
     L.dc_scatter_hits.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
     L.dc_scatter_hits.restype = C.c_int
     L.dc_scatter_stack.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]
@@ -144,7 +146,7 @@ def lib():
 EXPORTS = ("dc_create", "dc_bind", "dc_reset", "dc_step", "dc_set_actions", "dc_note_graph_replay", "dc_destroy", "dc_last_error", "dc_copy_state",
            "dc_state_bytes", "dc_lidar_project", "dc_lidar_raycast", "dc_launch_count", "dc_host_scatter_sphere", "dc_host_scatter_stack", "dc_scatter_hits",
            "dc_scatter_stack", "dc_abi_info", "dc_host_register", "dc_host_unregister", "dc_mirror_hits", "dc_lw_observe", "dc_quad_is_builtin", "dc_diff_hits", "dc_host_apply_pairs",
-           "dc_policy_create", "dc_policy_forward", "dc_policy_destroy", "dc_policy_create_ac", "dc_policy_act", "dc_gae", "dc_policy_serve")
+           "dc_policy_create", "dc_policy_forward", "dc_policy_destroy", "dc_policy_create_ac", "dc_policy_act", "dc_gae", "dc_policy_serve", "dc_set_ray_radii")
 
 
 def check(code: int, what: str):

@@ -85,7 +85,7 @@ class TaskConfig:
     vel_bonus: float = 1.0
     building: tuple = (0.0, 0.0, 0.1)
     fixed_lw_spawn: bool = False
-    lidar: str = "fused"              # "fused" (3,13,26) | "classic" (2,13,26)
+    lidar: str = "fused"              # "fused" (3,13,26) | "classic" (2,13,26) | "raycast" (3,13,26, needs ray_radius)
     family: str = "stage03"           # "stage03" (level4 tasks) | "stage02" (level3 L3Stage1) | "stage01" (level2) |
                                       # "level5" (threatsense Level5C1FusionTask: random agent, stacked-sphere fusion)
     initial_invaders: int = 4         # level5: wave k arms min((k-1)*invaders_per_round + initial_invaders, n_lm) munitions
@@ -105,10 +105,26 @@ class TaskConfig:
     noise_ratio: float | None = None  # None -> the model's motor_params.noise_ratio
     gyro_term: bool = False
     model: dict = field(default_factory=lambda: copy.deepcopy(CF2X))
+    # lidar="raycast": bounding radius (metres) of every wingman and of every munition, (r_lw, r_lm), that the rays of the
+    # agent's sphere are tested against.  No default: the reference's body dimensions (getVisualShapeData) are not known here.
+    ray_radius: tuple | None = None
 
     def __post_init__(self):
         if self.n_lm is None:
             self.n_lm = calculate_rounds(self.n_lw, self.munition)
+        if self.lidar == "raycast":
+            if self.family != "stage03" or self.lw_driver or self.eval_task:
+                raise ValueError("lidar='raycast' is built for the stage03 family without lw_driver / eval_task (the agent's "
+                                 "sphere only): not for level5 stacks, stage01/02 or policy-driven wingmen")
+            r = self.ray_radius
+            if r is None or len(r) != 2:
+                raise ValueError("lidar='raycast' needs ray_radius=(r_lw, r_lm), the bounding radius in metres of every wingman "
+                                 "and of every munition; there is no default")
+            if not all(math.isfinite(float(v)) and float(v) >= 0.0 for v in r):
+                raise ValueError(f"ray_radius must be finite and >= 0 metres, got {tuple(r)}")
+            self.ray_radius = (float(r[0]), float(r[1]))
+        elif self.ray_radius is not None:
+            raise ValueError("ray_radius is the bounding radius of lidar='raycast' and means nothing to lidar=%r" % self.lidar)
 
     @property
     def policy_slots(self) -> tuple:
@@ -121,7 +137,7 @@ class TaskConfig:
 
     @property
     def lidar_channels(self) -> int:
-        return 3 if self.lidar == "fused" else 2
+        return 2 if self.lidar == "classic" else 3
 
     @property
     def substeps(self) -> int:

@@ -20,6 +20,7 @@
 #include "stage03.cuh"
 #include "level5_stack.cuh"
 #include "driven.cuh"
+#include "raycast_env.cuh"
 
 namespace {
 
@@ -124,6 +125,10 @@ struct dc_sim {
     int32_t* mo_prev_n = nullptr;
     int2* lw_desc = nullptr;         // stage03 driven (dc_config.lw_driver): what dc_buffers.lw_lidar shows + Evaluation_Task.lw_kills
     int32_t* lw_kills = nullptr;
+    bool raycast = false;            // dc_config.lidar == DC_LIDAR_RAYCAST: env_kernel<FAM_RAYCAST> + raycast_sphere_kernel
+    float4* ray_snap = nullptr;      // env_kernel<FAM_RAYCAST>'s export of P4's inputs [E*D] (raycast_env.cuh)
+    float ray_r[2] = {0.f, 0.f};     // dc_set_ray_radii: bounding radius of a wingman / of a munition
+    bool reset_once = false;         // dc_reset has run: the radii are fixed from then on
     bool driven = false, has_nn = false;
     int mo_blocks = 0;
     int stack_blocks = 0;
@@ -238,12 +243,33 @@ template <typename R, int MODE, int FAM> auto env_kernel_for(int gs) -> void (*)
     return dc::env_kernel<R, MODE, FAM>;
 }
 
+// env_kernel of a step or reset; a ray-cast sim (stage03 only) runs its FAM_RAYCAST instantiation and then rebuilds the
+// agent's spheres
+template <typename R, int MODE, int FAM> cudaError_t launch_env(dc_sim* s, const dc::StepArgs<R>& a, cudaStream_t st, bool pdl) {
+    if constexpr (FAM == dc::FAM_STAGE03) {
+        if (s->raycast) {
+            dc::StepArgs<R> ea = a;
+            ea.ray_snap = s->ray_snap;
+            cudaError_t e = launch_step(s->gs == 8 ? dc::env_kernel<R, MODE, dc::FAM_RAYCAST, 8> : dc::env_kernel<R, MODE, dc::FAM_RAYCAST, 1>,
+                                        s->env_blocks, s->env_threads, s->smem, st, pdl, ea);
+            if (e != cudaSuccess) return e;
+            dc::RaySphereArgs<R> ra{};
+            ra.t = a.t; ra.agent = a.p.agent; ra.snap = s->ray_snap; ra.obs_lidar = a.obs_lidar; ra.lidar_ids = a.lidar_ids;
+            ra.ray_r[0] = s->ray_r[0]; ra.ray_r[1] = s->ray_r[1];
+            const int blocks = (s->cfg.n_envs + dc::RAY_ENV_WARPS - 1) / dc::RAY_ENV_WARPS;
+            g_launches.fetch_add(1, std::memory_order_relaxed);
+            return launch_step(dc::raycast_sphere_kernel<R>, blocks, dc::RAY_ENV_WARPS * 32, dc::ray_smem_bytes<R>(s->D), st, pdl, ra);
+        }
+    }
+    return launch_step(env_kernel_for<R, MODE, FAM>(s->gs), s->env_blocks, s->env_threads, s->smem, st, pdl, a);
+}
+
 template <typename R, int FAM> int launch_family(dc_sim* s, int mode, const uint8_t* mask, cudaStream_t st) {
     dc::StepArgs<R> a = make_args<R>(s, mask);
     if (mode == dc::MODE_RESET) {
         // env_kernel<RESET> rebuilds the whole work list the next dyn_kernel reads
         DC_CUDA(cudaMemsetAsync(s->count + s->parity, 0, sizeof(int32_t), st));
-        DC_CUDA(launch_step(env_kernel_for<R, dc::MODE_RESET, FAM>(s->gs), s->env_blocks, s->env_threads, s->smem, st, false, a));
+        DC_CUDA((launch_env<R, dc::MODE_RESET, FAM>(s, a, st, false)));
         g_launches.fetch_add(1, std::memory_order_relaxed);
         if constexpr (dc::fam_l5(FAM)) launch_stacks<R>(s, a, st);
     } else {
@@ -268,7 +294,7 @@ template <typename R, int FAM> int launch_family(dc_sim* s, int mode, const uint
         a.tl_slot += 1;
 #endif
         if (skip != 2)
-            DC_CUDA(launch_step(env_kernel_for<R, dc::MODE_STEP, FAM>(s->gs), s->env_blocks, s->env_threads, s->smem, st, pdl >= 1, a));
+            DC_CUDA((launch_env<R, dc::MODE_STEP, FAM>(s, a, st, pdl >= 1)));
         g_launches.fetch_add(2, std::memory_order_relaxed);
         if constexpr (dc::fam_l5(FAM)) {
             if (skip == 0) launch_stacks<R>(s, a, st);
@@ -323,6 +349,19 @@ template <typename R> int copy_drone_state(dc_sim* s, void* host, int to_device)
 }  // namespace
 
 namespace {
+// raycast_sphere_kernel's dynamic shared memory grows with the drones per env (ray_smem_bytes).  Its limit is an attribute of
+// the function, shared by every sim of the process on the current device: it is raised past the 48 KB default only when a
+// sim needs more, and never lowered, so creating a sim with fewer drones cannot make a larger sim's launches fail.
+template <typename K> cudaError_t raise_ray_smem_limit(K* kern, size_t bytes) {
+    if (bytes <= 48 * 1024) return cudaSuccess;
+    static std::mutex mu;
+    std::lock_guard<std::mutex> lk(mu);
+    cudaFuncAttributes fa{};
+    cudaError_t e = cudaFuncGetAttributes(&fa, kern);
+    if (e != cudaSuccess || (size_t)fa.maxDynamicSharedSizeBytes >= bytes) return e;
+    return cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+}
+
 // Run f(child, stream) for every sub-batch: child 0 on the caller's stream, the others on their own streams,
 // forked from and joined back into the caller's stream with events (also valid inside a stream capture).
 template <typename F> int fork_join(dc_sim* s, cudaStream_t st, F f) {
@@ -455,6 +494,9 @@ static int create_sim(const dc_config* cfg, int device, dc_sim** out, bool allow
         driven |= d != DC_DRIVER_LEGACY;
         has_nn |= d == DC_DRIVER_NN || d == DC_DRIVER_NN_ALLY;
     }
+    if (cfg->lidar == DC_LIDAR_RAYCAST && (cfg->family != DC_FAMILY_STAGE03 || driven))
+        return fail(DC_ERR_ARG, "dc_create: the ray-cast LiDAR is built for the stage03 family without lw_driver / eval_task "
+                                "(the agent's sphere only; level5 stacks, stage01/02 and policy-driven wingmen are not supported)");
     if (driven) {
         if (cfg->family != DC_FAMILY_STAGE03 || cfg->n_lw > 8 || cfg->lidar != DC_LIDAR_FUSED)
             return fail(DC_ERR_ARG, "dc_create: lw_driver / eval_task need family stage03, at most 8 wingmen and the fused LiDAR");
@@ -473,6 +515,7 @@ static int create_sim(const dc_config* cfg, int device, dc_sim** out, bool allow
     if (!s) return fail(DC_ERR_ARG, "dc_create: out of host memory");
     s->cfg = *cfg; s->device = device;
     s->driven = driven; s->has_nn = has_nn;
+    s->raycast = cfg->lidar == DC_LIDAR_RAYCAST;
     s->fam = kernel_family(cfg, driven);
     s->D = cfg->n_lw + cfg->n_lm;
     s->n_slots = (long long)cfg->n_envs * s->D;
@@ -550,7 +593,8 @@ static int create_sim(const dc_config* cfg, int device, dc_sim** out, bool allow
     t.n_envs = cfg->n_envs; t.n_lw = cfg->n_lw; t.n_lm = cfg->n_lm; t.D = s->D;
     t.munition = cfg->munition; t.step_increment = cfg->step_increment; t.max_step = cfg->max_step;
     t.initial_round = cfg->initial_round; t.substeps = cfg->substeps; t.lm_nav = cfg->lm_nav;
-    t.ally_mode = cfg->ally_mode; t.reward = cfg->reward; t.lidar = cfg->lidar;
+    t.ally_mode = cfg->ally_mode; t.reward = cfg->reward;
+    t.lidar = s->raycast ? DC_LIDAR_FUSED : cfg->lidar;      // env_kernel maintains the fused sphere the ray cast replaces
     t.fixed_lw_spawn = cfg->fixed_lw_spawn; t.auto_reset = cfg->auto_reset;
     t.family = cfg->family; t.support_munition = cfg->support_munition;
     t.initial_invaders = cfg->initial_invaders; t.invaders_per_round = cfg->invaders_per_round; t.max_rounds = cfg->max_rounds;
@@ -611,6 +655,10 @@ static int create_sim(const dc_config* cfg, int device, dc_sim** out, bool allow
         if (e == cudaSuccess) e = cudaMalloc((void**)&s->lw_desc, n_obs * s->D * sizeof(int2));
         if (e == cudaSuccess) e = cudaMemset(s->lw_desc, 0xFE, n_obs * s->D * sizeof(int2));      // dc::LW_DESC_UNUSED
     }
+    if (s->raycast) alloc0((void**)&s->ray_snap, (size_t)s->n_slots * sizeof(float4));
+    if (e == cudaSuccess && s->raycast)
+        e = s->rsz == 8 ? raise_ray_smem_limit(dc::raycast_sphere_kernel<double>, dc::ray_smem_bytes<double>(s->D))
+                        : raise_ray_smem_limit(dc::raycast_sphere_kernel<float>, dc::ray_smem_bytes<float>(s->D));
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
     if (e != cudaSuccess) { dc_destroy(s); return cuda_fail(e, "dc_create: device allocation"); }
     *out = s;
@@ -665,12 +713,15 @@ int dc_bind(dc_sim* s, const dc_buffers* b) {
         return fail(DC_ERR_ARG, "dc_bind: lidar_hits carries state and cannot be re-bound to another buffer");
     if (b->lidar_hits && (reinterpret_cast<uintptr_t>(b->lidar_hits) & 7))
         return fail(DC_ERR_ARG, "dc_bind: lidar_hits must be 8-byte aligned");
+    if (b->lidar_hits && s->cfg.lidar == DC_LIDAR_RAYCAST)
+        return fail(DC_ERR_ARG, "dc_bind: lidar_hits cannot describe a ray-cast sphere (one (cell, r_n) per drone slot; a bounding "
+                                "sphere covers several cells): leave it NULL with DC_LIDAR_RAYCAST");
     s->buf = *b; s->bound = true;
     for (size_t k = 0; k < s->kids.size(); ++k) {
         // a child sees its own rows of every [E, ...] tensor; stats is shared (atomics)
         const long long e0 = s->kid_start[k];
         const bool level5 = s->cfg.family == DC_FAMILY_LEVEL5;
-        const long long lidar_row = (long long)(level5 ? DC_LIDAR_STACK * 3 : (s->cfg.lidar == DC_LIDAR_FUSED ? 3 : 2)) * dc::N_CELLS;
+        const long long lidar_row = (long long)(level5 ? DC_LIDAR_STACK * 3 : (s->cfg.lidar == DC_LIDAR_CLASSIC ? 2 : 3)) * dc::N_CELLS;
         const long long hits_row = (long long)(level5 ? dc::STACK_MAX_SRC * s->D + 1 : s->D) * 2;
         dc_buffers c = *b;
         c.actions = b->actions + e0 * 4;
@@ -709,6 +760,7 @@ int dc_bind(dc_sim* s, const dc_buffers* b) {
 int dc_reset(dc_sim* s, const uint8_t* mask, void* stream) {
     if (!s) return fail(DC_ERR_ARG, "dc_reset: null sim");
     if (!s->bound) return fail(DC_ERR_UNBOUND, "dc_reset: call dc_bind first");
+    s->reset_once = true;
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     if (!s->kids.empty())
         return fork_join(s, st, [&](dc_sim* kid, cudaStream_t ks, int k) {
@@ -743,6 +795,17 @@ int dc_lw_observe(dc_sim* s, void* stream) {
     return DC_OK;
 }
 
+int dc_set_ray_radii(dc_sim* s, float r_lw, float r_lm) {
+    if (!s) return fail(DC_ERR_ARG, "dc_set_ray_radii: null sim");
+    if (s->cfg.lidar != DC_LIDAR_RAYCAST) return fail(DC_ERR_ARG, "dc_set_ray_radii: the sim was not created with DC_LIDAR_RAYCAST");
+    if (!(r_lw >= 0.0f && r_lm >= 0.0f && std::isfinite(r_lw) && std::isfinite(r_lm)))
+        return fail(DC_ERR_ARG, "dc_set_ray_radii: the radii must be finite and >= 0 (metres)");
+    if (s->reset_once) return fail(DC_ERR_ARG, "dc_set_ray_radii: the radii are fixed once dc_reset has run");
+    s->ray_r[0] = r_lw; s->ray_r[1] = r_lm;
+    for (dc_sim* kid : s->kids) { kid->ray_r[0] = r_lw; kid->ray_r[1] = r_lm; }
+    return DC_OK;
+}
+
 int dc_note_graph_replay(dc_sim* s) {
     if (!s) return fail(DC_ERR_ARG, "dc_note_graph_replay: null sim");
     for (dc_sim* kid : s->kids) kid->parity ^= 1;
@@ -768,6 +831,7 @@ void dc_destroy(dc_sim* s) {
     cudaFree(s->agent); cudaFree(s->env); cudaFree(s->lw_init); cudaFree(s->items[0]); cudaFree(s->items[1]);
     cudaFree(s->count); cudaFree(s->sphere_desc); cudaFree(s->last_dist); cudaFree(s->scratch);
     cudaFree(s->env5); cudaFree(s->ring_pose); cudaFree(s->ring_meta); cudaFree(s->ring_feat); cudaFree(s->stack_prev); cudaFree(s->stack_prev2); cudaFree(s->mo_prev); cudaFree(s->mo_prev_n); cudaFree(s->lw_desc); cudaFree(s->lw_kills);
+    cudaFree(s->ray_snap);
     delete s;
 }
 

@@ -28,7 +28,9 @@ namespace dc {
 // is split from FAM_L5 so that its extra code costs the hot level5 kernels nothing (it did: + 2.8 % on level5_c1 as
 // run-time branches); FAM_DRIVEN is stage03 with wingmen flown by policies inside the task (driven.cuh).
 enum { FAM_STAGE03 = DC_FAMILY_STAGE03, FAM_STAGE02 = DC_FAMILY_STAGE02, FAM_STAGE01 = DC_FAMILY_STAGE01,
-       FAM_L5 = DC_FAMILY_LEVEL5, FAM_L5_MULTI = 4, FAM_DRIVEN = 5 };
+       FAM_L5 = DC_FAMILY_LEVEL5, FAM_L5_MULTI = 4, FAM_DRIVEN = 5, FAM_RAYCAST = 6 };
+// FAM_RAYCAST names an env_kernel instantiation only: the stage03 step of a sim whose agent senses with the ray-cast LiDAR
+// (dc_config.lidar = DC_LIDAR_RAYCAST), which also exports what its LiDAR pass projected from (raycast_env.cuh).
 // the level5 (threatsense) envs: the RL agent is a random wingman, every wingman keeps an IMU record and a LiDAR ring
 __host__ __device__ constexpr bool fam_l5(int f) { return f == FAM_L5 || f == FAM_L5_MULTI; }
 // the families whose munitions come in waves, spawned by env_kernel's spawn pass
@@ -154,6 +156,7 @@ template <typename R> struct StepArgs {
     __device__ int env_of(int s) const { return (int)(((uint32_t)s * div_m) >> 20); }     // block slot -> block env
     int tl_slot;             // profiling builds (DC_PROFILE_PHASES): row of g_tl this launch stamps
     alignas(16) uint32_t rk[20];   // Philox round keys of (t.k0, t.k1) for philox4x32_10_rk (dyn_kernel's motor noise)
+    float4* ray_snap;        // env_kernel<FAM_RAYCAST>: [E*D] export of P4's inputs (RS_*); last, so no other field moves
 };
 
 #ifdef DC_PROFILE_PHASES      // launch timeline: first block start / last warp end of every step kernel, in globaltimer ns
@@ -1453,8 +1456,16 @@ template <typename R, int FAM> __device__ __forceinline__ void first_use_sphere(
     }
 }
 
-template <typename R, int MODE, int FAM, int GS = 1>
+// What P4 projects from, exported per slot by the FAM_RAYCAST instantiation for raycast_sphere_kernel (raycast_env.cuh) into
+// StepArgs::ray_snap: the float32 IMU snapshot position and a flag word -- RS_ENTITY: P4 projects this entity into the agent's
+// sphere (alive after the engagement, not the agent, the agent still a publisher); RS_UPDATE (slot 0 only): P4 updates the
+// env's sphere this step.  Every other instantiation exports nothing.
+enum { RS_ENTITY = 1, RS_UPDATE = 2 };
+
+// KFAM: the family (FAM_*), or FAM_RAYCAST -- the stage03 step plus the export above
+template <typename R, int MODE, int KFAM, int GS = 1>
 __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOCKS : 1)) env_kernel(const StepArgs<R> A) {
+    constexpr int FAM = KFAM == FAM_RAYCAST ? FAM_STAGE03 : KFAM;
     static_assert(GS == 1 || FAM == FAM_STAGE03, "lane groups are built for the stage03 family only");
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const TaskParams& T = A.t;
@@ -1711,6 +1722,14 @@ __global__ void __launch_bounds__(ENV_THREADS, (sizeof(R) == 4 ? DC_ENV_MIN_BLOC
 
     DC_STAMP(4);
     if (MODE == MODE_STEP) asm volatile("griddepcontrol.launch_dependents;");     // the next step's dyn_kernel waits for the whole grid
+    if constexpr (KFAM == FAM_RAYCAST) {
+        for (int s = S_LO + lane; s < S_HI; s += 32) {
+            const int le = A.env_of(s), d = s - le * D;
+            const bool on = MODE == MODE_STEP && (S.envflag[le] & EF_LIDAR);
+            const int f = d == 0 ? (on ? RS_UPDATE : 0) : ((on && (S.ev[s] & EV_MID)) ? RS_ENTITY : 0);
+            A.ray_snap[slot0 + s] = make_float4((float)S.imu[3 * s], (float)S.imu[3 * s + 1], (float)S.imu[3 * s + 2], __int_as_float(f));
+        }
+    }
     // ---- P4: LiDAR over the entities alive after engagement --------
     if (MODE == MODE_STEP && fam_l5(FAM)) {
         level5_ring_pass(A, S, env0, S_LO, S_HI, lane);

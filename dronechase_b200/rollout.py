@@ -29,6 +29,10 @@ from .sim import BatchedThreatEngageEnv
 
 class DeviceRollout:
     def __init__(self, env: BatchedThreatEngageEnv, n_steps: int):
+        if env.cfg.lidar == "raycast":
+            raise _lib.DroneChaseError("the rollout stores the sphere as its hit list, one (cell, r_n) per drone slot, which "
+                                       "cannot describe a ray-cast sphere (lidar='raycast'); hit-list storage of ray-cast "
+                                       "spheres is not built")
         if env.lidar_hits is None:
             raise _lib.DroneChaseError("create the env with with_hits=True: the rollout stores the sphere as its hit list")
         self.env, self.n_steps = env, int(n_steps)

@@ -22,7 +22,7 @@ from .config import TaskConfig, preset, quad_param_vector
 _NAV = {"air": 0, "full": 1}
 _ALLY = {"bt": 0, "stop": 1}
 _REWARD = {"vfinal": 0, "v2full": 1, "l5_fusion": 2}
-_LIDAR = {"fused": 0, "classic": 1}
+_LIDAR = {"fused": 0, "classic": 1, "raycast": 2}
 _DRIVER = {"legacy": 0, "nn": 1, "bt": 2, "stop": 3, "nn_ally": 4}
 INFO_KEYS = ("agent_kills", "allies_kills", "deads", "current_wave", "building_life", "step", "max_step",
              "episode_steps")
@@ -53,6 +53,9 @@ class BatchedThreatEngageEnv:
                  sub_batches: int = 0, with_student: bool = False):
         if isinstance(cfg, str):
             cfg = preset(cfg)
+        if cfg.lidar == "raycast" and with_hits:
+            raise ValueError("with_hits: the hit list holds one (cell, r_n) per drone slot and cannot describe a ray-cast sphere, "
+                             "whose bounding spheres cover several cells (hit-list storage of ray-cast spheres is not built)")
         if not torch.cuda.is_available():
             raise _lib.DroneChaseError("dronechase_b200 needs a CUDA device: there is no CPU fallback")
         self.cfg, self.n_envs, self.seed = cfg, int(n_envs), int(seed)
@@ -86,6 +89,8 @@ class BatchedThreatEngageEnv:
         self._c = c
         self._sim = C.c_void_p()
         _lib.check(self._L.dc_create(C.byref(c), self.device.index or 0, C.byref(self._sim)), "dc_create")
+        if cfg.lidar == "raycast":
+            _lib.check(self._L.dc_set_ray_radii(self._sim, *cfg.ray_radius), "dc_set_ray_radii")
         E, dev = self.n_envs, self.device
         f32 = dict(dtype=torch.float32, device=dev)
         self.actions = torch.zeros(E, 4, **f32)

@@ -268,6 +268,12 @@ class DroneChaseVecEnv(_VecEnvBase):
             raise ValueError("the multi-observer / evaluation level5 envs return no per-env observation dict: use "
                              "BatchedThreatEngageEnv(...).multi_obs / dronechase_b200.io_data.collect_data_multiobs, or the "
                              "single-env facades Level5DumbMultiObs / Level52BTEvaluationEnvironment")
+        if cfg.lidar == "raycast":
+            # a ray-cast sphere has no per-slot hit list: it crosses PCIe dense (4 KB per env)
+            if pairs_lidar or mapped_lidar:
+                raise ValueError("lidar='raycast' moves the sphere dense: pairs_lidar / mapped_lidar need the per-slot hit "
+                                 "list, which cannot describe a ray-cast sphere")
+            sparse_lidar, pairs_lidar, mapped_lidar = False, False, False
         self.sparse = bool(sparse_lidar)
         self._lidar_key = "stacked_spheres" if cfg.family == "level5" else "lidar"
         # level4/3/2 families: "pairs" (default) | "mapped" | "scatter" (hit list + host scatter, also the level5 way);

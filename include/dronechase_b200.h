@@ -53,7 +53,9 @@ enum { DC_NAV_AIR_COMBAT_ONLY = 0, DC_NAV_FULL = 1 };   /* loitering_munition_na
 enum { DC_ALLY_BEHAVIOR_TREE = 0, DC_ALLY_STOPPED = 1 }; /* loyalwingman_navigator.py / exp04_vFinal_task.py:240-242 */
 enum { DC_REWARD_VFINAL = 0, DC_REWARD_V2FULL = 1,      /* exp02_vFinal_task.py:422-568 / exp02_v2_full_task.py */
        DC_REWARD_L5_FUSION = 2 };                        /* level5 family only: level5_fusion_task.py:448-555 instead of the C1 reward */
-enum { DC_LIDAR_FUSED = 0, DC_LIDAR_CLASSIC = 1 };       /* (3,13,26) fused_lidar.py / (2,13,26) lidar.py */
+enum { DC_LIDAR_FUSED = 0, DC_LIDAR_CLASSIC = 1,        /* (3,13,26) fused_lidar.py / (2,13,26) lidar.py */
+       DC_LIDAR_RAYCAST = 2 };   /* (3,13,26), the fused layout: the agent's sphere ray-cast against bounding spheres
+                                    (dc_set_ray_radii); stage03 family without lw_driver / eval_task only, no lidar_hits */
 enum { DC_PRECISION_F32 = 0, DC_PRECISION_F64 = 1 };     /* arithmetic + state type of the dynamics */
 enum { DC_DRIVER_LEGACY = 0,    /* the task's own rule: slot 0 = dc_buffers.actions, the others dc_config.ally_mode */
        DC_DRIVER_NN = 1,        /* dc_buffers.lw_actions[:, j] whenever armed ("nn": driver.predict(compute_lw_observation)) */
@@ -217,6 +219,10 @@ int dc_set_actions(dc_sim* sim, const float* actions);
  * them alternately; after every replay call dc_note_graph_replay so that the host-side parity (used by dc_reset and
  * dc_copy_state) follows the device.  dronechase_b200.sim.BatchedThreatEngageEnv.step_graph does exactly this. */
 int dc_note_graph_replay(dc_sim* sim);
+/* DC_LIDAR_RAYCAST only: the bounding radius (metres, finite, >= 0) of every wingman and of every munition that the rays
+ * of the agent's sphere are tested against.  Valid between dc_create and the first dc_reset; both are 0 until set, which
+ * gives the fused projection's sphere bit for bit.  An observer inside a bounding sphere sees it in every cell. */
+int dc_set_ray_radii(dc_sim* sim, float r_lw, float r_lm);
 void dc_destroy(dc_sim* sim);
 const char* dc_last_error(void);
 
